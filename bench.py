@@ -5,6 +5,7 @@ configuration BASELINE.json quotes: 30-particle jets, batch 512 per GPU, maxdim 
 
     python bench.py --gpus N --steps K --warmup W            # one process per GPU (torchrun for N > 1)
     python bench.py --impl reference ...                     # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # + the results of the last timed step as DIR/<name>.npy (float64)
 
 Prints ONE JSON line (rank 0).  `value` = whole-job jets/s with the inputs resident in HBM; `e2e` = the same step
 through the public module API with the jets starting in pinned HOST memory and the loss read back every step;
@@ -281,6 +282,37 @@ def reference_subprocess(extra, timeout=600):
         return {"unavailable": repr(e)[:300]}
 
 
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(out_dir, fstep):
+    """Write what the step computed in its last run, the results a caller of FusedTrainStep receives, as float64 .npy files:
+    loss, recon, latent00, latent11, norm_factor, and grad_encoder / grad_decoder (every parameter's .grad flattened and
+    concatenated in named_parameters() order).  The inputs are seeded, so two builds can be compared output for output.  When
+    the per-jet arrays would take the files past DUMP_LIMIT_BYTES, they keep a fixed, seeded sample of jets, listed in
+    jet_index.npy."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    out = {"loss": fstep.loss}
+    for tag, model in (("encoder", fstep.enc), ("decoder", fstep.dec)):
+        out[f"grad_{tag}"] = torch.cat([p.grad.reshape(-1) for _, p in model.named_parameters()])
+    per_jet = {"recon": (fstep.recon, 1), "latent00": (fstep.latent00, 1), "latent11": (fstep.latent11, 1), "norm_factor": (fstep.norm_factor, 0)}
+    B = fstep.B
+    fixed_bytes = sum(t.numel() * 8 for t in out.values()) + 256 * (len(out) + len(per_jet) + 1)   # + .npy headers
+    jet_bytes = sum(t.numel() // B * 8 for t, _ in per_jet.values())
+    keep = (DUMP_LIMIT_BYTES - fixed_bytes) // (jet_bytes + 8)
+    idx = None
+    if B > keep:
+        idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out["jet_index"] = idx
+    for name, (t, axis) in per_jet.items():
+        out[name] = t if idx is None else t.index_select(axis, idx.to(t.device))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float64).cpu().numpy())
+
+
 def extra_cfg3_strong(enc, dec, world, rank, dev, timed, W, K):
     """BASELINE configs[2] as written: GLOBAL batch 4096 sharded over the ranks (strong scaling: 4096 / world jets per GPU)."""
     import torch
@@ -413,7 +445,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg3 (global batch 4096) / cfg4 / cfg5 objects of the line")
     ap.add_argument("--ref-device", default="cpu", help="reference arm only: cpu (the baseline) or cuda (stock ATen kernels, informative)")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the results of the last one as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 step")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -483,6 +520,8 @@ def main():
     for _ in range(W):
         fstep.run()
     ms_step, _ = timed(fstep.run, K)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fstep)
 
     # ---- end to end: pinned host jets -> device, loss back to the host, every step ----
     # (the jets of the step sit in pinned host memory; the H2D copy, the step and the D2H copy of the loss are one graph launch)

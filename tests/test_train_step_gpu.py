@@ -358,3 +358,68 @@ def test_peer_allreduce_single_rank_and_split_step():
                                    ptr(step.p4), ptr(step.norm_factor), ptr(step.ws_e), ptr(step.ws_d), ptr(step.latent00), ptr(step.latent11),
                                    ptr(step.sel), ptr(step.recon), ptr(step.g_recon), ptr(step.g_lat11), ptr(step.jet_loss), ptr(step.loss),
                                    ptr(step.g_all), step.off_d, ptr(step.part), step.l1, step.get_real, 2, st) == -1
+
+
+def test_bench_dump_outputs_are_the_timed_step_results(tmp_path):
+    """bench.py --dump-outputs writes the loss, reconstruction, latents, normalisation and gradients of its timed step; they
+    match the same step run here on the same seeded models and jets, and --steps is the number of timed steps it reports."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    from bench import CFG, build_models, synthetic_jets
+    from lgn_autoencoder_b200.train import FusedTrainStep
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    B, out = 16, tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "0", "--batch", str(B),
+                        "--no-cpu-baseline", "--no-extras", "--dump-outputs", str(out)], cwd=tmp_path, capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    assert line["steps"] == 2
+    dev = torch.device("cuda:0")
+    enc, dec = build_models(dev)
+    step = FusedTrainStep(enc, dec, B, l1_lambda=CFG["l1_lambda"], normalize=True, get_real="sum")
+    loss = step.step(synthetic_jets(B, CFG["n"], seed=100).to(dev))
+    torch.cuda.synchronize()
+    want = {"loss": loss, "recon": step.recon, "latent00": step.latent00, "latent11": step.latent11, "norm_factor": step.norm_factor,
+            "grad_encoder": torch.cat([p.grad.reshape(-1) for _, p in enc.named_parameters()]),
+            "grad_decoder": torch.cat([p.grad.reshape(-1) for _, p in dec.named_parameters()])}
+    assert sorted(os.listdir(out)) == sorted(f"{k}.npy" for k in want)
+    for name, ref in want.items():
+        got = np.load(out / f"{name}.npy")
+        assert got.dtype == np.float64 and got.shape == tuple(ref.shape), name
+        assert rel_err(torch.from_numpy(got), ref) < 1e-12, (name, rel_err(torch.from_numpy(got), ref))
+
+
+def test_bench_dump_outputs_sample_jets_past_the_size_limit(tmp_path, monkeypatch):
+    """When the per-jet arrays would take the dump past its size limit, it keeps a seeded, sorted sample of jets: jet_index
+    lists them, recon / latents are cut along the batch axis (1) and norm_factor along its only axis, and the files fit."""
+    import os
+
+    import numpy as np
+
+    import bench
+    from lgn_autoencoder_b200.train import FusedTrainStep
+    dev = torch.device("cuda:0")
+    B = 16
+    enc, dec = bench.build_models(dev)
+    step = FusedTrainStep(enc, dec, B, l1_lambda=bench.CFG["l1_lambda"], normalize=True, get_real="sum")
+    step.step(bench.synthetic_jets(B, bench.CFG["n"], seed=100).to(dev))
+    torch.cuda.synchronize()
+    n_grad = sum(p.numel() for m in (enc, dec) for p in m.parameters())
+    limit = 8 * (n_grad + 1) + 4096 + 6 * 2560     # room for the gradients, the loss, the headers and a few jets
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", limit)
+    out = tmp_path / "dump"
+    bench.dump_outputs(str(out), step)
+    assert sum(os.path.getsize(out / f) for f in os.listdir(out)) <= limit
+    idx = np.load(out / "jet_index.npy")
+    assert idx.dtype == np.float64 and 0 < len(idx) < B and np.all(np.diff(idx) > 0)
+    sel = torch.from_numpy(idx.astype(np.int64)).to(dev)
+    for name, t, axis in (("recon", step.recon, 1), ("latent00", step.latent00, 1), ("latent11", step.latent11, 1), ("norm_factor", step.norm_factor, 0)):
+        assert np.array_equal(np.load(out / f"{name}.npy"), t.index_select(axis, sel).cpu().numpy()), name
+    assert np.array_equal(np.load(out / "loss.npy"), step.loss.cpu().numpy())
+    bench.dump_outputs(str(tmp_path / "again"), step)
+    assert np.array_equal(np.load(tmp_path / "again" / "jet_index.npy"), idx)
