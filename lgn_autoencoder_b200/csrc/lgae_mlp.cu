@@ -604,11 +604,14 @@ int run_mlp(const LgaeModelDesc* d, int level, const double* theta, const double
             if (int rc = plan->seg(a.off_b[i], off, w, a.po_b[i], nout, grid)) return rc;
         }
     }
+    // nti = ceil(2C'/8): 1 for C' <= 4 output channels, 2 for C' = 5..8.  The hidden width is mlp_width * 2C' >= nin, and the
+    // modules admit widths up to 48 (ntw <= 6), so with nti = 2 every ntw from 2 to 6 is reachable.
     const int ntw = (a.width + 7) / 8, nti = (a.nin + 7) / 8;
 #define LGAE_MLP_CASE(W, I) \
     if (ntw == W && nti == I) return launch_mlp<W, I>(a, bwd, st);
     LGAE_MLP_CASE(1, 1) LGAE_MLP_CASE(2, 1) LGAE_MLP_CASE(3, 1) LGAE_MLP_CASE(4, 1)
     LGAE_MLP_CASE(5, 1) LGAE_MLP_CASE(6, 1)
+    LGAE_MLP_CASE(2, 2) LGAE_MLP_CASE(3, 2) LGAE_MLP_CASE(4, 2) LGAE_MLP_CASE(5, 2) LGAE_MLP_CASE(6, 2)
     LGAE_MLP_CASE(8, 2) LGAE_MLP_CASE(9, 2)
 #undef LGAE_MLP_CASE
     return LGAE_E_UNSUPPORTED;
