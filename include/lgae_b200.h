@@ -108,16 +108,13 @@ int64_t lgae_workspace_doubles(const LgaeModelDesc* d, int32_t batch);
  * 1 = V_in[level] (B,N,C,4,2) (level == n_levels gives the final features), 2 = pre-MLP scalars of level,
  * 3 = canonical momenta y (B,N,4,2), 4 = neighbour sums of level (B,N,C,10,2), 5 = masses (B,N) (encoder),
  * 6 = MLP activations of level (hidden, B*N, padded width), 7 = radial weights of level (B,N,C,32,4) (encoder, N <= 32),
- * 8 = dL/dR of level (B,N,C,32,4) (encoder, N <= 32; one buffer per level: the radial adjoint of a level overlaps the next one). */
+ * 8 = dL/dR of level (B,N,C,32,4) (encoder, N <= 32; one buffer per level). */
 int64_t lgae_workspace_offset(const LgaeModelDesc* d, int32_t batch, int32_t kind, int32_t level);
 /* Doubles of scratch for the per-CTA rows of parameter-gradient partials the backward entry points write (every
  * backward kernel owns a block of compact rows; one reduce launch sums them into gtheta, in a fixed order). */
 int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch);
 
 /* ---- whole-model entry points -------------------------------------------------------------------- */
-/* With LGAE_OVERLAP=1 (environment; off by default, no measured gain at batch 512) the encoder entry points run the
- * radial-function kernels on a library-owned side stream, forked from and joined back into `stream` with events (a CUDA-graph
- * capture of `stream` records them as a parallel branch); all work is complete in `stream` order when the call returns. */
 /* LGNEncoder.forward.  p4 (B,N,4) Cartesian (E,px,py,pz); node_mask (B,N) uint8 or NULL (=> p4[...,0] != 0).
  * Outputs, planar like the reference: lat00 (2,B,1,T_s,1), lat11 (2,B,1,T_v,4) with T = tau (x2 for min&max);
  * sel (int32, device) receives the selected particle indices for min/max modes: (4, 2, B, tau_max) laid out as
@@ -170,10 +167,12 @@ int lgae_train_step_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, con
                          int64_t gtheta_dec_offset, double* partials, double l1_lambda, int32_t get_real, int32_t phase, void* stream);
 /* Split step for data-parallel training (`phase` above): phase 0 runs the whole step.  phase 1 runs it up to the point where the
  * DECODER's gradient bucket gtheta[gtheta_dec_offset, ...) is final -- its reduce is the last thing enqueued on the library's
- * auxiliary stream of the current device, which this function returns (NULL when LGAE_NO_AUX=1) -- and phase 2 (same thread, same
- * arguments, directly afterwards) runs the encoder adjoint and the encoder bucket's reduce on `stream` and joins the auxiliary
- * stream back.  A caller enqueues the all-reduce of the decoder bucket on the auxiliary stream between the two calls: it then
- * overlaps the encoder adjoint (SURVEY.md section 8(e) describes the exchange; the reference itself is single-process). */
+ * auxiliary stream of the current device, which this function returns -- and phase 2 (same thread, same arguments, directly
+ * afterwards) runs the encoder adjoint and the encoder bucket's reduce on `stream` and joins the auxiliary stream back.  A caller
+ * enqueues the all-reduce of the decoder bucket on the auxiliary stream between the two calls: it then overlaps the encoder
+ * adjoint (SURVEY.md section 8(e) describes the exchange; the reference itself is single-process).  Every training step uses
+ * the auxiliary stream: if it cannot be created, this function returns NULL, the step fails with LGAE_E_CUDA, and
+ * lgae_last_cuda_error says why. */
 void* lgae_aux_stream(void);
 
 

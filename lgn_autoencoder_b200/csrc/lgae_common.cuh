@@ -311,12 +311,11 @@ struct PartPlan {
 // prologue that only touches step-constant data (weights in theta, index tables, barrier setup) and blocks in pdl_wait()
 // until all earlier kernels have completed and flushed their writes.  Every read of a predecessor's output and every global
 // write comes after pdl_wait().  The launch latency and the prologues of the ~45 kernels of a step overlap the previous
-// kernel's tail; captured in a CUDA graph the edges become programmatic dependencies.  LGAE_NO_PDL=1 disables it.
+// kernel's tail; captured in a CUDA graph the edges become programmatic dependencies.
 LGAE_DEV void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 LGAE_DEV void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // ---- host side ------------------------------------------------------------------------------------
-bool pdl_enabled();
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
     cudaLaunchConfig_t cfg = {};
@@ -328,7 +327,7 @@ inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 void count_launch(int n = 1);

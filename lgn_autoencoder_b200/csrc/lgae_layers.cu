@@ -522,11 +522,8 @@ static int lin_splits(int64_t rows) {
     const int64_t s = std::min<int64_t>((rows + 127) / 128, (int64_t)sm_count());
     return (int)std::max<int64_t>(1, s);
 }
-// LGAE_LINEAR_FMA=1 keeps the plain tiled-FMA kernels (A/B checks); widths above LMMA_MAX always use them.
-static bool lin_use_mma(int n_in, int n_out) {
-    static const bool off = [] { const char* e = getenv("LGAE_LINEAR_FMA"); return e && e[0] == '1'; }();
-    return !off && n_in <= LMMA_MAX && n_out <= LMMA_MAX;
-}
+// Widths above LMMA_MAX use the plain tiled-FMA kernels.
+static bool lin_use_mma(int n_in, int n_out) { return n_in <= LMMA_MAX && n_out <= LMMA_MAX; }
 template <bool BWDX>
 static int launch_lin_mma(const LinArgs& a, cudaStream_t st) {
     const int K = BWDX ? a.nout : a.nin, N = BWDX ? a.nin : a.nout;

@@ -11,7 +11,6 @@
 // MMA (phi (pairs x K) times W^T (K x 4C)) into shared memory and consumed by the (i, c) threads; the neighbour
 // sums stay in registers.  The only O(N^2) tensor that goes to HBM is the optional copy of the radial weights
 // R_ij[c] (r_save) that the training forward keeps for the adjoint, which then does not re-evaluate them.
-#include <cstdlib>
 #include <cstring>
 
 #include "lgae_common.cuh"
@@ -195,6 +194,7 @@ __host__ __device__ inline LevelSmem level_smem(bool enc, bool tiles, int N, int
 // ------------------------------------------------------------------------------------------------------------
 // PRE (encoder, N <= 32): the radial weights were computed by radial_fwd_kernel and are streamed from r_save (one
 // double4 per partner, prefetched one partner ahead); no radial tiles, no barriers inside the neighbour loop.
+// The decoder is launched as <false, 1, 3, true> and takes the O(N) closed form.
 template <bool ENC, int NT, int KS, bool PRE>
 __global__ void __launch_bounds__(256) level_fwd_kernel(const LevelArgs a) {
     extern __shared__ __align__(128) double smem[];
@@ -326,42 +326,30 @@ __global__ void __launch_bounds__(256) level_fwd_kernel(const LevelArgs a) {
             A1Y[mu] = cmul(R1c, csub(cmul(yi[mu], SS), SSY[mu]));
         }
     } else {
-    // one neighbour j with its radial weights: the four neighbour sums of this (particle, channel)
+    // encoder: one neighbour j with its radial weights: the four neighbour sums of this (particle, channel)
     auto pair = [&](int j, int js, cplx R0, cplx R1) {   // js: where partner j's features lie in S_s / V_s
         const cplx Sj = S_s[js * C + c];
         cplx Vj[4];
 #pragma unroll
         for (int mu = 0; mu < 4; ++mu) Vj[mu] = V_s[(js * C + c) * 4 + mu];
         cplx Y[4];
-        if (ENC) {
-            double d[4];
+        double d[4];
 #pragma unroll
-            for (int mu = 0; mu < 4; ++mu) d[mu] = pi[mu] - p_s[4 * j + mu];
-            canon_from_real(d, Y);
-        } else {
-#pragma unroll
-            for (int mu = 0; mu < 4; ++mu) Y[mu] = csub(yi[mu], reinterpret_cast<const cplx*>(p_s)[4 * j + mu]);
-        }
+        for (int mu = 0; mu < 4; ++mu) d[mu] = pi[mu] - p_s[4 * j + mu];
+        canon_from_real(d, Y);
 #pragma unroll
         for (int mu = 0; mu < 4; ++mu) cfma(A0V[mu], R0, Vj[mu]);
         cfma(A0S, R0, Sj);
         const cplx t = cmul(R1, Sj);
-        cplx e;
-        if (ENC) {
-            // Y0, Y2 are real, Y3 = -conj... structured: saves a third of the multiplies
-            cfmar(A1Y[0], t, Y[0].x);
-            cfma(A1Y[1], t, Y[1]);
-            cfmar(A1Y[2], t, Y[2].x);
-            cfma(A1Y[3], t, Y[3]);
-            e = cscale(Vj[0], Y[0].x);
-            cfma(e, Vj[1], Y[3]);
-            cfmar(e, Vj[2], -Y[2].x);
-            cfma(e, Vj[3], Y[1]);
-        } else {
-#pragma unroll
-            for (int mu = 0; mu < 4; ++mu) cfma(A1Y[mu], t, Y[mu]);
-            e = ceta(Vj, Y);
-        }
+        // Y0, Y2 are real, Y3 = -conj... structured: saves a third of the multiplies
+        cfmar(A1Y[0], t, Y[0].x);
+        cfma(A1Y[1], t, Y[1]);
+        cfmar(A1Y[2], t, Y[2].x);
+        cfma(A1Y[3], t, Y[3]);
+        cplx e = cscale(Vj[0], Y[0].x);
+        cfma(e, Vj[1], Y[3]);
+        cfmar(e, Vj[2], -Y[2].x);
+        cfma(e, Vj[3], Y[1]);
         cfma(A1E, R1, e);
     };
     if (ring) {
@@ -388,11 +376,11 @@ __global__ void __launch_bounds__(256) level_fwd_kernel(const LevelArgs a) {
 #pragma unroll
     for (int d = 0; d < PDF; ++d) {
         rq[d] = make_double4(0.0, 0.0, 0.0, 0.0);
-        if (ENC && PRE && d < N) rq[d] = rsv[(int64_t)d * C * 32];
+        if (PRE && d < N) rq[d] = rsv[(int64_t)d * C * 32];
     }
     for (int j0 = 0; j0 < N; j0 += TJ) {
         const int tj = min(TJ, N - j0);
-        if (ENC && !PRE) {
+        if (!PRE) {
             // the tile's partner features: global loads in flight during the radial tile, then into shared memory
             constexpr int NPF = (TJ * 5 + 31) / 32;
             cplx pf[NPF];
@@ -416,21 +404,21 @@ __global__ void __launch_bounds__(256) level_fwd_kernel(const LevelArgs a) {
 #pragma unroll kFwdUnroll
         for (int jj = 0; jj < tj; ++jj) {
             const int j = j0 + jj;
-            cplx R0 = R0c, R1 = R1c;
-            if (ENC && PRE) {
+            cplx R0 = czero(), R1 = czero();
+            if (PRE) {
                 R0 = cmake(rq[0].x, rq[0].y);
                 R1 = cmake(rq[0].z, rq[0].w);
 #pragma unroll
                 for (int d = 0; d + 1 < PDF; ++d) rq[d] = rq[d + 1];
                 if (j + PDF < N) rq[PDF - 1] = rsv[(int64_t)(j + PDF) * C * 32];
-            } else if (ENC) {
+            } else {
                 const double4 r = *reinterpret_cast<const double4*>(Rs + ((size_t)((jj * C + c) * 32 + lane)) * 4);
                 R0 = cmake(r.x, r.y);
                 R1 = cmake(r.z, r.w);
             }
-            pair(j, (ENC && !PRE) ? jj : j, R0, R1);
+            pair(j, PRE ? j : jj, R0, R1);
         }
-        if (ENC && !PRE) __syncthreads();
+        if (!PRE) __syncthreads();
     }
     }
     }
@@ -612,11 +600,11 @@ LGAE_DEV void mix_adjoint_block(int k, int Cout, int C5, int nm, int lane, const
 // One CTA works on one jet at a time (persistent over jets); warp = channel c, lane = particle.
 //   1. stage the jet, rebuild this thread's 25 cat entries from the saved neighbour sums, push the incoming gradients
 //      through the adjoint of the channel mix (registers + warp butterflies, no cat buffer in shared memory);
-//   2. neighbour loop over partners o, no barriers: role 1 (own = receiving node) yields dL/dR_{lane,o}, streamed to
-//      g_r for radial_bwd_kernel (encoder) or summed (decoder: constant radial weights); role 2 (own = neighbour)
-//      accumulates dL/dS_lane, dL/dV_lane in registers.  Encoder: R_{lane,o} is streamed from r_save, prefetched;
+//   2. encoder: neighbour loop over partners o, no barriers: role 1 (own = receiving node) yields dL/dR_{lane,o}, streamed to
+//      g_r for radial_bwd_kernel; role 2 (own = neighbour) accumulates dL/dS_lane, dL/dV_lane in registers; R_{lane,o} is
+//      streamed from r_save, prefetched.  Decoder: adjoint of the O(N) closed form (constant radial weights);
 //   3. when the CTA runs out of jets: one compact row of parameter-gradient partials (mix weights, decoder biases).
-template <bool ENC, int MAXT, int MINB, bool CF>
+template <bool ENC, int MAXT, int MINB>
 __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a) {
     extern __shared__ __align__(128) double smem[];
     const int N = a.N, C = a.C, Cout = a.Cout;
@@ -760,9 +748,9 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
             }
         }
         __syncthreads();  // gA_s of every channel is complete (role 2 reads other lanes' entries)
-        // ---- 2. neighbour loop ----
+        // ---- 2. adjoint of the neighbour sums ----
         cplx gy[4] = {czero(), czero(), czero(), czero()};
-        if (!ENC && CF) {
+        if (!ENC) {
             // Decoder, closed form: adjoint of  A0V_i = R0 SV, A0S_i = R0 SS, A1Y_i = R1 (y_i SS - SSY), A1E_i = R1 (eta(SV, y_i) - SVY)
             // with the jet-level moments SS, SV, SSY, SVY of the forward (recomputed here), all O(N).
             const cplx* y_s = reinterpret_cast<const cplx*>(p_s);
@@ -846,21 +834,13 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
             }
             gS = cadd(gS, gSa);
         } else {
+            // encoder: loop over the partners o
             double pa[4] = {0, 0, 0, 0};
-            cplx ya[4] = {czero(), czero(), czero(), czero()};
             if (live) {
-                if (ENC) {
 #pragma unroll
-                    for (int mu = 0; mu < 4; ++mu) pa[mu] = p_s[4 * i + mu];
-                } else {
-#pragma unroll
-                    for (int mu = 0; mu < 4; ++mu) ya[mu] = reinterpret_cast<const cplx*>(p_s)[4 * i + mu];
-                }
+                for (int mu = 0; mu < 4; ++mu) pa[mu] = p_s[4 * i + mu];
             }
-            const cplx Sa = live ? S_s[i * C + c] : czero();
-            cplx Va[4], gAa[10];
-#pragma unroll
-            for (int mu = 0; mu < 4; ++mu) Va[mu] = live ? V_s[(i * C + c) * 4 + mu] : czero();
+            cplx gAa[10];
 #ifndef LGAE_GAA_SMEM
 #pragma unroll
             for (int e = 0; e < 10; ++e) gAa[e] = gA_s[(c * 10 + e) * 32 + lane];
@@ -868,50 +848,31 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
             double4* grv = reinterpret_cast<double4*>(a.g_r) + ((int64_t)b * N * C + c) * 32 + lane;
 #pragma unroll kBwdUnroll
             for (int o = 0; o < N; ++o) {
-                cplx R0 = R0c, R1 = R1c;
-                if (ENC) {
-                    R0 = cmake(rq[0].x, rq[0].y);
-                    R1 = cmake(rq[0].z, rq[0].w);
+                const cplx R0 = cmake(rq[0].x, rq[0].y), R1 = cmake(rq[0].z, rq[0].w);
 #pragma unroll
-                    for (int d = 0; d + 1 < PDB; ++d) rq[d] = rq[d + 1];
-                    if (o + PDB < N) rq[PDB - 1] = rsv[(int64_t)(o + PDB) * C * 32];
-                }
+                for (int d = 0; d + 1 < PDB; ++d) rq[d] = rq[d + 1];
+                if (o + PDB < N) rq[PDB - 1] = rsv[(int64_t)(o + PDB) * C * 32];
                 const cplx So = S_s[o * C + c];
                 cplx Vo[4], Y[4];
 #pragma unroll
                 for (int mu = 0; mu < 4; ++mu) Vo[mu] = V_s[(o * C + c) * 4 + mu];
-                // encoder: Y = canon(p_i - p_o) = (d0, (ya, -yb), d3, (-ya, -yb)) with real d0, d3, ya, yb -- the contractions
+                // Y = canon(p_i - p_o) = (d0, (ya, -yb), d3, (-ya, -yb)) with real d0, d3, ya, yb -- the contractions
                 // with Y below use that structure (12 instead of 16 multiply-adds each)
-                double d0 = 0.0, d3 = 0.0, ya_ = 0.0, yb_ = 0.0;
-                if (ENC) {
-                    double d[4];
+                double d[4];
 #pragma unroll
-                    for (int mu = 0; mu < 4; ++mu) d[mu] = pa[mu] - p_s[4 * o + mu];
-                    canon_from_real(d, Y);
-                    d0 = Y[0].x; d3 = Y[2].x; ya_ = Y[1].x; yb_ = -Y[1].y;
-                } else {
-#pragma unroll
-                    for (int mu = 0; mu < 4; ++mu) Y[mu] = csub(ya[mu], reinterpret_cast<const cplx*>(p_s)[4 * o + mu]);
-                }
+                for (int mu = 0; mu < 4; ++mu) d[mu] = pa[mu] - p_s[4 * o + mu];
+                canon_from_real(d, Y);
+                const double d0 = Y[0].x, d3 = Y[2].x, ya_ = Y[1].x, yb_ = -Y[1].y;
                 // sum_mu conj(Y_mu) g_mu  and  eta(v, Y)
                 auto ydot = [&](const cplx* gq) {
-                    if (ENC) {
-                        const cplx dm = csub(gq[1], gq[3]), sp = cadd(gq[1], gq[3]);
-                        return cmake(fma(d0, gq[0].x, fma(d3, gq[2].x, fma(ya_, dm.x, -yb_ * sp.y))),
-                                     fma(d0, gq[0].y, fma(d3, gq[2].y, fma(ya_, dm.y, yb_ * sp.x))));
-                    }
-                    cplx w = czero();
-#pragma unroll
-                    for (int mu = 0; mu < 4; ++mu) cfmac(w, Y[mu], gq[mu]);
-                    return w;
+                    const cplx dm = csub(gq[1], gq[3]), sp = cadd(gq[1], gq[3]);
+                    return cmake(fma(d0, gq[0].x, fma(d3, gq[2].x, fma(ya_, dm.x, -yb_ * sp.y))),
+                                 fma(d0, gq[0].y, fma(d3, gq[2].y, fma(ya_, dm.y, yb_ * sp.x))));
                 };
                 auto yeta = [&](const cplx* v) {
-                    if (ENC) {
-                        const cplx vm = csub(v[3], v[1]), vp = cadd(v[1], v[3]);
-                        return cmake(fma(d0, v[0].x, fma(-d3, v[2].x, fma(ya_, vm.x, yb_ * vp.y))),
-                                     fma(d0, v[0].y, fma(-d3, v[2].y, fma(ya_, vm.y, -yb_ * vp.x))));
-                    }
-                    return ceta(v, Y);
+                    const cplx vm = csub(v[3], v[1]), vp = cadd(v[1], v[3]);
+                    return cmake(fma(d0, v[0].x, fma(-d3, v[2].x, fma(ya_, vm.x, yb_ * vp.y))),
+                                 fma(d0, v[0].y, fma(-d3, v[2].y, fma(ya_, vm.y, -yb_ * vp.x))));
                 };
                 // role 1: own = receiving node i, other = neighbour j.  Y = Y_ij.
                 {
@@ -927,23 +888,9 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
                     const cplx e = yeta(Vo);
                     cplx gR1 = cmulc(So, w);
                     cfmac(gR1, e, gAa[9]);
-                    if (ENC) {
-                        grv[(int64_t)o * C * 32] = make_double4(gR0.x, gR0.y, gR1.x, gR1.y);
-                    } else {
-                        gR0c = cadd(gR0c, live ? gR0 : czero());
-                        gR1c = cadd(gR1c, live ? gR1 : czero());
-                        // gy_i += conj(R1 S_j) gA1Y_i + conj(R1 ghat(V_j)) gA1E_i
-                        const cplx rs = cmul(R1, So);
-                        cplx gh[4];
-                        cghat(Vo, gh);
-#pragma unroll
-                        for (int mu = 0; mu < 4; ++mu) {
-                            cfmac(gy[mu], rs, gAa[5 + mu]);
-                            cfmac(gy[mu], cmul(R1, gh[mu]), gAa[9]);
-                        }
-                    }
+                    grv[(int64_t)o * C * 32] = make_double4(gR0.x, gR0.y, gR1.x, gR1.y);
                 }
-                // role 2: own = neighbour j, other = receiving node i.  Y_ij = -Y ; R_ij = R_ji (encoder).
+                // role 2: own = neighbour j, other = receiving node i.  Y_ij = -Y ; R_ij = R_ji.
                 {
                     cplx gAo[10];
 #pragma unroll
@@ -961,18 +908,6 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
                     }
                     cfmac(gS, R0, gAo[4]);
                     cfmac(gS, R1, w);
-                    if (!ENC) {
-                        // gy_j -= conj(R1 S_j) gA1Y_i + conj(R1 ghat(V_j)) gA1E_i
-                        const cplx rs = cmul(R1, Sa);
-                        cplx gha[4];
-                        cghat(Va, gha);
-#pragma unroll
-                        for (int mu = 0; mu < 4; ++mu) {
-                            cplx t = cmulc(rs, gAo[5 + mu]);
-                            cfmac(t, cmul(R1, gha[mu]), gAo[9]);
-                            gy[mu] = csub(gy[mu], t);
-                        }
-                    }
                 }
             }
         }
@@ -1020,13 +955,6 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
 // ------------------------------------------------------------------------------------------------------------
 static int pick_ks(int K) { return K <= 12 ? 3 : (K <= 20 ? 5 : (K <= 32 ? 8 : -1)); }
 
-// The decoder levels use the O(N) closed form unless LGAE_DEC_PAIRLOOP=1 asks for the reference-shaped O(N^2) neighbour
-// loop (kept for A/B checks of the closed form).
-static bool dec_pair_loop() {
-    static const bool v = [] { const char* e = getenv("LGAE_DEC_PAIRLOOP"); return e && e[0] == '1'; }();
-    return v;
-}
-
 template <bool ENC, int NT, int KS, bool PRE>
 static int launch_level_fwd(const LevelArgs& a, cudaStream_t st) {
     const LevelSmem L = level_smem(ENC, ENC && !PRE, a.N, a.C, a.Cout, KS);
@@ -1046,21 +974,19 @@ static int launch_level_bwd(const LevelArgs& a, int grid, cudaStream_t st) {
     const LevelBwdSmem L = level_bwd_smem(ENC, a.N, a.C, a.Cout);
     const size_t bytes = (size_t)L.total * sizeof(double);
     if (bytes > 227 * 1024) return LGAE_E_UNSUPPORTED;
-    const bool cf = !ENC && !dec_pair_loop();
     LaunchScope ls_("level_bwd", st);
-#define LGAE_LAUNCH(MAXT, MINB, CFV)                                          \
+#define LGAE_LAUNCH(MAXT, MINB)                                               \
     {                                                                         \
-        auto kern = level_bwd_kernel<ENC, MAXT, MINB, CFV>;                   \
+        auto kern = level_bwd_kernel<ENC, MAXT, (MINB)>;                      \
         if (int rc = ensure_smem((const void*)kern, bytes)) return rc;        \
         launch_k(kern, dim3(grid), dim3(32 * a.C), bytes, st, a);                               \
     }
-    if (a.C <= 3) {
-        if (cf) LGAE_LAUNCH(128, LGAE_LBWD_CF_MINB, true) else LGAE_LAUNCH(128, LGAE_LBWD_MINB, false)
-    } else if (a.C == 4) {
-        if (cf) LGAE_LAUNCH(128, LGAE_LBWD_CF_MINB_C4, true) else LGAE_LAUNCH(128, LGAE_LBWD_MINB_C4, false)
-    } else {
-        if (cf) LGAE_LAUNCH(256, 1, true) else LGAE_LAUNCH(256, 1, false)
-    }
+    if (a.C <= 3)
+        LGAE_LAUNCH(128, ENC ? LGAE_LBWD_MINB : LGAE_LBWD_CF_MINB)
+    else if (a.C == 4)
+        LGAE_LAUNCH(128, ENC ? LGAE_LBWD_MINB_C4 : LGAE_LBWD_CF_MINB_C4)
+    else
+        LGAE_LAUNCH(256, 1)
 #undef LGAE_LAUNCH
     return check_launch("level_bwd");
 }
@@ -1073,7 +999,7 @@ int level_bwd_grid(int batch) {
 
 static int dispatch_level_fwd(const LevelArgs& a, bool enc, cudaStream_t st) {
     if (a.C < 1 || a.C > LGAE_MAX_CHANNELS || a.Cout < 1 || a.Cout > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
-    if (!enc) return dec_pair_loop() ? launch_level_fwd<false, 1, 3, false>(a, st) : launch_level_fwd<false, 1, 3, true>(a, st);
+    if (!enc) return launch_level_fwd<false, 1, 3, true>(a, st);   // closed form
     if (a.r_save) return launch_level_fwd<true, 1, 3, true>(a, st);   // radial weights precomputed (N <= 32)
     const int nt = (4 * a.C + 7) / 8, ks = pick_ks(a.K);
     if (ks < 0) return LGAE_E_UNSUPPORTED;

@@ -236,7 +236,7 @@ LGAE_DEV void rad_fetch(const RadialArgs& a, const unsigned char* ti, const unsi
 }
 
 template <int NT, int KS>
-LGAE_DEV void radial_bwd_body(const RadialArgs& a) {
+__global__ void __launch_bounds__(128, LGAE_RBWD_CTAS) radial_bwd_kernel(const RadialArgs a) {
     constexpr int KP = 4 * KS;
     constexpr int NT2 = KS / 2 + 1;
     constexpr int NK = 8 * NT2, NCOL = 8 * NT;
@@ -358,15 +358,6 @@ LGAE_DEV void radial_bwd_body(const RadialArgs& a) {
     }
 }
 
-template <int NT, int KS>
-__global__ void __launch_bounds__(128, LGAE_RBWD_CTAS) radial_bwd_kernel(const RadialArgs a) {
-    radial_bwd_body<NT, KS>(a);
-}
-template <int NT, int KS>
-__global__ void __launch_bounds__(128, LGAE_RBWD_CTAS) radial_bwd_multi_kernel(const RadialMultiArgs m) {
-    radial_bwd_body<NT, KS>(m.lv[blockIdx.y]);
-}
-
 // ------------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------------
@@ -454,8 +445,11 @@ int run_radial_fwd_all(const LgaeModelDesc* d, const double* theta, const double
 int64_t radial_part_width(const LgaeModelDesc* d, int level) { return (int64_t)4 * d->channels[level] * (d->n_basis + 1) + 3 * d->n_basis; }
 
 // Adjoint: g_r (B,N,C,32,4) -> partial rows for a, b, c, linear.{0,1}.{weight,bias} of the level.
-static int prep_radial_bwd(RadialArgs& a, const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask,
-                           int batch, const double* g_r, const double* nrm, PartPlan* plan) {
+int run_radial_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
+                   const double* g_r, const double* nrm, PartPlan* plan, cudaStream_t st) {
+    if (!d || d->is_decoder || level < 0 || level >= d->n_levels || !g_r || !nrm || !plan) return LGAE_E_BADARG;
+    if (batch <= 0) return LGAE_OK;
+    RadialArgs a;
     fill(a, d, level, theta, p4, node_mask, batch);
     a.g_r = g_r;
     a.nrm = const_cast<double*>(nrm);
@@ -476,42 +470,8 @@ static int prep_radial_bwd(RadialArgs& a, const LgaeModelDesc* d, int level, con
     seg(a.off_w0, a.po_w0, (int64_t)2 * C * K); seg(a.off_b0, a.po_b0, 2 * C);
     seg(a.off_w1, a.po_w1, (int64_t)2 * C * K); seg(a.off_b1, a.po_b1, 2 * C);
     seg(a.off_a, a.po_a, K); seg(a.off_b, a.po_b, K); seg(a.off_c, a.po_c, K);
-    return rc;
-}
-int run_radial_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
-                   const double* g_r, const double* nrm, PartPlan* plan, cudaStream_t st) {
-    if (!d || d->is_decoder || level < 0 || level >= d->n_levels || !g_r || !nrm || !plan) return LGAE_E_BADARG;
-    if (batch <= 0) return LGAE_OK;
-    RadialArgs a;
-    if (int rc = prep_radial_bwd(a, d, level, theta, p4, node_mask, batch, g_r, nrm, plan)) return rc;
+    if (rc != LGAE_OK) return rc;
     return dispatch_radial(a, true, st);
-}
-// Whether run_radial_fwd_all / run_radial_bwd_all can serve this model (same MMA tiling on every level).
-bool radial_all_supported(const LgaeModelDesc* d) {
-    if (!d || d->is_decoder || d->n_particles > RAD_MAXN || pick_ks(d->n_basis) < 0) return false;
-    for (int l = 0; l < d->n_levels; ++l) {
-        if (d->channels[l] < 1 || d->channels[l] > LGAE_MAX_CHANNELS) return false;
-        if ((4 * d->channels[l] + 7) / 8 != (4 * d->channels[0] + 7) / 8) return false;
-    }
-    return true;
-}
-// The adjoints of all levels in one launch, after the last level adjoint has written its dL/dR.
-int run_radial_bwd_all(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
-                       const double* const* g_r, const double* nrm, PartPlan* plan, cudaStream_t st) {
-    if (!radial_all_supported(d) || !g_r || !nrm || !plan) return LGAE_E_UNSUPPORTED;
-    if (batch <= 0) return LGAE_OK;
-    RadialMultiArgs m;
-    for (int l = 0; l < d->n_levels; ++l)
-        if (int rc = prep_radial_bwd(m.lv[l], d, l, theta, p4, node_mask, batch, g_r[l], nrm, plan)) return rc;
-    const int nt = (4 * d->channels[0] + 7) / 8, ks = pick_ks(d->n_basis);
-    LaunchScope ls_("radial_bwd", st);
-#define LGAE_CASE(NTV, KSV) \
-    if (nt == NTV && ks == KSV) { launch_k(radial_bwd_multi_kernel<NTV, KSV>, dim3(radial_grid(), d->n_levels), dim3(128), 0, st, m); return check_launch("radial_bwd"); }
-    LGAE_CASE(1, 3) LGAE_CASE(2, 3) LGAE_CASE(3, 3) LGAE_CASE(4, 3)
-    LGAE_CASE(1, 5) LGAE_CASE(2, 5) LGAE_CASE(3, 5) LGAE_CASE(4, 5)
-    LGAE_CASE(1, 8) LGAE_CASE(2, 8) LGAE_CASE(3, 8) LGAE_CASE(4, 8)
-#undef LGAE_CASE
-    return LGAE_E_UNSUPPORTED;
 }
 
 }  // namespace lgae

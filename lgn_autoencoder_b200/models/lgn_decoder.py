@@ -4,7 +4,6 @@ Reference behaviours kept on purpose (SURVEY.md appendix A.6): the decoder's nod
 radial functions reduce to their Linear biases; the zonal (0,0) function is 1+1j; the latent scalars never reach
 the output."""
 import logging
-import os
 
 import torch
 
@@ -121,7 +120,7 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         zf_in, _, _ = self.zonal_fns_in(node_ps)
         node = self.input_func_node(zf_in)
         dec_nodes = [node]
-        if os.environ.get("LGAE_DEC_PAIRLOOP") == "1" or any(z != 1 for z in self.max_zf):
+        if any(z != 1 for z in self.max_zf):
             # the reference's O(N^2) form: pairwise zonal functions, (masked-out) radial functions, edge features, aggregation
             b, n = node_ps.shape[1], node_ps.shape[2]
             node_mask = torch.zeros(2, b, n, dtype=torch.float32, device=node_ps.device)     # lgn_decoder.py:335-340

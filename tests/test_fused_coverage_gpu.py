@@ -83,17 +83,17 @@ def cap_batch(sm_count):
 # ---------------------------------------------------------------------------------------------------------------------
 def mma_nt(c):
     """N-tiles of 8 columns of the radial MMA: 4 outputs (2 radial functions x complex) per channel.
-    lgae_radial.cu dispatch_radial (:402) and lgae_level.cu dispatch_level_fwd (:1078): nt = (4 * C + 7) / 8."""
+    lgae_radial.cu dispatch_radial (:393) and lgae_level.cu dispatch_level_fwd (:1004): nt = (4 * C + 7) / 8."""
     return (4 * c + 7) // 8
 
 
 def pick_ks(k):
-    """k-steps of the radial MMA for K = 2 * num_basis_fn columns: lgae_radial.cu:373, lgae_level.cu:1021."""
+    """k-steps of the radial MMA for K = 2 * num_basis_fn columns: lgae_radial.cu:364, lgae_level.cu:956."""
     return 3 if k <= 12 else (5 if k <= 20 else (8 if k <= 32 else None))
 
 
 def level_bwd_branch(c):
-    """Block size of the level adjoint: lgae_level.cu launch_level_bwd (:1057-1063): C <= 3 and C == 4 at 128 threads with their
+    """Block size of the level adjoint: lgae_level.cu launch_level_bwd (:984-989): C <= 3 and C == 4 at 128 threads with their
     own occupancy hints, C >= 5 at 256 threads."""
     return "c<=3" if c <= 3 else ("c==4" if c == 4 else "c>=5")
 
@@ -169,7 +169,7 @@ def test_config_tables_reach_every_specialisation():
     # get_real
     from lgn_autoencoder_b200.fused import GET_REAL_MODES
     assert set(GET_REAL) == set(GET_REAL_MODES)
-    # past the cap: 4 CTAs per SM (lgae_glue.cu glue_grid :1134, lgae_level.cu level_bwd_grid :1069)
+    # past the cap: 4 CTAs per SM (lgae_glue.cu glue_grid :1134, lgae_level.cu level_bwd_grid :995)
     assert cap_batch(148) > 4 * 148
     widest = [max(cfg["enc_channels"] + cfg["dec_channels"]) for cfg in CAP_CASES.values()]
     assert min(widest) <= 3 and max(widest) >= 5
@@ -333,7 +333,7 @@ def test_forward_more_than_32_particles_matches_oracle(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(CAP_CASES))
 def test_batch_past_the_persistent_grid(name):
-    """Batch 4 * SMs + 37: the level adjoint (lgae_level.cu level_bwd_kernel, jet loop :656) and the glue adjoints
+    """Batch 4 * SMs + 37: the level adjoint (lgae_level.cu level_bwd_kernel, jet loop :644) and the glue adjoints
     (lgae_glue.cu enc_latent_bwd_kernel :379, dec_input_bwd_kernel :540, latent_bridge_bwd_kernel :553) loop over more jets than they have CTAs, so some CTAs take a second jet and
     carry their gradient partials across it.  FusedTrainStep on the full batch against the oracle (gradients included), and
     against the same jets in chunks below the cap: per-jet reconstruction and loss bit-identical, gradient sums within 1e-11."""

@@ -85,16 +85,3 @@ def test_loss_and_gradients_match_reference(name):
         print(name, nm, [(k, f"{e[0]:.1e}", f"{e[1]:.1e}") for k, e in worst])
     assert_grads_close(mine_d, g["grads_dec"])
     assert_grads_close(mine_e, g["grads_enc"])
-
-
-def test_decoder_pair_loop_variant_matches_reference():
-    """The decoder levels default to the O(N) closed form; LGAE_DEC_PAIRLOOP=1 selects the reference-shaped O(N^2)
-    neighbour loop.  Both must reproduce the golden vectors (the flag is read once per process => subprocess)."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, LGAE_DEC_PAIRLOOP="1")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", os.path.join(root, "tests", "test_fused_gpu.py"),
-                        "-k", "matches_reference and not pair_loop"], env=env, cwd=root, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]

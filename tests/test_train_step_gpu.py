@@ -338,26 +338,26 @@ def test_peer_allreduce_single_rank_and_split_step():
     l0 = step.step(batch["p4"]).item()
     g0 = step.g_all.clone()
     step.g_all.zero_()
-    if lib.lgae_aux_stream():
-        pe, pd = step.pe, step.pd
-        th_e, _ = enc._flat_params()
-        th_d, _ = dec._flat_params()
-        for phase in (1, 2):
-            check(lib.lgae_train_step(C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(step.p4_in), ptr(step.mask), step.B, 0,
-                                      ptr(step.p4), ptr(step.norm_factor), ptr(step.ws_e), ptr(step.ws_d), ptr(step.latent00), ptr(step.latent11),
-                                      ptr(step.sel), ptr(step.recon), ptr(step.g_recon), ptr(step.g_lat11), ptr(step.jet_loss), ptr(step.loss),
-                                      ptr(step.g_all), step.off_d, ptr(step.part), step.l1, step.get_real, phase, st), "train_step phase")
-            if phase == 1:   # the decoder's bucket is final on the auxiliary stream
-                aux = torch.cuda.ExternalStream(int(lib.lgae_aux_stream()), device=dev)
-                aux.synchronize()
-                assert torch.equal(step.g_d, g0[step.off_d:])
-        torch.cuda.synchronize()
-        assert step.loss.item() == l0 and torch.equal(step.g_all, g0)
-        # phase 2 without phase 1 is refused
-        assert lib.lgae_train_step(C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(step.p4_in), ptr(step.mask), step.B, 0,
-                                   ptr(step.p4), ptr(step.norm_factor), ptr(step.ws_e), ptr(step.ws_d), ptr(step.latent00), ptr(step.latent11),
-                                   ptr(step.sel), ptr(step.recon), ptr(step.g_recon), ptr(step.g_lat11), ptr(step.jet_loss), ptr(step.loss),
-                                   ptr(step.g_all), step.off_d, ptr(step.part), step.l1, step.get_real, 2, st) == -1
+    assert lib.lgae_aux_stream(), lib.lgae_last_cuda_error()
+    pe, pd = step.pe, step.pd
+    th_e, _ = enc._flat_params()
+    th_d, _ = dec._flat_params()
+    for phase in (1, 2):
+        check(lib.lgae_train_step(C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(step.p4_in), ptr(step.mask), step.B, 0,
+                                  ptr(step.p4), ptr(step.norm_factor), ptr(step.ws_e), ptr(step.ws_d), ptr(step.latent00), ptr(step.latent11),
+                                  ptr(step.sel), ptr(step.recon), ptr(step.g_recon), ptr(step.g_lat11), ptr(step.jet_loss), ptr(step.loss),
+                                  ptr(step.g_all), step.off_d, ptr(step.part), step.l1, step.get_real, phase, st), "train_step phase")
+        if phase == 1:   # the decoder's bucket is final on the auxiliary stream
+            aux = torch.cuda.ExternalStream(int(lib.lgae_aux_stream()), device=dev)
+            aux.synchronize()
+            assert torch.equal(step.g_d, g0[step.off_d:])
+    torch.cuda.synchronize()
+    assert step.loss.item() == l0 and torch.equal(step.g_all, g0)
+    # phase 2 without phase 1 is refused
+    assert lib.lgae_train_step(C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(step.p4_in), ptr(step.mask), step.B, 0,
+                               ptr(step.p4), ptr(step.norm_factor), ptr(step.ws_e), ptr(step.ws_d), ptr(step.latent00), ptr(step.latent11),
+                               ptr(step.sel), ptr(step.recon), ptr(step.g_recon), ptr(step.g_lat11), ptr(step.jet_loss), ptr(step.loss),
+                               ptr(step.g_all), step.off_d, ptr(step.part), step.l1, step.get_real, 2, st) == -1
 
 
 def test_bench_dump_outputs_are_the_timed_step_results(tmp_path):

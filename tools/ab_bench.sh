@@ -1,5 +1,6 @@
 #!/bin/bash
-# Developer: A/B of environment knobs on the bench step.  usage: tools/ab_bench.sh "VAR=val VAR2=val" ...
+# Developer: A/B of library builds on the bench step (tools/build_variant.sh builds them).
+# usage: tools/ab_bench.sh "LGAE_B200_LIB=tools/variants/a.so" "LGAE_B200_LIB=tools/variants/b.so" ...
 for cfg in "$@"; do
   out=$(env $cfg python bench.py --no-extras --no-cpu-baseline --steps 200 2>/dev/null | tail -1)
   python - "$cfg" <<PY
