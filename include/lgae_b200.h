@@ -113,6 +113,12 @@ int64_t lgae_workspace_offset(const LgaeModelDesc* d, int32_t batch, int32_t kin
 /* Doubles of scratch for the per-CTA rows of parameter-gradient partials the backward entry points write (every
  * backward kernel owns a block of compact rows; one reduce launch sums them into gtheta, in a fixed order). */
 int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch);
+/* Doubles of the one caller-allocated scratch buffer of lgae_encoder_backward_tiled / lgae_decoder_backward_tiled: the
+ * adjoints of the neighbour sums (B*N*C*10 complex), the encoder's dL/dR of one level (B * ceil(N/32) * N * C * 128 doubles:
+ * 1.57 GB at B = 512, N = 150, C = 4) and the rows of parameter-gradient partials.  -1 for bad arguments, -2
+ * (LGAE_E_UNSUPPORTED) for a configuration the tiled adjoint cannot run (e.g. a latent or input-map adjoint whose shared
+ * memory does not fit at this particle count).  Needs no GPU. */
+int64_t lgae_backward_tiled_scratch_doubles(const LgaeModelDesc* d, int32_t batch);
 
 /* ---- whole-model entry points -------------------------------------------------------------------- */
 /* LGNEncoder.forward.  p4 (B,N,4) Cartesian (E,px,py,pz); node_mask (B,N) uint8 or NULL (=> p4[...,0] != 0).
@@ -122,22 +128,37 @@ int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch);
 int lgae_encoder_forward(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask,
                          int32_t batch, double* workspace, double* lat00, double* lat11, int32_t* sel, void* stream);
 /* Adjoint.  g_lat00 / g_lat11 may be NULL (treated as zero).  gtheta (n_params) is OVERWRITTEN with the
- * parameter gradient.  partials: scratch of lgae_partials_doubles(d, batch).  Needs N <= 32.
+ * parameter gradient.  partials: scratch of lgae_partials_doubles(d, batch).  Needs N <= 32 (any N: the tiled entry point).
  * l1_lambda != 0 folds the L1 regulariser (lgn_encoder.py:249-250, utils/train.py:483-492) into the same launches:
  * gtheta += l1_lambda sign(theta) and, when loss_accumulate != NULL, loss_accumulate[0] += l1_lambda |theta|_1. */
 int lgae_encoder_backward(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask,
                           int32_t batch, double* workspace, const int32_t* sel, const double* g_lat00,
                           const double* g_lat11, double* gtheta, double* partials, double l1_lambda,
                           double* loss_accumulate, void* stream);
+/* The same adjoint for any N >= 1 (the forward is lgae_encoder_forward unchanged).  It works on blocks of 32 particles and
+ * re-evaluates the radial weights tile by tile instead of reading saved ones; at N <= 32 it runs one block per jet.
+ * scratch: lgae_backward_tiled_scratch_doubles(d, batch) doubles, in place of `partials`; everything else as
+ * lgae_encoder_backward (gtheta overwritten, L1 folded in).  LGAE_E_UNSUPPORTED, before any launch, where the size query
+ * returns -2. */
+int lgae_encoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask,
+                                int32_t batch, double* workspace, const int32_t* sel, const double* g_lat00,
+                                const double* g_lat11, double* gtheta, double* scratch, double l1_lambda,
+                                double* loss_accumulate, void* stream);
 /* LGNDecoder.forward.  lat11 (2,B,1,tau_v,4) planar complex Cartesian.  recon (2,B,N,4); gen00 (2,B,N,1,1) or NULL
  * (NULL: the output scalars are not wanted, the last level's scalar MLP -- which feeds only them -- is then not run;
  * pass g_gen00 = NULL to the backward accordingly). */
 int lgae_decoder_forward(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch,
                          double* workspace, double* recon, double* gen00, void* stream);
-/* g_recon (2,B,N,4); g_gen00 (2,B,N,1,1) or NULL.  g_lat11 (2,B,1,tau_v,4) receives the latent gradient. */
+/* g_recon (2,B,N,4); g_gen00 (2,B,N,1,1) or NULL.  g_lat11 (2,B,1,tau_v,4) receives the latent gradient.  Needs N <= 32 (any N:
+ * the tiled entry point); LGAE_E_UNSUPPORTED before any launch otherwise. */
 int lgae_decoder_backward(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch,
                           double* workspace, const double* g_recon, const double* g_gen00, double* g_lat11,
                           double* gtheta, double* partials, double l1_lambda, double* loss_accumulate, void* stream);
+/* The same adjoint for any N >= 1, with `scratch` (lgae_backward_tiled_scratch_doubles) in place of `partials`; g_lat11
+ * receives the latent gradient.  The closed-form level adjoint runs one CTA per jet over its blocks of 32 particles. */
+int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch,
+                                double* workspace, const double* g_recon, const double* g_gen00, double* g_lat11,
+                                double* gtheta, double* scratch, double l1_lambda, double* loss_accumulate, void* stream);
 
 /* ---- the whole training step ---------------------------------------------------------------------- */
 /* utils/train.py:283-327 in one call: [normalize_p4] -> encoder -> decoder -> chamfer (sum over the batch) of get_real(recon) +

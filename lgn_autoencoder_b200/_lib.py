@@ -104,10 +104,13 @@ _PROTOS = {
     "lgae_workspace_doubles": (C.c_int64, [_D, C.c_int32]),
     "lgae_workspace_offset": (C.c_int64, [_D, C.c_int32, C.c_int32, C.c_int32]),
     "lgae_partials_doubles": (C.c_int64, [_D, C.c_int32]),
+    "lgae_backward_tiled_scratch_doubles": (C.c_int64, [_D, C.c_int32]),
     "lgae_encoder_forward": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P]),
     "lgae_encoder_backward": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
     "lgae_decoder_forward": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P]),
     "lgae_decoder_backward": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
+    "lgae_encoder_backward_tiled": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
+    "lgae_decoder_backward_tiled": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
     "lgae_train_step_partials_doubles": (C.c_int64, [_D, _D, C.c_int32]),
     "lgae_train_step": (C.c_int, [_D, _D, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int64, _P,
                                   C.c_double, C.c_int32, C.c_int32, _P]),

@@ -25,8 +25,15 @@ int run_radial_fwd(const LgaeModelDesc* d, int level, const double* theta, const
                    double* r, double* nrm, cudaStream_t st);
 int run_radial_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
                    const double* g_r, const double* nrm, PartPlan* plan, cudaStream_t st);
+int run_level_bwd_tiled(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
+                        const double* s_in, const double* v_in, const double* sums, double* gA, double* g_r, const double* g_s_pre,
+                        const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st);
+int level_bwd_tiled_check(const LgaeModelDesc* d);
+int64_t level_tiled_part_doubles(const LgaeModelDesc* d, int level, int batch);
+int glue_bwd_check(const LgaeModelDesc* d);
 int64_t radial_nrm_stride(int n);
 int radial_grid();
+int radial_tiled_grid();
 int64_t radial_part_width(const LgaeModelDesc* d, int level);
 int level_bwd_grid(int batch);
 int64_t level_part_width(const LgaeModelDesc* d, int level);
@@ -229,6 +236,32 @@ static int check_desc(const LgaeModelDesc* d) {
     return LGAE_OK;
 }
 
+// Scratch of the tiled adjoint (lgae_backward_tiled_scratch_doubles): [gA | g_r | partial rows + reduce scratch].
+//   gA  (B,N,Cmax,10) complex: adjoints of the neighbour sums of the current level
+//   g_r (B,nib,N,Cmax,32,4), encoder only: dL/dR of the current level's ordered pairs, the only O(N^2) piece
+struct TiledScratch {
+    int64_t gA, gr, part, total;
+};
+static TiledScratch tiled_scratch(const LgaeModelDesc* d, int64_t B) {
+    TiledScratch T;
+    const int64_t N = d->n_particles, cm = max_channels(d), nib = (N + 31) / 32;
+    T.gA = 0;
+    T.gr = T.gA + ((B * N * cm * 20 + 3) & ~int64_t(3));
+    T.part = T.gr + (d->is_decoder ? 0 : B * nib * N * cm * 128);
+    int64_t n = glue_part_doubles(d, (int)B) + reduce_scratch_doubles();
+    for (int l = 0; l < d->n_levels; ++l) {
+        n += level_tiled_part_doubles(d, l, (int)B);
+        if (!d->is_decoder) n += (int64_t)radial_tiled_grid() * radial_part_width(d, l);
+        if (d->has_mlp) n += (int64_t)mlp_bwd_grid() * mlp_part_width(d, l);
+    }
+    T.total = T.part + n;
+    return T;
+}
+static int tiled_check(const LgaeModelDesc* d) {
+    if (int rc = level_bwd_tiled_check(d)) return rc;
+    return glue_bwd_check(d);
+}
+
 // The momenta the encoder kernels read: p4 itself, or (input_scale != 1) the scaled copy kept in the workspace, written here
 // when `write` (forward) and re-used by the adjoint.
 static const double* scaled_input(const LgaeModelDesc* d, const double* p4, int64_t batch, double* ws, bool write, cudaStream_t st, int* rc) {
@@ -334,6 +367,12 @@ int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch) {
     }
     return n;
 }
+int64_t lgae_backward_tiled_scratch_doubles(const LgaeModelDesc* d, int32_t batch) {
+    const int rc = check_desc(d);
+    if (rc == LGAE_E_BADARG || batch < 0) return -1;
+    if (rc != LGAE_OK || tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    return tiled_scratch(d, batch).total;
+}
 
 }  // extern "C"
 
@@ -371,9 +410,10 @@ static int enc_forward_launch(const LgaeModelDesc* d, const double* theta, const
 // Launch sequence of the encoder adjoint; appends its blocks / segments to `plan` (no reduce).
 static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
                                double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, PartPlan& plan,
-                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr) {
+                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr, double* tiled = nullptr) {
     if (batch > 0) {
         const Layout L = layout(d, batch);
+        const TiledScratch T = tiled_scratch(d, batch);
         const int64_t rows = (int64_t)batch * d->n_particles;
         const int nl = d->n_levels;
         int cur = 0;
@@ -391,6 +431,14 @@ static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, cons
                 } else {
                     g_spre = ws + L.gS[cur];
                 }
+            }
+            if (tiled) {   // tiled adjoint: radial weights re-evaluated, dL/dR of every level in one scratch buffer
+                LGAE_TRY(run_level_bwd_tiled(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], tiled + T.gA,
+                                             tiled + T.gr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
+                LGAE_TRY(run_radial_bwd(d, l, theta, p4, node_mask, batch, tiled + T.gr, nullptr, &plan, st));
+                cur ^= 1;
+                gs_zero = false;
+                continue;
             }
             if (L.rsave[l] < 0 || L.gr[l] < 0) return LGAE_E_UNSUPPORTED;
             LGAE_TRY(run_level_bwd(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], ws + L.rsave[l], ws + L.gr[l],
@@ -440,7 +488,7 @@ static int dec_forward_launch(const LgaeModelDesc* d, const double* theta, const
 
 static int dec_backward_launch(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws,
                                const double* g_recon, const double* g_gen00, double* g_lat11, PartPlan& plan, cudaStream_t st,
-                               bool with_output = true, bool with_input = true) {
+                               bool with_output = true, bool with_input = true, double* tiled = nullptr) {
     if (batch > 0) {
         const Layout L = layout(d, batch);
         const int64_t rows = (int64_t)batch * d->n_particles;
@@ -460,8 +508,13 @@ static int dec_backward_launch(const LgaeModelDesc* d, const double* theta, cons
                     g_spre = ws + L.gS[cur];
                 }
             }
-            LGAE_TRY(run_level_bwd(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], nullptr, nullptr, g_spre,
-                                   ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
+            if (tiled)
+                LGAE_TRY(run_level_bwd_tiled(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l],
+                                             tiled + tiled_scratch(d, batch).gA, nullptr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1],
+                                             ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
+            else
+                LGAE_TRY(run_level_bwd(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], nullptr, nullptr, g_spre,
+                                       ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
             cur ^= 1;
             gs_zero = false;
         }
@@ -516,9 +569,37 @@ int lgae_decoder_backward(const LgaeModelDesc* d, const double* theta, const dou
     LGAE_TRY(check_desc(d));
     if (!d->is_decoder || !theta || !gtheta || !partials || batch < 0 || (batch > 0 && (!lat11 || !ws || !g_recon || !g_lat11)))
         return LGAE_E_BADARG;
+    if (d->n_particles > 32) return LGAE_E_UNSUPPORTED;   // before anything is launched: the adjoint holds one particle per lane
     PartPlan plan;
     plan.base = partials;
     LGAE_TRY(dec_backward_launch(d, theta, lat11, batch, ws, g_recon, g_gen00, g_lat11, plan, (cudaStream_t)stream));
+    return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
+}
+
+int lgae_encoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
+                                double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
+                                double* scratch, double l1_lambda, double* loss_accumulate, void* stream) {
+    LGAE_TRY(check_desc(d));
+    if (d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
+    LGAE_TRY(tiled_check(d));
+    PartPlan plan;
+    plan.base = scratch + tiled_scratch(d, batch).part;
+    int rc = LGAE_OK;
+    p4 = scaled_input(d, p4, batch, ws, false, (cudaStream_t)stream, &rc);
+    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream, true, nullptr, scratch));
+    return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
+}
+
+int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws,
+                                const double* g_recon, const double* g_gen00, double* g_lat11, double* gtheta, double* scratch,
+                                double l1_lambda, double* loss_accumulate, void* stream) {
+    LGAE_TRY(check_desc(d));
+    if (!d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!lat11 || !ws || !g_recon || !g_lat11)))
+        return LGAE_E_BADARG;
+    LGAE_TRY(tiled_check(d));
+    PartPlan plan;
+    plan.base = scratch + tiled_scratch(d, batch).part;
+    LGAE_TRY(dec_backward_launch(d, theta, lat11, batch, ws, g_recon, g_gen00, g_lat11, plan, (cudaStream_t)stream, true, true, scratch));
     return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
 }
 

@@ -446,7 +446,7 @@ __global__ void __launch_bounds__(256) latent_bridge_kernel(const LatentArgs a, 
     dec_input_body(d, lat);
 }
 
-// Persistent over jets, one thread per particle (N <= blockDim.x required).
+// Persistent over jets; the threads loop over the particles.
 struct DecInBwdSm { cplx *lat, *gP_s, *gwg, *gin; };
 __device__ __forceinline__ DecInBwdSm dec_input_bwd_init(const DecInArgs& a, double* smem) {
     const int tid = threadIdx.x, N = a.N, C = a.C, tau = a.tau;
@@ -467,8 +467,7 @@ __device__ __forceinline__ void dec_input_bwd_jet(const DecInArgs& a, const DecI
         __syncthreads();
         for (int t = tid; t < tau * 4; t += blockDim.x)
             lat[t] = cmake(a.lat11[(int64_t)(0 * B + b) * tau * 4 + t], a.lat11[(int64_t)(1 * B + b) * tau * 4 + t]);
-        if (tid < N) {
-            const int i = tid;
+        for (int i = tid; i < N; i += blockDim.x) {
             const int64_t node = (int64_t)b * N + i;
             cplx gy[4], y[4];
 #pragma unroll
@@ -1213,7 +1212,6 @@ int run_dec_input_bwd(const LgaeModelDesc* d, const double* theta, int B, const 
                       const double* gy, double* g_lat11, PartPlan* plan, cudaStream_t st) {
     DecInArgs a = dec_in_args(d, theta, B, lat11, y, nullptr, nullptr);
     a.gS = gS; a.gV = gV; a.gy = gy; a.g_lat11 = g_lat11;
-    if (a.N > 128) return LGAE_E_UNSUPPORTED;
     const int grid = glue_grid(B);
     {
         const int64_t ng = (int64_t)2 * a.N * a.tau, w = ng + 4 * a.C, off = plan->block(grid, w);
@@ -1419,4 +1417,14 @@ int run_l1(const double* theta, int64_t n, double lambda, double* out, double* g
     return check_launch("l1");
 }
 
+}  // namespace lgae
+
+namespace lgae {
+// LGAE_OK if the adjoints of the model's input and output maps fit their kernels' shared memory at its particle count (the
+// checks run_enc_latent_bwd / run_dec_input_bwd make before launching), else LGAE_E_UNSUPPORTED.  No GPU needed.
+int glue_bwd_check(const LgaeModelDesc* d) {
+    const size_t n = d->is_decoder ? dec_input_bwd_smem_cplx(d->n_particles, d->channels[0], d->tau_v)
+                                   : enc_latent_bwd_smem_cplx(d->n_particles, d->channels[d->n_levels], d->tau_s, d->tau_v, d->latent_mode);
+    return n * sizeof(cplx) > 200 * 1024 ? LGAE_E_UNSUPPORTED : LGAE_OK;
+}
 }  // namespace lgae

@@ -1079,3 +1079,516 @@ int64_t level_part_width(const LgaeModelDesc* d, int level) {
 }
 
 }  // namespace lgae
+
+// ============================================================================================================
+// Tiled adjoint, any N (lgae_encoder_backward_tiled / lgae_decoder_backward_tiled).  The per-lane adjoint above holds
+// one particle per lane and streams the saved radial weights of every pair, so it stops at 32 particles.  This one
+// works like the N > 32 forward: a CTA of 32 C threads (warp = channel, lane = particle of a block of 32) takes one
+// (jet, particle block) unit at a time, persistent over the units in a fixed order, and the encoder re-evaluates the
+// radial weights tile by tile with radial_tile.  Three kernels per level:
+//   level_bwd_mix_tiled  adjoint of the channel mix -> gA (the adjoints of the 10 neighbour sums, (B,N,C,10) complex) in
+//                        scratch, node and self-product parts of dL/dS, dL/dV, one row of mix-weight partials per CTA;
+//   level_bwd_nbr_tiled  encoder: neighbour loop over partner tiles.  Role 1 writes dL/dR_{i,o} to g_r, laid out as the
+//                        per-lane adjoint's (B,N_o,C,32_i,4) with a block axis: (B, nib, N_o, C, 32_i, 4); role 2 adds the
+//                        neighbour part of dL/dS_i, dL/dV_i (accumulated in partner order) to the mix kernel's values;
+//   level_bwd_cf_tiled   decoder: adjoint of the O(N) closed form, one CTA per jet looping over the blocks.
+// ============================================================================================================
+namespace lgae {
+
+struct TiledMixSmem {
+    int m00, m11, gm, gout;
+    int total;
+};
+__host__ __device__ inline TiledMixSmem tiled_mix_smem(int C, int Cout) {
+    TiledMixSmem s;
+    const int nm = Cout * 5 * C;
+    int o = 0;
+    s.m00 = o; o += 2 * nm;
+    s.m11 = o; o += 2 * nm;
+    s.gm = o; o += 4 * nm;               // [irrep][c'][k] complex accumulators, live for the whole CTA
+    s.gout = o; o += 2 * Cout * 5 * 32;  // incoming gradients of the unit [(c'*5+comp)][32] complex
+    s.total = o;
+    return s;
+}
+
+__global__ void __launch_bounds__(256) level_bwd_mix_tiled(const LevelArgs a, double* gA) {
+    extern __shared__ __align__(128) double smem[];
+    const int N = a.N, C = a.C, Cout = a.Cout, nib = (N + 31) / 32;
+    const int tid = threadIdx.x, lane = tid & 31, c = tid >> 5;
+    const TiledMixSmem L = tiled_mix_smem(C, Cout);
+    cplx* m00_s = reinterpret_cast<cplx*>(smem + L.m00);
+    cplx* m11_s = reinterpret_cast<cplx*>(smem + L.m11);
+    double* gm_d = smem + L.gm;
+    cplx* gout_s = reinterpret_cast<cplx*>(smem + L.gout);
+    const int nm = Cout * 5 * C, C5 = 5 * C;
+
+    pdl_launch();
+    for (int t = tid; t < nm; t += blockDim.x) {
+        m00_s[t] = cmake(a.theta[a.off_m00 + t], a.theta[a.off_m00 + nm + t]);
+        m11_s[t] = cmake(a.theta[a.off_m11 + t], a.theta[a.off_m11 + nm + t]);
+    }
+    for (int t = tid; t < 4 * nm; t += blockDim.x) gm_d[t] = 0.0;
+    pdl_wait();
+    const cplx* gsp = reinterpret_cast<const cplx*>(a.g_s_pre);
+    const cplx* gvo = reinterpret_cast<const cplx*>(a.g_v_out);
+    for (int u = blockIdx.x; u < a.B * nib; u += gridDim.x) {
+        const int b = u / nib, i0 = (u % nib) * 32, i = i0 + lane;
+        const bool live = i < N;
+        const int64_t node = (int64_t)b * N + i;
+        __syncthreads();   // the previous unit's gradients are consumed
+        for (int it = tid; it < 32 * Cout * 5; it += blockDim.x) {
+            const int il = it & 31, r = it >> 5, co = r / 5, comp = r % 5;
+            const int64_t nd = (int64_t)b * N + i0 + il;
+            cplx v = czero();
+            if (i0 + il < N) {
+                if (comp == 0) {
+                    if (gsp) v = gsp[nd * Cout + co];
+                } else {
+                    v = gvo[(nd * Cout + co) * 4 + comp - 1];
+                }
+            }
+            gout_s[r * 32 + il] = v;
+        }
+        cplx A[10], Si = czero(), Vi[4];
+        const cplx* sums = reinterpret_cast<const cplx*>(a.sums) + (node * C + c) * 10;
+#pragma unroll
+        for (int e = 0; e < 10; ++e) A[e] = live ? sums[e] : czero();
+        if (live) Si = reinterpret_cast<const cplx*>(a.s_in)[node * C + c];
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) Vi[mu] = live ? reinterpret_cast<const cplx*>(a.v_in)[(node * C + c) * 4 + mu] : czero();
+        __syncthreads();
+        // the five blocks of the concatenation, as in level_bwd_kernel
+        cplx gS = czero(), gV[4] = {czero(), czero(), czero(), czero()}, gAl[10];
+        cplx cat5[5], gc[5];
+        cat5[0] = cscale(A[9], 0.5);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) cat5[1 + mu] = cmul_1pi(A[mu]);
+        mix_adjoint_block(c, Cout, C5, nm, lane, cat5, gout_s, m00_s, m11_s, gm_d, gc);
+        gAl[9] = cscale(gc[0], 0.5);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) gAl[mu] = cmul_1mi(gc[1 + mu]);
+        cat5[0] = cmul_1pi(A[4]);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) cat5[1 + mu] = A[5 + mu];
+        mix_adjoint_block(C + c, Cout, C5, nm, lane, cat5, gout_s, m00_s, m11_s, gm_d, gc);
+        gAl[4] = cmul_1mi(gc[0]);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) gAl[5 + mu] = gc[1 + mu];
+        cat5[0] = Si;
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) cat5[1 + mu] = Vi[mu];
+        mix_adjoint_block(2 * C + c, Cout, C5, nm, lane, cat5, gout_s, m00_s, m11_s, gm_d, gc);
+        gS = gc[0];
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) gV[mu] = gc[1 + mu];
+        cplx gh[4];
+        cghat(Vi, gh);
+        cat5[0] = cscale(ceta(Vi, Vi), 0.5);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) cat5[1 + mu] = cmul(Vi[mu], Si);
+        mix_adjoint_block(3 * C + c, Cout, C5, nm, lane, cat5, gout_s, m00_s, m11_s, gm_d, gc);
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) {
+            cfmac(gV[mu], gh[mu], gc[0]);
+            cfmac(gV[mu], Si, gc[1 + mu]);
+            cfmac(gS, Vi[mu], gc[1 + mu]);
+        }
+        cat5[0] = cmul(Si, Si);
+        mix_adjoint_block(4 * C + c, Cout, C5, nm, lane, cat5, gout_s, m00_s, m11_s, gm_d, gc);
+        cfmac(gS, Si, cscale(gc[0], 2.0));
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) {
+            cfmac(gV[mu], Si, gc[1 + mu]);
+            cfmac(gS, Vi[mu], gc[1 + mu]);
+        }
+        if (live) {
+            cplx* dst = reinterpret_cast<cplx*>(gA) + (node * C + c) * 10;
+#pragma unroll
+            for (int e = 0; e < 10; ++e) dst[e] = gAl[e];
+            reinterpret_cast<cplx*>(a.g_s_in)[node * C + c] = gS;
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) reinterpret_cast<cplx*>(a.g_v_in)[(node * C + c) * 4 + mu] = gV[mu];
+        }
+    }
+    __syncthreads();
+    double* row = a.part + (int64_t)blockIdx.x * a.part_stride;
+    for (int t = tid; t < nm; t += blockDim.x) {
+        row[a.po_m00 + t] = gm_d[2 * t];
+        row[a.po_m00 + nm + t] = gm_d[2 * t + 1];
+        row[a.po_m11 + t] = gm_d[2 * (nm + t)];
+        row[a.po_m11 + nm + t] = gm_d[2 * (nm + t) + 1];
+    }
+}
+
+struct TiledNbrSmem {
+    int p, msk, abc, S, V, gA, Rs;
+    int total;
+};
+__host__ __device__ inline TiledNbrSmem tiled_nbr_smem(int N, int C, int KS) {
+    TiledNbrSmem s;
+    int o = 0;
+    s.p = o; o += 4 * N;
+    s.msk = o; o += ((N + 7) / 8 + 2) & ~1;
+    s.abc = o; o += (3 * 4 * KS + 1) & ~1;
+    s.S = o; o += 2 * TJ * C;    // the partner tile's node features and neighbour-sum adjoints
+    s.V = o; o += 8 * TJ * C;
+    s.gA = o; o += 20 * TJ * C;
+    o = (o + 3) & ~3;
+    s.Rs = o; o += TJ * C * 32 * 4;   // radial weights of the tile, as radial_tile writes them
+    s.total = o;
+    return s;
+}
+
+template <int NT, int KS>
+__global__ void __launch_bounds__(256) level_bwd_nbr_tiled(const LevelArgs a, const double* gA) {
+    extern __shared__ __align__(128) double smem[];
+    const int N = a.N, C = a.C, nib = (N + 31) / 32;
+    const int tid = threadIdx.x, lane = tid & 31, c = tid >> 5;
+    const TiledNbrSmem L = tiled_nbr_smem(N, C, KS);
+    double* p_s = smem + L.p;
+    uint8_t* msk_s = reinterpret_cast<uint8_t*>(smem + L.msk);
+    double* abc_s = smem + L.abc;
+    cplx* S_s = reinterpret_cast<cplx*>(smem + L.S);
+    cplx* V_s = reinterpret_cast<cplx*>(smem + L.V);
+    cplx* gA_s = reinterpret_cast<cplx*>(smem + L.gA);
+    double* Rs = smem + L.Rs;
+
+    pdl_launch();
+    double wf[KS][NT], bf[NT][2];
+    load_radial_frags<NT, KS>(a, wf, bf, abc_s);
+    pdl_wait();
+    const cplx* gAg = reinterpret_cast<const cplx*>(gA);
+    for (int u = blockIdx.x; u < a.B * nib; u += gridDim.x) {
+        const int b = u / nib, ib = u % nib, i0 = ib * 32, i = i0 + lane;
+        const bool live = i < N;
+        const int64_t node = (int64_t)b * N + i;
+        __syncthreads();   // the previous unit is done with p_s / msk_s
+        const double* pg = a.p + (int64_t)b * N * 4;
+        for (int t = tid; t < 4 * N; t += blockDim.x) p_s[t] = pg[t];
+        for (int t = tid; t < N; t += blockDim.x) msk_s[t] = a.node_mask ? a.node_mask[(int64_t)b * N + t] : (pg[4 * t] != 0.0);
+        double pa[4] = {0, 0, 0, 0};
+        cplx gAa[10], gS = czero(), gV[4];
+#pragma unroll
+        for (int e = 0; e < 10; ++e) gAa[e] = live ? gAg[(node * C + c) * 10 + e] : czero();
+        if (live) {
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) pa[mu] = pg[4 * i + mu];
+            gS = reinterpret_cast<const cplx*>(a.g_s_in)[node * C + c];
+        }
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) gV[mu] = live ? reinterpret_cast<const cplx*>(a.g_v_in)[(node * C + c) * 4 + mu] : czero();
+        double4* grv = reinterpret_cast<double4*>(a.g_r) + ((((int64_t)b * nib + ib) * N) * C + c) * 32 + lane;
+        for (int j0 = 0; j0 < N; j0 += TJ) {
+            const int tj = min(TJ, N - j0);
+            __syncthreads();   // p_s / msk_s staged; the previous tile's buffers are consumed
+            {
+                const int64_t base = (int64_t)b * N + j0;
+                const cplx* sg = reinterpret_cast<const cplx*>(a.s_in) + base * C;
+                const cplx* vg = reinterpret_cast<const cplx*>(a.v_in) + base * C * 4;
+                const cplx* ag = gAg + base * C * 10;
+                const int ns = tj * C;
+                for (int t = tid; t < 15 * ns; t += blockDim.x) {
+                    if (t < ns) S_s[t] = sg[t];
+                    else if (t < 5 * ns) V_s[t - ns] = vg[t - ns];
+                    else gA_s[t - 5 * ns] = ag[t - 5 * ns];
+                }
+            }
+            radial_tile<NT, KS>(p_s, msk_s, N, C, i0, j0, tj, abc_s, wf, bf, Rs);
+            __syncthreads();
+            for (int jj = 0; jj < tj; ++jj) {
+                const int o = j0 + jj;
+                const double4 r = *reinterpret_cast<const double4*>(Rs + ((size_t)((jj * C + c) * 32 + lane)) * 4);
+                const cplx R0 = cmake(r.x, r.y), R1 = cmake(r.z, r.w);
+                const cplx So = S_s[jj * C + c];
+                cplx Vo[4], Y[4];
+#pragma unroll
+                for (int mu = 0; mu < 4; ++mu) Vo[mu] = V_s[(jj * C + c) * 4 + mu];
+                double d[4];
+#pragma unroll
+                for (int mu = 0; mu < 4; ++mu) d[mu] = pa[mu] - p_s[4 * o + mu];
+                canon_from_real(d, Y);
+                const double d0 = Y[0].x, d3 = Y[2].x, ya_ = Y[1].x, yb_ = -Y[1].y;
+                auto ydot = [&](const cplx* gq) {
+                    const cplx dm = csub(gq[1], gq[3]), sp = cadd(gq[1], gq[3]);
+                    return cmake(fma(d0, gq[0].x, fma(d3, gq[2].x, fma(ya_, dm.x, -yb_ * sp.y))),
+                                 fma(d0, gq[0].y, fma(d3, gq[2].y, fma(ya_, dm.y, yb_ * sp.x))));
+                };
+                auto yeta = [&](const cplx* v) {
+                    const cplx vm = csub(v[3], v[1]), vp = cadd(v[1], v[3]);
+                    return cmake(fma(d0, v[0].x, fma(-d3, v[2].x, fma(ya_, vm.x, yb_ * vp.y))),
+                                 fma(d0, v[0].y, fma(-d3, v[2].y, fma(ya_, vm.y, -yb_ * vp.x))));
+                };
+                // role 1: own = receiving node i, other = neighbour o
+                if (live) {
+                    cplx gR0 = czero();
+#pragma unroll
+                    for (int mu = 0; mu < 4; ++mu) cfmac(gR0, Vo[mu], gAa[mu]);
+                    const cplx w = ydot(gAa + 5);
+                    cfmac(gR0, So, gAa[4]);
+                    const cplx e = yeta(Vo);
+                    cplx gR1 = cmulc(So, w);
+                    cfmac(gR1, e, gAa[9]);
+                    grv[(int64_t)o * C * 32] = make_double4(gR0.x, gR0.y, gR1.x, gR1.y);
+                }
+                // role 2: own = neighbour i of the receiving node o.  Y_oi = -Y ; R_oi = R_io.
+                {
+                    const cplx* gAo = gA_s + (jj * C + c) * 10;
+                    cplx Yn[4], gh[4];
+#pragma unroll
+                    for (int mu = 0; mu < 4; ++mu) Yn[mu] = cneg(Y[mu]);
+                    cghat(Yn, gh);
+                    const cplx w = cneg(ydot(gAo + 5));
+                    const cplx r1g = cmulc(R1, gAo[9]);
+#pragma unroll
+                    for (int mu = 0; mu < 4; ++mu) {
+                        cfmac(gV[mu], R0, gAo[mu]);
+                        cfmac(gV[mu], gh[mu], r1g);
+                    }
+                    cfmac(gS, R0, gAo[4]);
+                    cfmac(gS, R1, w);
+                }
+            }
+        }
+        if (live) {
+            reinterpret_cast<cplx*>(a.g_s_in)[node * C + c] = gS;
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) reinterpret_cast<cplx*>(a.g_v_in)[(node * C + c) * 4 + mu] = gV[mu];
+        }
+    }
+}
+
+// Decoder: the closed form's adjoint (see level_bwd_kernel) with the jet-level moments and the 30 jet-level adjoint sums
+// accumulated over the particles lane-strided (particle j in lane j % 32, in increasing j, then one warp butterfly: a
+// fixed order), then the per-particle dL/dS, dL/dV (added to the mix kernel's values) and dL/dy block by block.
+__global__ void __launch_bounds__(256) level_bwd_cf_tiled(const LevelArgs a, const double* gA) {
+    extern __shared__ __align__(128) double smem[];
+    const int N = a.N, C = a.C;
+    const int tid = threadIdx.x, lane = tid & 31, c = tid >> 5;
+    cplx* gy_s = reinterpret_cast<cplx*>(smem);   // [(c*4+mu)][32]
+    pdl_launch();
+    const double b0 = a.theta[a.off_b0 + c], b1 = a.theta[a.off_b1 + c];
+    const cplx R0c = cmake(b0, b0), R1c = cmake(b1, b1);
+    cplx gR0c = czero(), gR1c = czero();
+    pdl_wait();
+    for (int b = blockIdx.x; b < a.B; b += gridDim.x) {
+        const cplx* y_g = reinterpret_cast<const cplx*>(a.p) + (int64_t)b * N * 4;
+        const cplx* S_g = reinterpret_cast<const cplx*>(a.s_in) + (int64_t)b * N * C;
+        const cplx* V_g = reinterpret_cast<const cplx*>(a.v_in) + (int64_t)b * N * C * 4;
+        const cplx* gA_g = reinterpret_cast<const cplx*>(gA) + (int64_t)b * N * C * 10;
+        // jet moments, summed as the forward sums them
+        double m[20];
+#pragma unroll
+        for (int t = 0; t < 20; ++t) m[t] = 0.0;
+        for (int j = lane; j < N; j += 32) {
+            const cplx Sj = S_g[j * C + c];
+            cplx Vj[4], yj[4];
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) { Vj[mu] = V_g[(j * C + c) * 4 + mu]; yj[mu] = y_g[4 * j + mu]; }
+            m[0] += Sj.x; m[1] += Sj.y;
+            const cplx e = ceta(Vj, yj);
+            m[18] += e.x; m[19] += e.y;
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) {
+                m[2 + 2 * mu] += Vj[mu].x; m[3 + 2 * mu] += Vj[mu].y;
+                const cplx sy = cmul(Sj, yj[mu]);
+                m[10 + 2 * mu] += sy.x; m[11 + 2 * mu] += sy.y;
+            }
+        }
+        warp_allsum_n<20>(m);
+        const cplx SS = cmake(m[0], m[1]), SVY = cmake(m[18], m[19]);
+        cplx SV[4], SSY[4], ghsv[4];
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) { SV[mu] = cmake(m[2 + 2 * mu], m[3 + 2 * mu]); SSY[mu] = cmake(m[10 + 2 * mu], m[11 + 2 * mu]); }
+        cghat(SV, ghsv);
+        // jet-level sums: [sum gA0V (4) | sum gA0S | sum gT (4) | sum gU | sum conj(y) gT | sum conj(ghat(y)) gU (4)]
+        double r[30];
+#pragma unroll
+        for (int t = 0; t < 30; ++t) r[t] = 0.0;
+        for (int i = lane; i < N; i += 32) {
+            cplx ya[4], gAa[10];
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) ya[mu] = y_g[4 * i + mu];
+#pragma unroll
+            for (int e = 0; e < 10; ++e) gAa[e] = gA_g[(i * C + c) * 10 + e];
+            const cplx gU = cmulc(R1c, gAa[9]);
+            cplx gr0 = cmulc(SS, gAa[4]);
+            const cplx U = csub(ceta(SV, ya), SVY);
+            cplx gr1 = cmulc(U, gAa[9]);
+            cplx yt = czero();
+            cplx ghy[4];
+            cghat(ya, ghy);
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) {
+                const cplx gT = cmulc(R1c, gAa[5 + mu]);
+                cfmac(gr0, SV[mu], gAa[mu]);
+                const cplx T = csub(cmul(ya[mu], SS), SSY[mu]);
+                cfmac(gr1, T, gAa[5 + mu]);
+                cfmac(yt, ya[mu], gT);
+                r[2 * mu] += gAa[mu].x; r[2 * mu + 1] += gAa[mu].y;
+                r[10 + 2 * mu] += gT.x; r[11 + 2 * mu] += gT.y;
+                const cplx t = cmulc(ghy[mu], gU);
+                r[22 + 2 * mu] += t.x; r[23 + 2 * mu] += t.y;
+            }
+            r[8] += gAa[4].x; r[9] += gAa[4].y;
+            r[18] += gU.x; r[19] += gU.y;
+            r[20] += yt.x; r[21] += yt.y;
+            gR0c = cadd(gR0c, gr0);
+            gR1c = cadd(gR1c, gr1);
+        }
+        warp_allsum_n<30>(r);
+        cplx gSS = cmulc(R0c, cmake(r[8], r[9]));
+        gSS = cadd(gSS, cmake(r[20], r[21]));
+        const cplx gSVY = cneg(cmake(r[18], r[19]));
+        cplx gSVm[4], gSSYm[4];
+#pragma unroll
+        for (int mu = 0; mu < 4; ++mu) {
+            gSVm[mu] = cadd(cmulc(R0c, cmake(r[2 * mu], r[2 * mu + 1])), cmake(r[22 + 2 * mu], r[23 + 2 * mu]));
+            gSSYm[mu] = cneg(cmake(r[10 + 2 * mu], r[11 + 2 * mu]));
+        }
+        for (int i0 = 0; i0 < N; i0 += 32) {
+            const int i = i0 + lane;
+            const bool live = i < N;
+            cplx gy[4] = {czero(), czero(), czero(), czero()};
+            if (live) {
+                cplx ya[4], Va[4], ghy[4], ghv[4];
+                const cplx Sa = S_g[i * C + c], gU = cmulc(R1c, gA_g[(i * C + c) * 10 + 9]);
+#pragma unroll
+                for (int mu = 0; mu < 4; ++mu) { ya[mu] = y_g[4 * i + mu]; Va[mu] = V_g[(i * C + c) * 4 + mu]; }
+                cghat(ya, ghy);
+                cghat(Va, ghv);
+                cplx* gs_d = reinterpret_cast<cplx*>(a.g_s_in) + ((int64_t)b * N + i) * C + c;
+                cplx* gv_d = reinterpret_cast<cplx*>(a.g_v_in) + (((int64_t)b * N + i) * C + c) * 4;
+                cplx gSa = gSS;
+#pragma unroll
+                for (int mu = 0; mu < 4; ++mu) {
+                    cfmac(gSa, ya[mu], gSSYm[mu]);
+                    cplx gv = gSVm[mu];
+                    cfmac(gv, ghy[mu], gSVY);
+                    gv_d[mu] = cadd(gv_d[mu], gv);
+                    cplx g = cmulc(SS, cmulc(R1c, gA_g[(i * C + c) * 10 + 5 + mu]));
+                    cfmac(g, ghsv[mu], gU);
+                    cfmac(g, Sa, gSSYm[mu]);
+                    cfmac(g, ghv[mu], gSVY);
+                    gy[mu] = g;
+                }
+                *gs_d = cadd(*gs_d, gSa);
+            }
+#pragma unroll
+            for (int mu = 0; mu < 4; ++mu) gy_s[(c * 4 + mu) * 32 + lane] = gy[mu];
+            __syncthreads();
+            const int nb = min(32, N - i0);
+            for (int t = tid; t < 4 * nb; t += blockDim.x) {
+                const int il = t >> 2, mu = t & 3;
+                cplx* dst = reinterpret_cast<cplx*>(a.g_y) + ((int64_t)b * N + i0 + il) * 4 + mu;
+                cplx acc = *dst;
+                for (int cc = 0; cc < C; ++cc) acc = cadd(acc, gy_s[(cc * 4 + mu) * 32 + il]);   // fixed order: deterministic
+                *dst = acc;
+            }
+            __syncthreads();
+        }
+    }
+    double* row = a.part + (int64_t)blockIdx.x * a.part_stride;
+    const double v0 = warp_sum(gR0c.x + gR0c.y), v1 = warp_sum(gR1c.x + gR1c.y);
+    if (lane == 0) {
+        row[a.po_b0 + c] = v0;
+        row[a.po_b1 + c] = v1;
+    }
+}
+
+// ---- host side of the tiled adjoint ----
+#define LGAE_TRY(expr)                  \
+    do {                                \
+        const int rc_ = (expr);         \
+        if (rc_ != LGAE_OK) return rc_; \
+    } while (0)
+
+static int level_tiled_check(const LevelArgs& a, bool enc, size_t* nbr_bytes) {
+    if (a.C < 1 || a.C > LGAE_MAX_CHANNELS || a.Cout < 1 || a.Cout > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
+    if ((size_t)tiled_mix_smem(a.C, a.Cout).total * sizeof(double) > 227 * 1024) return LGAE_E_UNSUPPORTED;
+    if (!enc) return 2 * 4 * 32 * a.C * sizeof(double) > 227 * 1024 ? LGAE_E_UNSUPPORTED : LGAE_OK;
+    const int ks = pick_ks(a.K);
+    if (ks < 0) return LGAE_E_UNSUPPORTED;
+    const size_t bytes = (size_t)tiled_nbr_smem(a.N, a.C, ks).total * sizeof(double);
+    if (bytes > 227 * 1024) return LGAE_E_UNSUPPORTED;
+    if (nbr_bytes) *nbr_bytes = bytes;
+    return LGAE_OK;
+}
+
+// LGAE_OK if the tiled adjoint runs every level of the model, else LGAE_E_UNSUPPORTED (no GPU needed).
+int level_bwd_tiled_check(const LgaeModelDesc* d) {
+    for (int l = 0; l < d->n_levels; ++l) {
+        LevelArgs a;
+        fill_level_args(a, d, l, nullptr, nullptr, nullptr, 1, nullptr, nullptr, nullptr, nullptr);
+        if (int rc = level_tiled_check(a, !d->is_decoder, nullptr)) return rc;
+    }
+    return LGAE_OK;
+}
+
+// Width (doubles) of the partial rows of one level of the tiled adjoint, over all its kernels.
+int64_t level_tiled_part_doubles(const LgaeModelDesc* d, int level, int batch) {
+    const int C = d->channels[level], Cout = d->channels[level + 1], nib = (d->n_particles + 31) / 32;
+    int64_t n = (int64_t)level_bwd_grid(batch * nib) * 4 * Cout * 5 * C;
+    if (d->is_decoder) n += (int64_t)level_bwd_grid(batch) * 2 * C;
+    return n;
+}
+
+// Adjoint of one level for any N.  gA: (B,N,C,10) complex scratch; g_r (encoder): (B, nib, N, C, 32, 4) scratch of dL/dR,
+// for run_radial_bwd with nrm == NULL.  Reserves blocks of `plan` for the partial rows and declares their segments.
+int run_level_bwd_tiled(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
+                        const double* s_in, const double* v_in, const double* sums, double* gA, double* g_r, const double* g_s_pre,
+                        const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st) {
+    if (!d || level < 0 || level >= d->n_levels || !plan || !gA) return LGAE_E_BADARG;
+    if (batch <= 0) return LGAE_OK;
+    const bool enc = !d->is_decoder;
+    if (enc ? !g_r : !g_y) return LGAE_E_BADARG;
+    LevelArgs a;
+    fill_level_args(a, d, level, theta, p_or_y, node_mask, batch, s_in, v_in, const_cast<double*>(sums), nullptr);
+    a.r_save = nullptr;
+    a.g_r = g_r;
+    a.g_s_pre = g_s_pre; a.g_v_out = g_v_out; a.g_s_in = g_s_in; a.g_v_in = g_v_in; a.g_y = g_y;
+    size_t nbr_bytes = 0;
+    LGAE_TRY(level_tiled_check(a, enc, &nbr_bytes));
+    const int C = a.C, nm2 = 2 * a.Cout * 5 * C, nib = (a.N + 31) / 32;
+    const int grid = level_bwd_grid(batch * nib);
+    {   // channel mix: rows [m00 | m11]
+        const int64_t w = 2 * (int64_t)nm2, off = plan->block(grid, w);
+        a.part = plan->base + off; a.part_stride = w; a.po_m00 = 0; a.po_m11 = nm2;
+        LGAE_TRY(plan->seg(a.off_m00, off, w, 0, nm2, grid));
+        LGAE_TRY(plan->seg(a.off_m11, off, w, nm2, nm2, grid));
+        const size_t bytes = (size_t)tiled_mix_smem(C, a.Cout).total * sizeof(double);
+        LGAE_TRY(ensure_smem((const void*)level_bwd_mix_tiled, bytes));
+        LaunchScope ls_("level_bwd_mix_tiled", st);
+        launch_k(level_bwd_mix_tiled, dim3(grid), dim3(32 * C), bytes, st, a, gA);
+        LGAE_TRY(check_launch("level_bwd_mix_tiled"));
+    }
+    if (enc) {
+        const int nt = (4 * C + 7) / 8, ks = pick_ks(a.K);
+        LaunchScope ls_("level_bwd_nbr_tiled", st);
+#define LGAE_CASE(NTV, KSV)                                                                      \
+    if (nt == NTV && ks == KSV) {                                                                \
+        auto kern = level_bwd_nbr_tiled<NTV, KSV>;                                               \
+        LGAE_TRY(ensure_smem((const void*)kern, nbr_bytes));                               \
+        launch_k(kern, dim3(grid), dim3(32 * C), nbr_bytes, st, a, (const double*)gA);           \
+        return check_launch("level_bwd_nbr_tiled");                                              \
+    }
+        LGAE_CASE(1, 3) LGAE_CASE(2, 3) LGAE_CASE(3, 3) LGAE_CASE(4, 3)
+        LGAE_CASE(1, 5) LGAE_CASE(2, 5) LGAE_CASE(3, 5) LGAE_CASE(4, 5)
+        LGAE_CASE(1, 8) LGAE_CASE(2, 8) LGAE_CASE(3, 8) LGAE_CASE(4, 8)
+#undef LGAE_CASE
+        return LGAE_E_UNSUPPORTED;
+    }
+    {   // decoder closed form: rows [b0 | b1]
+        const int gj = level_bwd_grid(batch);
+        const int64_t w = 2 * C, off = plan->block(gj, w);
+        a.part = plan->base + off; a.part_stride = w; a.po_b0 = 0; a.po_b1 = C;
+        LGAE_TRY(plan->seg(a.off_b0, off, w, 0, C, gj));
+        LGAE_TRY(plan->seg(a.off_b1, off, w, C, C, gj));
+        const size_t bytes = (size_t)2 * 4 * 32 * C * sizeof(double);
+        LGAE_TRY(ensure_smem((const void*)level_bwd_cf_tiled, bytes));
+        LaunchScope ls_("level_bwd_cf_tiled", st);
+        launch_k(level_bwd_cf_tiled, dim3(gj), dim3(32 * C), bytes, st, a, (const double*)gA);
+        return check_launch("level_bwd_cf_tiled");
+    }
+}
+
+}  // namespace lgae

@@ -442,18 +442,22 @@ int run_radial_fwd_all(const LgaeModelDesc* d, const double* theta, const double
     return LGAE_E_UNSUPPORTED;
 }
 
+static int dispatch_radial_bwd_tiled(const RadialArgs& a, cudaStream_t st);
+int radial_tiled_grid();
+
 int64_t radial_part_width(const LgaeModelDesc* d, int level) { return (int64_t)4 * d->channels[level] * (d->n_basis + 1) + 3 * d->n_basis; }
 
-// Adjoint: g_r (B,N,C,32,4) -> partial rows for a, b, c, linear.{0,1}.{weight,bias} of the level.
+// Adjoint: g_r (B,N,C,32,4) -> partial rows for a, b, c, linear.{0,1}.{weight,bias} of the level.  nrm == NULL: any N, g_r in the
+// tiled adjoint's blocked layout (B, nib, N, C, 32, 4), the norms recomputed from p4 (radial_bwd_tiled_kernel).
 int run_radial_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
                    const double* g_r, const double* nrm, PartPlan* plan, cudaStream_t st) {
-    if (!d || d->is_decoder || level < 0 || level >= d->n_levels || !g_r || !nrm || !plan) return LGAE_E_BADARG;
+    if (!d || d->is_decoder || level < 0 || level >= d->n_levels || !g_r || !plan) return LGAE_E_BADARG;
     if (batch <= 0) return LGAE_OK;
     RadialArgs a;
     fill(a, d, level, theta, p4, node_mask, batch);
     a.g_r = g_r;
     a.nrm = const_cast<double*>(nrm);
-    const int C = a.C, K = a.K, grid = radial_grid();
+    const int C = a.C, K = a.K, grid = nrm ? radial_grid() : radial_tiled_grid();
     int64_t w = 0;
     a.po_w0 = w; w += (int64_t)2 * C * K;
     a.po_b0 = w; w += 2 * C;
@@ -471,7 +475,208 @@ int run_radial_bwd(const LgaeModelDesc* d, int level, const double* theta, const
     seg(a.off_w1, a.po_w1, (int64_t)2 * C * K); seg(a.off_b1, a.po_b1, 2 * C);
     seg(a.off_a, a.po_a, K); seg(a.off_b, a.po_b, K); seg(a.off_c, a.po_c, K);
     if (rc != LGAE_OK) return rc;
-    return dispatch_radial(a, true, st);
+    return nrm ? dispatch_radial(a, true, st) : dispatch_radial_bwd_tiled(a, st);
+}
+
+}  // namespace lgae
+
+// ============================================================================================================
+// Adjoint for any N (tiled level adjoint): the math of radial_bwd_kernel, with three differences.  The pair index is decoded
+// arithmetically (the unsigned char tables above hold 32 particles), the norms are recomputed from p4 (there is no nrm
+// record past 32 particles), and dL/dR is read from the blocked layout (B, nib, N_o, C, 32_i, 4) of level_bwd_nbr_tiled.
+// ============================================================================================================
+namespace lgae {
+
+// Resident CTAs per SM (register cap 255: at 3, i.e. 168 registers, the wider tilings spill the decoded pair indices).
+constexpr int RAD_TILED_CTAS = 2;
+int radial_tiled_grid() { return RAD_TILED_CTAS * sm_count(); }   // CTAs = rows of partials
+
+// unordered pair p = j (j + 1) / 2 + i (i <= j) -> (i, j)
+LGAE_DEV void pair_decode(int p, int& i, int& j) {
+    int t = (int)((__dsqrt_rn(8.0 * p + 1.0) - 1.0) * 0.5);
+    while (t * (t + 1) / 2 > p) --t;
+    while ((t + 1) * (t + 2) / 2 <= p) ++t;
+    j = t;
+    i = p - t * (t + 1) / 2;
+}
+
+template <int NT>
+LGAE_DEV void rad_fetch_tiled(const RadialArgs& a, int unit, int NU, int NP, const int (&col_cc)[NT], const int (&col_x)[NT], int lane,
+                              RadOperands<NT>& op) {
+    const int N = a.N, C = a.C, q = lane & 3, nib = (N + 31) / 32;
+    const int b = unit / NU, p0 = (unit - b * NU) * RAD_UNIT;
+    const double* gb = a.g_r + (int64_t)b * nib * N * C * 128;
+    const double* pb = a.p4 + (int64_t)b * N * 4;
+    {   // norm of pair p0 + (lane & 15) as the forward evaluates it; NaN = masked edge or padding
+        const int pid = p0 + (lane & 15);
+        double n = __longlong_as_double(0x7ff8000000000000LL);
+        if (pid < NP) {
+            int i, j;
+            pair_decode(pid, i, j);
+            const double4 pi = *reinterpret_cast<const double4*>(pb + 4 * i);
+            const double4 pj = *reinterpret_cast<const double4*>(pb + 4 * j);
+            const double vi[4] = {pi.x, pi.y, pi.z, pi.w}, vj[4] = {pj.x, pj.y, pj.z, pj.w};
+            const double nn = rad_pair_norm(vi, vj);
+            const bool mi = a.node_mask ? a.node_mask[(int64_t)b * N + i] != 0 : pi.x != 0.0;
+            const bool mj = a.node_mask ? a.node_mask[(int64_t)b * N + j] != 0 : pj.x != 0.0;
+            if (mi && mj && nn != 0.0) n = nn;
+        }
+        op.n = n;
+    }
+    // dL/dR of receiving node r, partner s
+    auto at = [&](int r, int s, int cc, int x) { return gb[((((int64_t)(r >> 5) * N + s) * C + cc) * 32 + (r & 31)) * 4 + x]; };
+#pragma unroll
+    for (int u = 0; u < 2; ++u)
+#pragma unroll
+        for (int ks = 0; ks < 2; ++ks) {
+            const int pid = p0 + 8 * u + q + 4 * ks;
+            const bool valid = pid < NP;
+            int i = 0, j = 0;
+            if (valid) pair_decode(pid, i, j);
+#pragma unroll
+            for (int mt = 0; mt < NT; ++mt) {
+                double v0 = 0.0, v1 = 0.0;
+                if (valid && col_cc[mt] >= 0) {
+                    v0 = at(i, j, col_cc[mt], col_x[mt]);
+                    if (i != j) v1 = at(j, i, col_cc[mt], col_x[mt]);
+                }
+                op.g[u][ks][mt][0] = v0;
+                op.g[u][ks][mt][1] = v1;
+            }
+        }
+}
+
+template <int NT, int KS>
+__global__ void __launch_bounds__(128, RAD_TILED_CTAS) radial_bwd_tiled_kernel(const RadialArgs a) {
+    constexpr int KP = 4 * KS;
+    constexpr int NT2 = KS / 2 + 1;
+    constexpr int NK = 8 * NT2, NCOL = 8 * NT;
+    __shared__ double abc_s[3 * KP];
+    __shared__ double w_s[NCOL * KP];
+    __shared__ double red[2 * NCOL * NK];
+    const int N = a.N, C = a.C, K = a.K;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int g = lane >> 2, q = lane & 3;
+    pdl_launch();
+    for (int k = threadIdx.x; k < KP; k += blockDim.x) {
+        abc_s[k] = k < K ? a.theta[a.off_a + k] : 0.0;
+        abc_s[KP + k] = k < K ? a.theta[a.off_b + k] : 0.0;
+        abc_s[2 * KP + k] = k < K ? a.theta[a.off_c + k] : 0.0;
+    }
+    for (int t = threadIdx.x; t < NCOL * KP; t += blockDim.x) w_s[t] = rad_w(a, t / KP, t % KP);
+    pdl_wait();
+    __syncthreads();
+    double G1[NT][NT2][2], G2[NT][NT2][2];
+#pragma unroll
+    for (int mt = 0; mt < NT; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < NT2; ++nt) G1[mt][nt][0] = G1[mt][nt][1] = G2[mt][nt][0] = G2[mt][nt][1] = 0.0;
+    int col_cc[NT], col_x[NT];
+#pragma unroll
+    for (int mt = 0; mt < NT; ++mt) {
+        const int col = 8 * mt + g;
+        col_cc[mt] = col < 4 * C ? (col >> 2) : -1;
+        col_x[mt] = col & 3;
+    }
+    double ck[NT2], c_one[NT2], c_msk[NT2];
+    bool isb[NT2];
+#pragma unroll
+    for (int nt = 0; nt < NT2; ++nt) {
+        const int k = 8 * nt + g;
+        isb[nt] = k < K;
+        ck[nt] = isb[nt] ? abc_s[2 * KP + k] : 0.0;
+        c_one[nt] = k == K ? 1.0 : 0.0;
+        c_msk[nt] = k == K + 1 ? 1.0 : 0.0;
+    }
+    const int NP = N * (N + 1) / 2, NU = (NP + RAD_UNIT - 1) / RAD_UNIT;
+    const int64_t total = (int64_t)a.B * NU, twarps = (int64_t)gridDim.x * nwarps;
+    const int64_t per = (total + twarps - 1) / twarps;
+    const int64_t u_begin = ((int64_t)blockIdx.x * nwarps + warp) * per, u_end = u_begin + per < total ? u_begin + per : total;
+    RadOperands<NT> cur, nxt;
+    if (u_begin < u_end) rad_fetch_tiled<NT>(a, (int)u_begin, NU, NP, col_cc, col_x, lane, cur);
+    for (int64_t unit = u_begin; unit < u_end; ++unit) {
+        if (unit + 1 < u_end) rad_fetch_tiled<NT>(a, (int)(unit + 1), NU, NP, col_cc, col_x, lane, nxt);
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+#pragma unroll
+            for (int ks = 0; ks < 2; ++ks) {
+                const double n2 = __shfl_sync(0xffffffffu, cur.n, 8 * u + q + 4 * ks);
+                const bool m2 = n2 == n2;
+                double a3[NT];
+#pragma unroll
+                for (int mt = 0; mt < NT; ++mt) a3[mt] = cur.g[u][ks][mt][0] + cur.g[u][ks][mt][1];
+                const double ns = m2 ? n2 : 0.0, nn = ns * ns;
+                double b1[NT2], b2[NT2];
+#pragma unroll
+                for (int nt = 0; nt < NT2; ++nt) {
+                    const double cn = ck[nt] * ns;
+                    const double rd = rcp_ge1(1.0 + cn * cn + 1e-16);
+                    b1[nt] = isb[nt] ? (m2 ? rd : 0.0) : c_one[nt] + (m2 ? c_msk[nt] : 0.0);
+                    b2[nt] = isb[nt] ? nn * rd * rd : 0.0;
+                }
+#pragma unroll
+                for (int nt = 0; nt < NT2; ++nt)
+#pragma unroll
+                    for (int mt = 0; mt < NT; ++mt) {
+                        dmma(G1[mt][nt][0], G1[mt][nt][1], a3[mt], b1[nt]);
+                        dmma(G2[mt][nt][0], G2[mt][nt][1], a3[mt], b2[nt]);
+                    }
+            }
+        }
+        cur = nxt;
+    }
+    for (int w = 0; w < nwarps; ++w) {
+        if (warp == w) {
+#pragma unroll
+            for (int mt = 0; mt < NT; ++mt)
+#pragma unroll
+                for (int nt = 0; nt < NT2; ++nt)
+#pragma unroll
+                    for (int e = 0; e < 2; ++e) {
+                        double* d1 = &red[(8 * mt + g) * NK + 8 * nt + 2 * q + e];
+                        double* d2 = d1 + NCOL * NK;
+                        *d1 = w == 0 ? G1[mt][nt][e] : *d1 + G1[mt][nt][e];
+                        *d2 = w == 0 ? G2[mt][nt][e] : *d2 + G2[mt][nt][e];
+                    }
+        }
+        __syncthreads();
+    }
+    double* row = a.part + (int64_t)blockIdx.x * a.part_stride;
+    const double* g1 = red;
+    const double* g2 = red + NCOL * NK;
+    for (int t = threadIdx.x; t < 4 * C * (K + 1); t += blockDim.x) {
+        const int col = t / (K + 1), k = t % (K + 1);
+        const int l = (col >> 1) & 1, o = 2 * (col >> 2) + (col & 1);
+        if (k < K)
+            row[(l ? a.po_w1 : a.po_w0) + (int64_t)o * K + k] = abc_s[KP + k] * g1[col * NK + k] + abc_s[k] * g1[col * NK + K + 1];
+        else
+            row[(l ? a.po_b1 : a.po_b0) + o] = g1[col * NK + K];
+    }
+    for (int t = threadIdx.x; t < 3 * K; t += blockDim.x) {
+        const int x = t / K, k = t % K;
+        double s = 0.0;
+        for (int col = 0; col < 4 * C; ++col)
+            s += w_s[col * KP + k] * (x == 0 ? g1[col * NK + K + 1] : x == 1 ? g1[col * NK + k] : g2[col * NK + k]);
+        if (x == 2) s *= -2.0 * abc_s[KP + k] * abc_s[2 * KP + k];
+        row[(x == 0 ? a.po_a : x == 1 ? a.po_b : a.po_c) + k] = s;
+    }
+}
+
+static int dispatch_radial_bwd_tiled(const RadialArgs& a, cudaStream_t st) {
+    if (a.C < 1 || a.C > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
+    const int nt = (4 * a.C + 7) / 8, ks = pick_ks(a.K);
+    if (ks < 0) return LGAE_E_UNSUPPORTED;
+    LaunchScope ls_("radial_bwd_tiled", st);
+#define LGAE_CASE(NTV, KSV)                                                                                   \
+    if (nt == NTV && ks == KSV) {                                                                             \
+        launch_k(radial_bwd_tiled_kernel<NTV, KSV>, dim3(radial_tiled_grid()), dim3(128), 0, st, a);                \
+        return check_launch("radial_bwd_tiled");                                                              \
+    }
+    LGAE_CASE(1, 3) LGAE_CASE(2, 3) LGAE_CASE(3, 3) LGAE_CASE(4, 3)
+    LGAE_CASE(1, 5) LGAE_CASE(2, 5) LGAE_CASE(3, 5) LGAE_CASE(4, 5)
+    LGAE_CASE(1, 8) LGAE_CASE(2, 8) LGAE_CASE(3, 8) LGAE_CASE(4, 8)
+#undef LGAE_CASE
+    return LGAE_E_UNSUPPORTED;
 }
 
 }  // namespace lgae

@@ -127,6 +127,21 @@ class FusedPlan:
         n = self._lib.lgae_partials_doubles(C.byref(self.desc), batch)
         return torch.empty(max(int(n), 1), dtype=torch.float64, device=device)
 
+    def tiled_scratch(self, batch: int, device) -> torch.Tensor:
+        """Scratch of the tiled adjoint (any N) for ``batch`` jets."""
+        n = self._lib.lgae_backward_tiled_scratch_doubles(C.byref(self.desc), batch)
+        if n < 0:
+            raise NotImplementedError(f"configuration not supported by the tiled fused adjoint: {self.tiled_reason()}")
+        return torch.empty(max(int(n), 1), dtype=torch.float64, device=device)
+
+    def tiled_reason(self) -> Optional[str]:
+        """None if the tiled adjoint runs this model, else the reason (no GPU needed)."""
+        n = self._lib.lgae_backward_tiled_scratch_doubles(C.byref(self.desc), 1)
+        if n >= 0:
+            return None
+        return ("a latent / input-map adjoint or a level adjoint whose shared memory does not fit at "
+                f"{self.n_particles} particles")
+
     def ws_tensor(self, ws: torch.Tensor, batch: int, kind: int, level: int, shape) -> torch.Tensor:
         off = self._lib.lgae_workspace_offset(C.byref(self.desc), batch, kind, level)
         if off < 0:
@@ -173,6 +188,17 @@ def encoder_backward_raw(plan: FusedPlan, theta, p4, node_mask, ws, sel, g00, g1
     return gtheta
 
 
+def encoder_backward_tiled_raw(plan: FusedPlan, theta, p4, node_mask, ws, sel, g00, g11):
+    """encoder_backward_raw for any N: the tiled adjoint (lgae_encoder_backward_tiled)."""
+    lib = plan._lib
+    dev = p4.device
+    gtheta = torch.empty(plan.n_params, dtype=torch.float64, device=dev)
+    scratch = plan.tiled_scratch(p4.shape[0], dev)
+    check(lib.lgae_encoder_backward_tiled(C.byref(plan.desc), ptr(theta), ptr(p4), ptr(node_mask), p4.shape[0], ptr(ws), ptr(sel),
+                                          ptr(g00), ptr(g11), ptr(gtheta), ptr(scratch), 0.0, None, _stream()), "encoder_backward_tiled")
+    return gtheta
+
+
 def decoder_forward_raw(plan: FusedPlan, theta, lat11, want_gen00: bool = False):
     lib = plan._lib
     b = lat11.shape[1]
@@ -194,6 +220,19 @@ def decoder_backward_raw(plan: FusedPlan, theta, lat11, ws, g_recon, g_gen00):
     part = plan.partials(b, dev)
     check(lib.lgae_decoder_backward(C.byref(plan.desc), ptr(theta), ptr(lat11), b, ptr(ws), ptr(g_recon), ptr(g_gen00), ptr(g_lat11),
                                     ptr(gtheta), ptr(part), 0.0, None, _stream()), "decoder_backward")
+    return g_lat11, gtheta
+
+
+def decoder_backward_tiled_raw(plan: FusedPlan, theta, lat11, ws, g_recon, g_gen00):
+    """decoder_backward_raw for any N: the tiled adjoint (lgae_decoder_backward_tiled)."""
+    lib = plan._lib
+    dev = lat11.device
+    b = lat11.shape[1]
+    gtheta = torch.empty(plan.n_params, dtype=torch.float64, device=dev)
+    g_lat11 = torch.empty_like(lat11)
+    scratch = plan.tiled_scratch(b, dev)
+    check(lib.lgae_decoder_backward_tiled(C.byref(plan.desc), ptr(theta), ptr(lat11), b, ptr(ws), ptr(g_recon), ptr(g_gen00), ptr(g_lat11),
+                                          ptr(gtheta), ptr(scratch), 0.0, None, _stream()), "decoder_backward_tiled")
     return g_lat11, gtheta
 
 
@@ -237,7 +276,8 @@ class _EncoderFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g00, g11):
         plan = ctx.plan
-        gtheta = encoder_backward_raw(plan, ctx.theta, ctx.p4, ctx.node_mask, ctx.ws, ctx.sel, _contig(g00), _contig(g11))
+        bwd = encoder_backward_raw if plan.n_particles <= 32 else encoder_backward_tiled_raw   # one particle per lane, or tiled
+        gtheta = bwd(plan, ctx.theta, ctx.p4, ctx.node_mask, ctx.ws, ctx.sel, _contig(g00), _contig(g11))
         return None, gtheta, None, None, None
 
 
@@ -260,7 +300,8 @@ class _DecoderFn(torch.autograd.Function):
         plan = ctx.plan
         if g_recon is None:
             g_recon = torch.zeros((2, ctx.lat11.shape[1], plan.n_particles, 4), dtype=torch.float64, device=ctx.lat11.device)
-        g_lat11, gtheta = decoder_backward_raw(plan, ctx.theta, ctx.lat11, ctx.ws, g_recon.contiguous(), _contig(g_gen00))
+        bwd = decoder_backward_raw if plan.n_particles <= 32 else decoder_backward_tiled_raw
+        g_lat11, gtheta = bwd(plan, ctx.theta, ctx.lat11, ctx.ws, g_recon.contiguous(), _contig(g_gen00))
         return None, gtheta, g_lat11, None, None
 
 

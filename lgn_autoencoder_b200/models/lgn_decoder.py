@@ -60,10 +60,13 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         self.num_learnable_parameters = sum(p.nelement() for p in self.parameters() if p.requires_grad)
 
         self._fused_reason = self._why_not_fused()
+        self._tiled_reason = None   # why autograd calls with N > 32 train through the composite (None: the tiled fused adjoint)
         if self._fused_reason is None:
             self._build_plan("decoder", n_particles=num_output_particles, channels=list(num_channels), num_basis_fn=num_basis_fn, mlp=mlp,
                              mlp_depth=mlp_depth if mlp else 0, mlp_width=mlp_width if mlp else 0, tau_s=tau_latent_scalars,
                              tau_v=tau_latent_vectors)
+            if num_output_particles > 32:
+                self._tiled_reason = self._plan.tiled_reason()
 
     def _why_not_fused(self):
         if any(m != 2 for m in self.level_maxdim):
@@ -92,9 +95,9 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         lat11 = latent_features[(1, 1)]
         if lat11.device.type != "cuda":
             raise RuntimeError("lgn_autoencoder_b200 runs on CUDA devices only (no CPU fallback)")
-        # the fused adjoint holds one particle per lane (N <= 32): larger jets train through the layer-level composite
+        # N > 32 trains on the tiled fused adjoint unless it cannot run this configuration (_tiled_reason)
         needs_grad = torch.is_grad_enabled() and (lat11.requires_grad or any(p.requires_grad for p in self.parameters()))
-        if self.fused and not (needs_grad and self.num_output_particles > 32):
+        if self.fused and not (needs_grad and self.num_output_particles > 32 and self._tiled_reason is not None):
             return self._forward_fused(lat11, covariance_test, nodes_all)
         return self._forward_generic(latent_features, covariance_test, nodes_all)
 

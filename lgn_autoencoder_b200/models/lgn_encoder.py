@@ -73,10 +73,13 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         self.num_learnable_parameters = sum(p.nelement() for p in self.parameters() if p.requires_grad)
 
         self._fused_reason = self._why_not_fused()
+        self._tiled_reason = None   # why autograd calls with N > 32 train through the composite (None: the tiled fused adjoint)
         if self._fused_reason is None:
             self._build_plan("encoder", n_particles=self.num_input_particles, channels=list(num_channels), num_basis_fn=num_basis_fn,
                              mlp=mlp, mlp_depth=mlp_depth if mlp else 0, mlp_width=mlp_width if mlp else 0,
                              latent_mode=map_to_latent, tau_s=tau_latent_scalars, tau_v=tau_latent_vectors, input_scale=scale)
+            if self.num_input_particles > 32:
+                self._tiled_reason = self._plan.tiled_reason()
 
     # ---------------------------------------------------------------------------------------------------------
     def _why_not_fused(self):
@@ -116,10 +119,10 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         p4 = torch.as_tensor(data["p4"]).to(self.device, self.dtype)
         if p4.device.type != "cuda":
             raise RuntimeError("lgn_autoencoder_b200 runs on CUDA devices only (no CPU fallback); construct the model with device='cuda'")
-        # the fused adjoint holds one particle per lane (N <= 32): larger jets train through the layer-level composite,
-        # whose autograd covers any N; forward-only calls keep the fused kernels (blocks of 32 particles)
+        # N > 32 trains on the tiled fused adjoint; a configuration it cannot run (_tiled_reason) trains through the
+        # layer-level composite, whose autograd covers any N; forward-only calls keep the fused kernels
         needs_grad = torch.is_grad_enabled() and (p4.requires_grad or any(p.requires_grad for p in self.parameters()))
-        if self.fused and "scalars" not in data and not (needs_grad and p4.shape[1] > 32):
+        if self.fused and "scalars" not in data and not (needs_grad and p4.shape[1] > 32 and self._tiled_reason is not None):
             return self._forward_fused(data, p4, covariance_test)
         return self._forward_generic(data, p4, covariance_test)
 
