@@ -167,7 +167,8 @@ int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, con
  * all-reduce exchanges them), produced by one gradient-init and one reduce launch for both models.  p4_in (B,N,4); when
  * normalize != 0 the normalised jets go to p4 and the per-jet factors to norm_factor (B), otherwise p4 / norm_factor are
  * unused.  loss (1) is overwritten; jet_loss (B) gets the per-jet chamfer distances; recon / g_recon (2,B,N,4), lat00, lat11,
- * sel, g_lat11 as in the model entry points.  partials: lgae_train_step_partials_doubles(enc, dec, batch) doubles. */
+ * sel, g_lat11 as in the model entry points.  partials: lgae_train_step_partials_doubles(enc, dec, batch) doubles.  Needs
+ * N <= 32 (LGAE_E_UNSUPPORTED before any launch otherwise; any N: lgae_train_step_tiled below). */
 int64_t lgae_train_step_partials_doubles(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int32_t batch);
 int lgae_train_step(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
                     const double* p4_in, const uint8_t* node_mask, int32_t batch, int32_t normalize, double* p4,
@@ -186,6 +187,28 @@ int lgae_train_step_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, con
                          double* norm_factor, double* ws_enc, double* ws_dec, double* lat00, double* lat11, int32_t* sel,
                          double* recon, double* g_recon, double* g_lat11, double* jet_loss, double* loss, double* gtheta,
                          int64_t gtheta_dec_offset, double* partials, double l1_lambda, int32_t get_real, int32_t phase, void* stream);
+/* The training step with the tiled adjoints (lgae_encoder_backward_tiled / lgae_decoder_backward_tiled) for any N >= 1, e.g. padded
+ * 150-particle jets.  Arguments, phases, streams and results as lgae_train_step / lgae_train_step_host, with `scratch` in place of
+ * `partials`: lgae_train_step_tiled_scratch_doubles(enc, dec, batch) doubles holding the adjoints of the neighbour sums (one
+ * region for both models, B*N*Cmax*10 complex), the encoder's dL/dR of one level (B * ceil(N/32) * N * C * 128 doubles: 1.57 GB at
+ * B = 512, N = 150, C = 4) and the rows of parameter-gradient partials.  The size query returns -1 for bad arguments and -2
+ * (LGAE_E_UNSUPPORTED) where either model's tiled adjoint or one of the step's fused glue kernels does not fit its shared memory;
+ * it needs no GPU, and the step then fails with LGAE_E_UNSUPPORTED before launching anything.  At N <= 32 the tiled step also
+ * runs: the forward then still writes the saved radial weights, which the tiled adjoint does not read, and the forward results
+ * are bit-identical to lgae_train_step's. */
+int64_t lgae_train_step_tiled_scratch_doubles(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int32_t batch);
+int lgae_train_step_tiled(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
+                          const double* p4_in, const uint8_t* node_mask, int32_t batch, int32_t normalize, double* p4,
+                          double* norm_factor, double* ws_enc, double* ws_dec, double* lat00, double* lat11, int32_t* sel,
+                          double* recon, double* g_recon, double* g_lat11, double* jet_loss, double* loss, double* gtheta,
+                          int64_t gtheta_dec_offset, double* scratch, double l1_lambda, int32_t get_real, int32_t phase, void* stream);
+int lgae_train_step_tiled_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc,
+                               const double* theta_dec, const double* host_p4, const uint8_t* host_mask, double* host_loss,
+                               double* p4_in, uint8_t* node_mask, int32_t batch, int32_t normalize, double* p4,
+                               double* norm_factor, double* ws_enc, double* ws_dec, double* lat00, double* lat11, int32_t* sel,
+                               double* recon, double* g_recon, double* g_lat11, double* jet_loss, double* loss, double* gtheta,
+                               int64_t gtheta_dec_offset, double* scratch, double l1_lambda, int32_t get_real, int32_t phase,
+                               void* stream);
 /* Split step for data-parallel training (`phase` above): phase 0 runs the whole step.  phase 1 runs it up to the point where the
  * DECODER's gradient bucket gtheta[gtheta_dec_offset, ...) is final -- its reduce is the last thing enqueued on the library's
  * auxiliary stream of the current device, which this function returns -- and phase 2 (same thread, same arguments, directly

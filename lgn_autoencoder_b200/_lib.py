@@ -117,6 +117,11 @@ _PROTOS = {
     "lgae_aux_stream": (C.c_void_p, []),
     "lgae_train_step_host": (C.c_int, [_D, _D, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
                                        C.c_int64, _P, C.c_double, C.c_int32, C.c_int32, _P]),
+    "lgae_train_step_tiled_scratch_doubles": (C.c_int64, [_D, _D, C.c_int32]),
+    "lgae_train_step_tiled": (C.c_int, [_D, _D, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                        C.c_int64, _P, C.c_double, C.c_int32, C.c_int32, _P]),
+    "lgae_train_step_tiled_host": (C.c_int, [_D, _D, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                             _P, _P, C.c_int64, _P, C.c_double, C.c_int32, C.c_int32, _P]),
     "lgae_chamfer": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "lgae_anomaly_scores": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     "lgae_normalize_p4": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P]),

@@ -31,6 +31,7 @@ int run_level_bwd_tiled(const LgaeModelDesc* d, int level, const double* theta, 
 int level_bwd_tiled_check(const LgaeModelDesc* d);
 int64_t level_tiled_part_doubles(const LgaeModelDesc* d, int level, int batch);
 int glue_bwd_check(const LgaeModelDesc* d);
+int train_step_glue_check(const LgaeModelDesc* de, const LgaeModelDesc* dd);
 int64_t radial_nrm_stride(int n);
 int radial_grid();
 int radial_tiled_grid();
@@ -261,6 +262,31 @@ static int tiled_check(const LgaeModelDesc* d) {
     if (int rc = level_bwd_tiled_check(d)) return rc;
     return glue_bwd_check(d);
 }
+// The tiled adjoint's two large regions inside a caller's scratch; gA == nullptr selects the per-lane adjoint.
+struct TiledBufs {
+    double* gA = nullptr;
+    double* gr = nullptr;   // encoder only
+};
+
+// Scratch of the tiled training step (lgae_train_step_tiled_scratch_doubles):
+//   [gA | g_r | decoder rows, encoder rows | reduce scratch (psum) | dec_tail counter]
+// gA is sized for the larger model and used by the decoder adjoint, then by the encoder adjoint (same stream, in that order).
+// The rows region holds both models' tiled partial rows (each with its own glue rows and reduce scratch, as in
+// lgae_backward_tiled_scratch_doubles) and the dec_tail rows, like lgae_train_step_partials_doubles does for the per-lane step;
+// the last reduce scratch takes the L1 partial sums of the gradient init, the last double the dec_tail completion counter.
+struct StepScratch {
+    int64_t gA, gr, part, total;
+};
+static StepScratch step_scratch(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int64_t B) {
+    const TiledScratch e = tiled_scratch(enc, B), d = tiled_scratch(dec, B);
+    const int64_t ga_e = e.gr - e.gA, ga_d = d.gr - d.gA;
+    StepScratch S;
+    S.gA = 0;
+    S.gr = ga_e > ga_d ? ga_e : ga_d;
+    S.part = S.gr + (e.part - e.gr);
+    S.total = S.part + (e.total - e.part) + (d.total - d.part) + B * 4 * dec->channels[dec->n_levels] + 1;
+    return S;
+}
 
 // The momenta the encoder kernels read: p4 itself, or (input_scale != 1) the scaled copy kept in the workspace, written here
 // when `write` (forward) and re-used by the adjoint.
@@ -373,6 +399,13 @@ int64_t lgae_backward_tiled_scratch_doubles(const LgaeModelDesc* d, int32_t batc
     if (rc != LGAE_OK || tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
     return tiled_scratch(d, batch).total;
 }
+int64_t lgae_train_step_tiled_scratch_doubles(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int32_t batch) {
+    const int re = check_desc(enc), rd = check_desc(dec);
+    if (re == LGAE_E_BADARG || rd == LGAE_E_BADARG || batch < 0 || enc->is_decoder || !dec->is_decoder) return -1;
+    if (re != LGAE_OK || rd != LGAE_OK || tiled_check(enc) != LGAE_OK || tiled_check(dec) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    if (const int rc = train_step_glue_check(enc, dec)) return rc == LGAE_E_BADARG ? -1 : LGAE_E_UNSUPPORTED;
+    return step_scratch(enc, dec, batch).total;
+}
 
 }  // extern "C"
 
@@ -410,10 +443,9 @@ static int enc_forward_launch(const LgaeModelDesc* d, const double* theta, const
 // Launch sequence of the encoder adjoint; appends its blocks / segments to `plan` (no reduce).
 static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
                                double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, PartPlan& plan,
-                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr, double* tiled = nullptr) {
+                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr, TiledBufs tiled = {}) {
     if (batch > 0) {
         const Layout L = layout(d, batch);
-        const TiledScratch T = tiled_scratch(d, batch);
         const int64_t rows = (int64_t)batch * d->n_particles;
         const int nl = d->n_levels;
         int cur = 0;
@@ -432,17 +464,14 @@ static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, cons
                     g_spre = ws + L.gS[cur];
                 }
             }
-            if (tiled) {   // tiled adjoint: radial weights re-evaluated, dL/dR of every level in one scratch buffer
-                LGAE_TRY(run_level_bwd_tiled(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], tiled + T.gA,
-                                             tiled + T.gr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
-                LGAE_TRY(run_radial_bwd(d, l, theta, p4, node_mask, batch, tiled + T.gr, nullptr, &plan, st));
-                cur ^= 1;
-                gs_zero = false;
-                continue;
+            if (tiled.gA) {   // tiled adjoint: radial weights re-evaluated, dL/dR of every level in one scratch buffer
+                LGAE_TRY(run_level_bwd_tiled(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], tiled.gA,
+                                             tiled.gr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
+            } else {
+                if (L.rsave[l] < 0 || L.gr[l] < 0) return LGAE_E_UNSUPPORTED;
+                LGAE_TRY(run_level_bwd(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], ws + L.rsave[l],
+                                       ws + L.gr[l], g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
             }
-            if (L.rsave[l] < 0 || L.gr[l] < 0) return LGAE_E_UNSUPPORTED;
-            LGAE_TRY(run_level_bwd(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], ws + L.rsave[l], ws + L.gr[l],
-                                   g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
             if (aux && l == 0) {
                 // the input-map adjoint (small) runs next to the last radial adjoint; both only feed the final reduce
                 LGAE_CUDA_TRY(cudaEventRecord(aux->fork[1], st), "aux fork");
@@ -450,7 +479,10 @@ static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, cons
                 LGAE_TRY(run_enc_input_bwd(d, p4, ws + L.mass, batch, ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], &plan, aux->s));
                 LGAE_CUDA_TRY(cudaEventRecord(aux->join[2], aux->s), "aux join");
             }
-            LGAE_TRY(run_radial_bwd(d, l, theta, p4, node_mask, batch, ws + L.gr[l], ws + L.nrm, &plan, st));
+            if (tiled.gA)
+                LGAE_TRY(run_radial_bwd(d, l, theta, p4, node_mask, batch, tiled.gr, nullptr, &plan, st));
+            else
+                LGAE_TRY(run_radial_bwd(d, l, theta, p4, node_mask, batch, ws + L.gr[l], ws + L.nrm, &plan, st));
             cur ^= 1;
             gs_zero = false;
         }
@@ -488,7 +520,7 @@ static int dec_forward_launch(const LgaeModelDesc* d, const double* theta, const
 
 static int dec_backward_launch(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws,
                                const double* g_recon, const double* g_gen00, double* g_lat11, PartPlan& plan, cudaStream_t st,
-                               bool with_output = true, bool with_input = true, double* tiled = nullptr) {
+                               bool with_output = true, bool with_input = true, double* tiled_gA = nullptr) {
     if (batch > 0) {
         const Layout L = layout(d, batch);
         const int64_t rows = (int64_t)batch * d->n_particles;
@@ -508,10 +540,9 @@ static int dec_backward_launch(const LgaeModelDesc* d, const double* theta, cons
                     g_spre = ws + L.gS[cur];
                 }
             }
-            if (tiled)
-                LGAE_TRY(run_level_bwd_tiled(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l],
-                                             tiled + tiled_scratch(d, batch).gA, nullptr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1],
-                                             ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
+            if (tiled_gA)
+                LGAE_TRY(run_level_bwd_tiled(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], tiled_gA,
+                                             nullptr, g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
             else
                 LGAE_TRY(run_level_bwd(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], nullptr, nullptr, g_spre,
                                        ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], ws + L.gy, &plan, st));
@@ -582,11 +613,13 @@ int lgae_encoder_backward_tiled(const LgaeModelDesc* d, const double* theta, con
     LGAE_TRY(check_desc(d));
     if (d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
     LGAE_TRY(tiled_check(d));
+    const TiledScratch T = tiled_scratch(d, batch);
     PartPlan plan;
-    plan.base = scratch + tiled_scratch(d, batch).part;
+    plan.base = scratch + T.part;
     int rc = LGAE_OK;
     p4 = scaled_input(d, p4, batch, ws, false, (cudaStream_t)stream, &rc);
-    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream, true, nullptr, scratch));
+    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream, true, nullptr,
+                                 TiledBufs{scratch + T.gA, scratch + T.gr}));
     return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
 }
 
@@ -597,9 +630,10 @@ int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, con
     if (!d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!lat11 || !ws || !g_recon || !g_lat11)))
         return LGAE_E_BADARG;
     LGAE_TRY(tiled_check(d));
+    const TiledScratch T = tiled_scratch(d, batch);
     PartPlan plan;
-    plan.base = scratch + tiled_scratch(d, batch).part;
-    LGAE_TRY(dec_backward_launch(d, theta, lat11, batch, ws, g_recon, g_gen00, g_lat11, plan, (cudaStream_t)stream, true, true, scratch));
+    plan.base = scratch + T.part;
+    LGAE_TRY(dec_backward_launch(d, theta, lat11, batch, ws, g_recon, g_gen00, g_lat11, plan, (cudaStream_t)stream, true, true, scratch + T.gA));
     return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
 }
 
@@ -627,20 +661,27 @@ static thread_local bool tl_phase1 = false;
 // all-reduce of the decoder bucket -- which then overlaps the encoder adjoint; phase 2 joins the auxiliary stream back.  host_p4 / host_mask / host_loss (pinned host memory, may be NULL): the jets
 // are copied to p4_in (and the mask to node_mask) at the start and the loss back at the end, on the same stream -- after the
 // auxiliary branch has been forked, so that weight packing and gradient init overlap the host-to-device copy.
+// tiled: the adjoints are the tiled ones (any N) and `buf` is the scratch of lgae_train_step_tiled_scratch_doubles; otherwise
+// the per-lane ones (N <= 32) and `buf` is the partials buffer of lgae_train_step_partials_doubles.
 static int train_step_impl(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
                            double* p4_in, uint8_t* node_mask, int32_t batch, int32_t normalize, double* p4, double* norm_factor,
                            double* ws_enc, double* ws_dec, double* lat00, double* lat11, int32_t* sel, double* recon, double* g_recon,
-                           double* g_lat11, double* jet_loss, double* loss, double* gtheta, int64_t gtheta_dec_offset, double* partials,
+                           double* g_lat11, double* jet_loss, double* loss, double* gtheta, int64_t gtheta_dec_offset, double* buf,
                            double l1_lambda, int32_t get_real, const double* host_p4, const uint8_t* host_mask, double* host_loss, int32_t phase,
-                           void* stream) {
+                           bool tiled, void* stream) {
     LGAE_TRY(check_desc(enc));
     LGAE_TRY(check_desc(dec));
     if (enc->is_decoder || !dec->is_decoder || batch < 1 || gtheta_dec_offset < enc->n_params) return LGAE_E_BADARG;
     if (get_real < LGAE_GET_REAL_REAL || get_real > LGAE_GET_REAL_NORM || phase < 0 || phase > 2) return LGAE_E_BADARG;
     if (!theta_enc || !theta_dec || !p4_in || !p4 || !ws_enc || !ws_dec || !lat00 || !lat11 || !sel || !recon || !g_recon || !g_lat11 ||
-        !jet_loss || !loss || !gtheta || !partials)
+        !jet_loss || !loss || !gtheta || !buf)
         return LGAE_E_BADARG;
-    if (enc->n_particles > 32) return LGAE_E_UNSUPPORTED;
+    if (!tiled && enc->n_particles > 32) return LGAE_E_UNSUPPORTED;   // the per-lane adjoint holds one particle per lane
+    // size of `buf`; for the tiled step also the refusal of a configuration before anything is launched
+    const int64_t n_buf = tiled ? lgae_train_step_tiled_scratch_doubles(enc, dec, batch) : lgae_train_step_partials_doubles(enc, dec, batch);
+    if (n_buf < 0) return (int)n_buf;
+    const StepScratch SS = tiled ? step_scratch(enc, dec, batch) : StepScratch{};
+    double* partials = tiled ? buf + SS.part : buf;   // the two plans' rows
     cudaStream_t st = (cudaStream_t)stream;
     const double* x = normalize ? p4 : p4_in;
     const bool scaled = has_input_scale(enc);
@@ -648,9 +689,9 @@ static int train_step_impl(const LgaeModelDesc* enc, const LgaeModelDesc* dec, c
     if (!aux) return LGAE_E_CUDA;
     if (phase == 2 && !tl_phase1) return LGAE_E_BADARG;
     std::lock_guard<std::mutex> aux_lock(g_aux_mu);
-    // L1 partial sums of the gradient init: the second reduce-scratch region at the end of `partials` (the first one, behind the
+    // L1 partial sums of the gradient init: the second reduce-scratch region at the end of `buf` (the first one, behind the
     // plan's blocks, is unused by this entry point)
-    double* psum = partials + lgae_train_step_partials_doubles(enc, dec, batch) - 1 - reduce_scratch_doubles();
+    double* psum = buf + n_buf - 1 - reduce_scratch_doubles();
     const int64_t n_all = enc->n_params + dec->n_params;
     PartPlan plan_d, plan_e;
     int rc_scale = LGAE_OK;
@@ -707,11 +748,12 @@ static int train_step_impl(const LgaeModelDesc* enc, const LgaeModelDesc* dec, c
     {
         // fused decoder tail: reconstruction, chamfer (+ batch sum), loss gradient, adjoint of the output map
         const Layout Ld = layout(dec, batch);
-        unsigned int* counter = reinterpret_cast<unsigned int*>(partials + lgae_train_step_partials_doubles(enc, dec, batch) - 1);
+        unsigned int* counter = reinterpret_cast<unsigned int*>(buf + n_buf - 1);
         LGAE_TRY(run_dec_tail(dec, theta_dec, batch, enc->n_particles, ws_dec + Ld.V[dec->n_levels], x, recon, g_recon, ws_dec + Ld.gV[0],
                               jet_loss, loss, counter, get_real, &plan_d, st));
     }
-    LGAE_TRY(dec_backward_launch(dec, theta_dec, lat11, batch, ws_dec, g_recon, nullptr, g_lat11, plan_d, st, false, false));
+    LGAE_TRY(dec_backward_launch(dec, theta_dec, lat11, batch, ws_dec, g_recon, nullptr, g_lat11, plan_d, st, false, false,
+                                 tiled ? buf + SS.gA : nullptr));
     {
         // fused adjoint of the bridge: decoder input map, then encoder latent map, latent gradient handed over on chip
         const Layout Le = layout(enc, batch), Ld = layout(dec, batch);
@@ -742,7 +784,8 @@ static int train_step_impl(const LgaeModelDesc* enc, const LgaeModelDesc* dec, c
     }
     // (split step: whatever the caller enqueued on the auxiliary stream between the phases is joined here too)
     LGAE_CUDA_TRY(cudaEventRecord(aux->join[3], aux->s), "aux join");
-    LGAE_TRY(enc_backward_launch(enc, theta_enc, xe, node_mask, batch, ws_enc, sel, nullptr, g_lat11, plan_e, st, false, aux));
+    LGAE_TRY(enc_backward_launch(enc, theta_enc, xe, node_mask, batch, ws_enc, sel, nullptr, g_lat11, plan_e, st, false, aux,
+                                 tiled ? TiledBufs{buf + SS.gA, buf + SS.gr} : TiledBufs{}));
     LGAE_CUDA_TRY(cudaStreamWaitEvent(st, aux->join[1], 0), "aux join wait");
     LGAE_CUDA_TRY(cudaStreamWaitEvent(st, aux->join[3], 0), "aux join wait");
     return run_reduce_segs(&plan_e, n_all, gtheta, psum, 0.0, nullptr, st);
@@ -757,7 +800,7 @@ int lgae_train_step(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const do
                     double l1_lambda, int32_t get_real, int32_t phase, void* stream) {
     return train_step_impl(enc, dec, theta_enc, theta_dec, const_cast<double*>(p4_in), const_cast<uint8_t*>(node_mask), batch, normalize, p4,
                            norm_factor, ws_enc, ws_dec, lat00, lat11, sel, recon, g_recon, g_lat11, jet_loss, loss, gtheta, gtheta_dec_offset,
-                           partials, l1_lambda, get_real, nullptr, nullptr, nullptr, phase, stream);
+                           partials, l1_lambda, get_real, nullptr, nullptr, nullptr, phase, false, stream);
 }
 
 int lgae_train_step_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
@@ -769,7 +812,29 @@ int lgae_train_step_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, con
     if (!host_p4 || !host_loss) return LGAE_E_BADARG;
     return train_step_impl(enc, dec, theta_enc, theta_dec, p4_in, node_mask, batch, normalize, p4, norm_factor, ws_enc, ws_dec, lat00, lat11, sel,
                            recon, g_recon, g_lat11, jet_loss, loss, gtheta, gtheta_dec_offset, partials, l1_lambda, get_real, host_p4, host_mask,
-                           host_loss, phase, stream);
+                           host_loss, phase, false, stream);
+}
+
+int lgae_train_step_tiled(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
+                          const double* p4_in, const uint8_t* node_mask, int32_t batch, int32_t normalize, double* p4, double* norm_factor,
+                          double* ws_enc, double* ws_dec, double* lat00, double* lat11, int32_t* sel, double* recon, double* g_recon,
+                          double* g_lat11, double* jet_loss, double* loss, double* gtheta, int64_t gtheta_dec_offset, double* scratch,
+                          double l1_lambda, int32_t get_real, int32_t phase, void* stream) {
+    return train_step_impl(enc, dec, theta_enc, theta_dec, const_cast<double*>(p4_in), const_cast<uint8_t*>(node_mask), batch, normalize, p4,
+                           norm_factor, ws_enc, ws_dec, lat00, lat11, sel, recon, g_recon, g_lat11, jet_loss, loss, gtheta, gtheta_dec_offset,
+                           scratch, l1_lambda, get_real, nullptr, nullptr, nullptr, phase, true, stream);
+}
+
+int lgae_train_step_tiled_host(const LgaeModelDesc* enc, const LgaeModelDesc* dec, const double* theta_enc, const double* theta_dec,
+                               const double* host_p4, const uint8_t* host_mask, double* host_loss, double* p4_in, uint8_t* node_mask,
+                               int32_t batch, int32_t normalize, double* p4, double* norm_factor, double* ws_enc, double* ws_dec,
+                               double* lat00, double* lat11, int32_t* sel, double* recon, double* g_recon, double* g_lat11, double* jet_loss,
+                               double* loss, double* gtheta, int64_t gtheta_dec_offset, double* scratch, double l1_lambda, int32_t get_real,
+                               int32_t phase, void* stream) {
+    if (!host_p4 || !host_loss) return LGAE_E_BADARG;
+    return train_step_impl(enc, dec, theta_enc, theta_dec, p4_in, node_mask, batch, normalize, p4, norm_factor, ws_enc, ws_dec, lat00, lat11, sel,
+                           recon, g_recon, g_lat11, jet_loss, loss, gtheta, gtheta_dec_offset, scratch, l1_lambda, get_real, host_p4, host_mask,
+                           host_loss, phase, true, stream);
 }
 
 int lgae_chamfer(const double* recon, const double* target, int32_t batch, int32_t n, int32_t m, int32_t get_real, double* loss,

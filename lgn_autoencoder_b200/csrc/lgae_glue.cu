@@ -1191,16 +1191,20 @@ int run_dec_input(const LgaeModelDesc* d, const double* theta, int B, const doub
     launch_k(dec_input_kernel, dim3(B), dim3(128), bytes, st, a);
     return check_launch("dec_input");
 }
+// Shared memory of enc_latent_body (the first region of latent_bridge_kernel's).
+static size_t latent_bridge_scratch_bytes(const LgaeModelDesc* de) {
+    const int rows = de->latent_mode == LGAE_LATENT_MIX ? 1 : de->n_particles;
+    return (size_t)rows * (de->tau_s + 4 * de->tau_v) * sizeof(cplx);
+}
 // enc_latent + dec_input fused (training step / inference of both models back to back).
 int run_latent_bridge(const LgaeModelDesc* de, const double* theta_e, const LgaeModelDesc* dd, const double* theta_d, int B, const double* S,
                       const double* V, double* lat00, double* lat11, int32_t* sel, double* y, double* S0, double* V0, cudaStream_t st, int parts) {
     LatentArgs a = latent_args(de, theta_e, B, S, V);
     a.lat00 = lat00; a.lat11 = lat11; a.sel = sel; a.parts = parts;
     DecInArgs di = dec_in_args(dd, theta_d, B, lat11, y, S0, V0);
-    const int rows = a.mode == LGAE_LATENT_MIX ? 1 : a.N;
     const int mult = a.mode == LGAE_LATENT_MINMAX ? 2 : 1;
     if (di.tau != mult * a.tau_v) return LGAE_E_BADARG;   // decoder latent width must be the encoder's output width
-    const size_t scratch = (size_t)rows * (a.tau_s + 4 * a.tau_v) * sizeof(cplx);
+    const size_t scratch = latent_bridge_scratch_bytes(de);
     const size_t bytes = scratch + (size_t)di.tau * 4 * sizeof(cplx);
     if (bytes > 200 * 1024) return LGAE_E_UNSUPPORTED;
     if (int rc = ensure_smem((const void*)latent_bridge_kernel, bytes)) return rc;
@@ -1227,6 +1231,18 @@ int run_dec_input_bwd(const LgaeModelDesc* d, const double* theta, int B, const 
     launch_k(dec_input_bwd_kernel, dim3(grid), dim3(128), bytes, st, a);
     return check_launch("dec_input_bwd");
 }
+// Shared memory of latent_bridge_bwd_kernel: [dec_input_bwd | enc_latent_bwd | latent gradient], in complex numbers, each
+// region rounded up to 8.  0 if the two models do not fit together (latent widths or particle counts differ).
+static size_t latent_bridge_bwd_cd(const LgaeModelDesc* dd) {
+    return (dec_input_bwd_smem_cplx(dd->n_particles, dd->channels[0], dd->tau_v) + 7) & ~(size_t)7;
+}
+static size_t latent_bridge_bwd_smem_cplx(const LgaeModelDesc* dd, const LgaeModelDesc* de) {
+    const int mult = de->latent_mode == LGAE_LATENT_MINMAX ? 2 : 1;
+    if (dd->tau_v != mult * de->tau_v || dd->n_particles != de->n_particles) return 0;
+    const size_t ce = (enc_latent_bwd_smem_cplx(de->n_particles, de->channels[de->n_levels], de->tau_s, de->tau_v, de->latent_mode) + 7) &
+                      ~(size_t)7;
+    return latent_bridge_bwd_cd(dd) + ce + (size_t)dd->tau_v * 4;
+}
 // dec_input_bwd + enc_latent_bwd fused (training step).  g_lat11 is still written (API output).
 int run_latent_bridge_bwd(const LgaeModelDesc* dd, const double* theta_d, const LgaeModelDesc* de, const double* theta_e, int B,
                           const double* lat11, double* y, const double* gS_d, const double* gV_d, const double* gy, double* g_lat11,
@@ -1236,11 +1252,10 @@ int run_latent_bridge_bwd(const LgaeModelDesc* dd, const double* theta_d, const 
     // the encoder's plan continues where the decoder's ends
     DecInArgs di = dec_in_args(dd, theta_d, B, lat11, y, nullptr, nullptr);
     di.gS = gS_d; di.gV = gV_d; di.gy = gy; di.g_lat11 = g_lat11;
-    if (di.N > 128) return LGAE_E_UNSUPPORTED;
     LatentArgs a = latent_args(de, theta_e, B, S, V);
     a.sel = const_cast<int32_t*>(sel); a.g_lat00 = nullptr; a.g_lat11 = nullptr; a.gS = gS_e; a.gV = gV_e;
-    const int mult = a.mode == LGAE_LATENT_MINMAX ? 2 : 1;
-    if (di.tau != mult * a.tau_v || di.N != a.N) return LGAE_E_BADARG;
+    const size_t smem = latent_bridge_bwd_smem_cplx(dd, de);
+    if (smem == 0) return LGAE_E_BADARG;
     const int mix = a.mode == LGAE_LATENT_MIX;
     const int cin = mix ? a.N * a.C : a.C;
     const int grid = glue_grid(B);
@@ -1258,9 +1273,8 @@ int run_latent_bridge_bwd(const LgaeModelDesc* dd, const double* theta_d, const 
         if (int rc = plan_e->seg(a.off11, off, w, n00, n11, grid)) return rc;
         a.partials = plan_e->base + off; a.part_stride = w; a.po00 = 0; a.po11 = n00;
     }
-    const size_t cd = (dec_input_bwd_smem_cplx(di.N, di.C, di.tau) + 7) & ~(size_t)7;
-    const size_t ce = (enc_latent_bwd_smem_cplx(a.N, a.C, a.tau_s, a.tau_v, a.mode) + 7) & ~(size_t)7;
-    const size_t bytes = (cd + ce + (size_t)di.tau * 4) * sizeof(cplx);
+    const size_t cd = latent_bridge_bwd_cd(dd), ce = smem - cd - (size_t)di.tau * 4;
+    const size_t bytes = smem * sizeof(cplx);
     if (bytes > 200 * 1024) return LGAE_E_UNSUPPORTED;
     if (int rc = ensure_smem((const void*)latent_bridge_bwd_kernel, bytes)) return rc;
     LaunchScope ls_("latent_bridge_bwd", st);
@@ -1373,6 +1387,9 @@ int run_scores(const double* recon, const double* target, const double* factor, 
     launch_k(scores_kernel, dim3(B), dim3(128), bytes, st, recon, target, factor, B, N, mode, out);
     return check_launch("anomaly_scores");
 }
+static size_t dec_tail_bytes(int N, int M, int C) {
+    return ((size_t)N * C * 4 + N * 4 + C) * sizeof(cplx) + (size_t)(4 * N + 4 * M + N + M) * sizeof(double) + (size_t)(N + M) * sizeof(int);
+}
 // mix_to_output + chamfer + their adjoints for a training step (see dec_tail_kernel).  `counter`: 4 bytes of device scratch.
 int run_dec_tail(const LgaeModelDesc* d, const double* theta, int B, int M, const double* V, const double* target, double* recon,
                  double* g_recon, double* gV, double* jet_loss, double* loss, unsigned int* counter, int mode, PartPlan* plan, cudaStream_t st) {
@@ -1386,7 +1403,7 @@ int run_dec_tail(const LgaeModelDesc* d, const double* theta, int B, int M, cons
     if (int rc = plan->seg(d->off_out00, off, w, 0, 2 * C, B)) return rc;
     if (int rc = plan->seg(d->off_out11, off, w, 2 * C, 2 * C, B)) return rc;
     a.partials = plan->base + off; a.part_stride = w;
-    const size_t bytes = ((size_t)N * C * 4 + N * 4 + C) * sizeof(cplx) + (size_t)(4 * N + 4 * M + N + M) * sizeof(double) + (size_t)(N + M) * sizeof(int);
+    const size_t bytes = dec_tail_bytes(N, M, C);
     if (bytes > 200 * 1024) return LGAE_E_UNSUPPORTED;
     if (int rc = ensure_smem((const void*)dec_tail_kernel, bytes)) return rc;
     if (cudaMemsetAsync(counter, 0, sizeof(unsigned int), st) != cudaSuccess) return check_launch("memset counter");
@@ -1426,5 +1443,17 @@ int glue_bwd_check(const LgaeModelDesc* d) {
     const size_t n = d->is_decoder ? dec_input_bwd_smem_cplx(d->n_particles, d->channels[0], d->tau_v)
                                    : enc_latent_bwd_smem_cplx(d->n_particles, d->channels[d->n_levels], d->tau_s, d->tau_v, d->latent_mode);
     return n * sizeof(cplx) > 200 * 1024 ? LGAE_E_UNSUPPORTED : LGAE_OK;
+}
+// The same for the fused glue kernels of the training step (latent_bridge, dec_tail, latent_bridge_bwd), with the checks their
+// launchers make: LGAE_E_BADARG if the two models do not fit together, LGAE_E_UNSUPPORTED if a kernel's shared memory does not
+// fit.  No GPU needed.
+int train_step_glue_check(const LgaeModelDesc* de, const LgaeModelDesc* dd) {
+    const size_t bridge_bwd = latent_bridge_bwd_smem_cplx(dd, de);
+    if (bridge_bwd == 0) return LGAE_E_BADARG;
+    const size_t lim = 200 * 1024;
+    if (bridge_bwd * sizeof(cplx) > lim || latent_bridge_scratch_bytes(de) + (size_t)dd->tau_v * 4 * sizeof(cplx) > lim ||
+        dec_tail_bytes(dd->n_particles, de->n_particles, dd->channels[dd->n_levels]) > lim)
+        return LGAE_E_UNSUPPORTED;
+    return LGAE_OK;
 }
 }  // namespace lgae

@@ -65,23 +65,43 @@ class FusedTrainStep:
     returns the loss as a 0-d device tensor; afterwards ``param.grad`` of every encoder / decoder parameter holds the
     gradient of  chamfer_sum + l1_lambda * l1_scale * |theta|_1  (summed over ranks if a process group is active).
     ``recon`` (2,B,N,4), ``latent00/11``, ``norm_factor`` (B,) expose the step's other results.
+
+    ``adjoint`` picks the backward kernels: ``"per_lane"`` (one particle per lane, at most 32 particles per jet) or ``"tiled"``
+    (blocks of 32 particles, any particle count, e.g. padded 150-particle jets; ``lgae_train_step_tiled``).  The tiled step
+    keeps the encoder's dL/dR of one level in its scratch: B * ceil(N/32) * N * C * 128 doubles, 1.57 GB at B = 512, N = 150,
+    C = 4, on top of the workspaces.
     """
+
+    ADJOINTS = ("per_lane", "tiled")
 
     def __init__(self, encoder, decoder, batch: int, l1_lambda: float = 1e-8, l1_scale: float = 1.0, normalize: bool = True,
                  use_labels: bool = False, use_graph: bool = True, group=None, get_real: str = "real", overlap_allreduce: bool = False,
-                 peer_allreduce: bool = False):
+                 peer_allreduce: bool = False, adjoint: str = "per_lane"):
+        if adjoint not in self.ADJOINTS:
+            raise ValueError(f"adjoint must be one of {self.ADJOINTS}, not {adjoint!r}")
         if not (getattr(encoder, "fused", False) and getattr(decoder, "fused", False)):
             raise NotImplementedError("FusedTrainStep needs the fused (maxdim 2) encoder and decoder")
         self.enc, self.dec, self.B = encoder, decoder, int(batch)
         self.pe, self.pd = encoder._plan, decoder._plan
-        if self.pe.n_particles > 32:
-            raise NotImplementedError("the adjoint kernels hold one particle per lane: at most 32 particles per jet")
+        self.tiled = adjoint == "tiled"
+        if self.pe.n_particles > 32 and not self.tiled:
+            raise NotImplementedError("the per-lane adjoint holds one particle per lane: at most 32 particles per jet "
+                                      "(adjoint='tiled' takes any number)")
         self.l1 = float(l1_lambda) * float(l1_scale)
         self.normalize = normalize
         self.get_real = fused.get_real_mode(get_real)
         self.overlap_allreduce = overlap_allreduce
         self.group = group
         self.lib = _lib.load()
+        if self.tiled:
+            n_part = self.lib.lgae_train_step_tiled_scratch_doubles(C.byref(self.pe.desc), C.byref(self.pd.desc), self.B)
+            if n_part == -2:
+                reason = self.pe.tiled_reason() or self.pd.tiled_reason() or "a glue kernel of the step does not fit its shared memory"
+                raise NotImplementedError(f"configuration not supported by the tiled training step: {reason}")
+            if n_part < 0:
+                raise ValueError("encoder and decoder do not form one training step (latent widths or particle counts differ)")
+        else:
+            n_part = self.lib.lgae_train_step_partials_doubles(C.byref(self.pe.desc), C.byref(self.pd.desc), self.B)
         dev = next(encoder.parameters()).device
         self.dev = dev
         f64 = dict(dtype=torch.float64, device=dev)
@@ -92,8 +112,7 @@ class FusedTrainStep:
         self.norm_factor = torch.ones(B, **f64)
         self.mask = torch.ones((B, N), dtype=torch.uint8, device=dev) if use_labels else None
         self.ws_e, self.ws_d = self.pe.workspace(B, dev), self.pd.workspace(B, dev)
-        n_part = self.lib.lgae_train_step_partials_doubles(C.byref(self.pe.desc), C.byref(self.pd.desc), B)
-        self.part = torch.empty(max(int(n_part), 1), **f64)
+        self.part = torch.empty(max(int(n_part), 1), **f64)   # partials, or the tiled step's scratch
         self.latent00 = torch.empty((2, B, 1, ts, 1), **f64)
         self.latent11 = torch.empty((2, B, 1, tv, 4), **f64)
         self.sel = torch.empty((4, 2, B, max(self.pe.tau_s, self.pe.tau_v)), dtype=torch.int32, device=dev)
@@ -201,7 +220,8 @@ class FusedTrainStep:
         th_e, _ = self.enc._flat_params()
         th_d, _ = self.dec._flat_params()
         self._thetas = (th_e.data_ptr(), th_d.data_ptr())
-        self._phases(lambda phase: check(lib.lgae_train_step(
+        fn = lib.lgae_train_step_tiled if self.tiled else lib.lgae_train_step
+        self._phases(lambda phase: check(fn(
             C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(self.p4_in), ptr(self.mask), B, 1 if self.normalize else 0,
             ptr(self.p4), ptr(self.norm_factor), ptr(self.ws_e), ptr(self.ws_d), ptr(self.latent00), ptr(self.latent11), ptr(self.sel),
             ptr(self.recon), ptr(self.g_recon), ptr(self.g_lat11), ptr(self.jet_loss), ptr(self.loss), ptr(self.g_step), self.off_d,
@@ -294,7 +314,8 @@ class FusedTrainStep:
         th_e, _ = self.enc._flat_params()
         th_d, _ = self.dec._flat_params()
         self._thetas = (th_e.data_ptr(), th_d.data_ptr())
-        self._phases(lambda phase: check(lib.lgae_train_step_host(
+        fn = lib.lgae_train_step_tiled_host if self.tiled else lib.lgae_train_step_host
+        self._phases(lambda phase: check(fn(
             C.byref(pe.desc), C.byref(pd.desc), ptr(th_e), ptr(th_d), ptr(self.host_p4), ptr(self.host_mask), ptr(self.host_loss),
             ptr(self.p4_in), ptr(self.mask), B, 1 if self.normalize else 0, ptr(self.p4), ptr(self.norm_factor), ptr(self.ws_e),
             ptr(self.ws_d), ptr(self.latent00), ptr(self.latent11), ptr(self.sel), ptr(self.recon), ptr(self.g_recon), ptr(self.g_lat11),

@@ -27,15 +27,17 @@ CFG = dict(n=150, enc_channels=[3, 3, 4, 4], dec_channels=[4, 4, 3, 3], tau_s=1,
 FP64_PEAK_TFLOPS = 37.1   # measured with tools/fp64_peak.cu: profiles/fp64_peak_r01.json
 
 
-def build(dev, seed=0):
+def build(dev, seed=0, n=None):
+    """The cfg-1 encoder and decoder at CFG["n"] particles (or n)."""
     from lgn_autoencoder_b200.models import LGNDecoder, LGNEncoder
+    n = CFG["n"] if n is None else n
     torch.manual_seed(seed)
     common = dict(maxdim=[2], num_basis_fn=CFG["num_basis_fn"], max_zf=[1], weight_init="randn", level_gain=[1.0], activation="leakyrelu",
                   mlp=True, mlp_depth=CFG["mlp_depth"], mlp_width=CFG["mlp_width"], device=torch.device("cpu"), dtype=torch.float64)
-    enc = LGNEncoder(num_input_particles=CFG["n"], tau_input_scalars=1, tau_input_vectors=1, tau_latent_scalars=CFG["tau_s"],
+    enc = LGNEncoder(num_input_particles=n, tau_input_scalars=1, tau_input_vectors=1, tau_latent_scalars=CFG["tau_s"],
                      tau_latent_vectors=CFG["tau_v"], num_channels=CFG["enc_channels"], jet_features=False,
                      map_to_latent=CFG["map_to_latent"], **common)
-    dec = LGNDecoder(tau_latent_scalars=2 * CFG["tau_s"], tau_latent_vectors=2 * CFG["tau_v"], num_output_particles=CFG["n"],
+    dec = LGNDecoder(tau_latent_scalars=2 * CFG["tau_s"], tau_latent_vectors=2 * CFG["tau_v"], num_output_particles=n,
                      tau_output_scalars=1, tau_output_vectors=1, num_channels=CFG["dec_channels"], cg_dict=enc.cg_dict, **common)
     return enc.to(dev), dec.to(dev)
 
