@@ -144,6 +144,25 @@ int lgae_encoder_backward_tiled(const LgaeModelDesc* d, const double* theta, con
                                 int32_t batch, double* workspace, const int32_t* sel, const double* g_lat00,
                                 const double* g_lat11, double* gtheta, double* scratch, double l1_lambda,
                                 double* loss_accumulate, void* stream);
+/* The encoder adjoints with the gradient with respect to the jets.  Arguments as lgae_encoder_backward /
+ * lgae_encoder_backward_tiled, plus g_p4 (B,N,4), overwritten with dL/dp4 of the caller's unscaled p4, and gp_scratch
+ * (lgae_encoder_input_grad_scratch_doubles(d, batch) doubles).  g_p4 == NULL: exactly the entry point without _p4 (gp_scratch
+ * unused).  The parameter gradient is bit-identical either way.  dL/dp4 gathers the input map (mass scalar and canonical vector),
+ * the edge features R_ij canon(p_i - p_j) and the pair norms of the radial functions of every level; min / max selections are
+ * constants.  Where p^2 == 0 exactly (zero-momentum padding) the mass scalar's term, 0 * inf in the reference, is dropped, so
+ * every particle gets a finite gradient (DESIGN.md section 4e).  Deterministic, no atomics. */
+int lgae_encoder_backward_p4(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask,
+                             int32_t batch, double* workspace, const int32_t* sel, const double* g_lat00,
+                             const double* g_lat11, double* gtheta, double* partials, double l1_lambda,
+                             double* loss_accumulate, double* g_p4, double* gp_scratch, void* stream);
+int lgae_encoder_backward_tiled_p4(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask,
+                                   int32_t batch, double* workspace, const int32_t* sel, const double* g_lat00,
+                                   const double* g_lat11, double* gtheta, double* scratch, double l1_lambda,
+                                   double* loss_accumulate, double* g_p4, double* gp_scratch, void* stream);
+/* Doubles of gp_scratch: B*N*4, plus B*N*Cmax*20 at N <= 32.  -1 for bad arguments (including a decoder descriptor), -2
+ * (LGAE_E_UNSUPPORTED) where the adjoint matching N (per-lane at N <= 32, tiled above) or the input-gradient kernels refuse the
+ * configuration.  Needs no GPU. */
+int64_t lgae_encoder_input_grad_scratch_doubles(const LgaeModelDesc* d, int32_t batch);
 /* LGNDecoder.forward.  lat11 (2,B,1,tau_v,4) planar complex Cartesian.  recon (2,B,N,4); gen00 (2,B,N,1,1) or NULL
  * (NULL: the output scalars are not wanted, the last level's scalar MLP -- which feeds only them -- is then not run;
  * pass g_gen00 = NULL to the backward accordingly). */
@@ -236,6 +255,15 @@ int lgae_anomaly_scores(const double* recon, const double* target, const double*
                         double* scores, void* stream);
 /* normalize_p4(..., 'overall_max') (utils/normalize_p4.py:39-52): out = p4 / (max|p4| + 1e-16) per jet. */
 int lgae_normalize_p4(const double* p4, int32_t batch, int32_t n, double* out, double* factor, void* stream);
+/* Adjoint of lgae_normalize_p4: g_p4 (B,N,4) overwritten from g_out (B,N,4) and g_factor (B), either may be NULL (zero).  The
+ * factor's gradient reaches the maxima as torch's amax adjoint routes it: split evenly between tied particles and, inside a
+ * particle, between tied components. */
+int lgae_normalize_p4_backward(const double* p4, int32_t batch, int32_t n, const double* g_out, const double* g_factor,
+                               double* g_p4, void* stream);
+/* d loss / d target (B,M,4) of lgae_chamfer, overwritten, scaled by *g_loss (device scalar) when g_loss != NULL.  Nearest
+ * neighbours are chosen as lgae_chamfer chooses them (first index of the minimum). */
+int lgae_chamfer_target_grad(const double* recon, const double* target, int32_t batch, int32_t n, int32_t m, int32_t get_real,
+                             const double* g_loss, double* g_target, void* stream);
 /* L1 regulariser: out[0] (+)= lambda * sum |theta| ; gtheta += lambda * sign(theta)  (lgn_encoder.py:249-250). */
 int lgae_l1(const double* theta, int64_t n, double lambda, double* out_accumulate, double* gtheta_accumulate,
             void* stream);

@@ -110,6 +110,9 @@ _PROTOS = {
     "lgae_decoder_forward": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P]),
     "lgae_decoder_backward": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
     "lgae_encoder_backward_tiled": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
+    "lgae_encoder_backward_p4": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P, _P, _P]),
+    "lgae_encoder_backward_tiled_p4": (C.c_int, [_D, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P, _P, _P]),
+    "lgae_encoder_input_grad_scratch_doubles": (C.c_int64, [_D, C.c_int32]),
     "lgae_decoder_backward_tiled": (C.c_int, [_D, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_double, _P, _P]),
     "lgae_train_step_partials_doubles": (C.c_int64, [_D, _D, C.c_int32]),
     "lgae_train_step": (C.c_int, [_D, _D, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int64, _P,
@@ -125,6 +128,8 @@ _PROTOS = {
     "lgae_chamfer": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "lgae_anomaly_scores": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     "lgae_normalize_p4": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P]),
+    "lgae_normalize_p4_backward": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
+    "lgae_chamfer_target_grad": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),
     "lgae_l1": (C.c_int, [_P, C.c_int64, C.c_double, _P, _P, _P]),
     "lgae_level_forward": (C.c_int, [_D, C.c_int32, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "lgae_level_backward": (C.c_int, [_D, C.c_int32, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -18,7 +18,16 @@ int run_level_fwd(const LgaeModelDesc* d, int level, const double* theta, const 
                   const double* s_in, const double* v_in, double* sums, double* r_save, double* s_pre, double* v_out, cudaStream_t st);
 int run_level_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
                   const double* s_in, const double* v_in, const double* sums, const double* r_save, double* g_r, const double* g_s_pre,
-                  const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st);
+                  const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st,
+                  double* g_a = nullptr);
+int pgrad_check(const LgaeModelDesc* d);
+int run_pgrad_level(const LgaeModelDesc* d, int level, const double* theta, const double* p, const uint8_t* node_mask, int batch,
+                    const double* s_in, const double* v_in, const double* gA, double* gp, cudaStream_t st);
+int run_pgrad_input(const LgaeModelDesc* d, const double* theta, const double* p, int batch, const double* gS, const double* gV,
+                    const double* gp, double scale, double* g_p4, cudaStream_t st);
+int run_chamfer_target_grad(const double* recon, const double* target, int B, int N, int M, int mode, const double* g_loss,
+                            double* g_target, cudaStream_t st);
+int run_normalize_bwd(const double* p4, int B, int N, const double* g_out, const double* g_factor, double* g_p4, cudaStream_t st);
 int run_radial_fwd_all(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
                        double* const* r, double* nrm, cudaStream_t st);
 int run_radial_fwd(const LgaeModelDesc* d, int level, const double* theta, const double* p4, const uint8_t* node_mask, int batch,
@@ -268,6 +277,27 @@ struct TiledBufs {
     double* gr = nullptr;   // encoder only
 };
 
+// Scratch of the encoder's input gradient (lgae_encoder_input_grad_scratch_doubles): [gp | gA]
+//   gp (B,N,4): dL/dp of the levels, accumulated in level order
+//   gA (B,N,Cmax,10) complex, N <= 32 only: the per-lane level adjoint's neighbour-sum adjoints of the current level (the tiled
+//      adjoint keeps them in its own scratch)
+struct InputGradScratch {
+    int64_t gp, gA, total;
+};
+static InputGradScratch input_grad_scratch(const LgaeModelDesc* d, int64_t B) {
+    InputGradScratch G;
+    const int64_t nodes = B * d->n_particles;
+    G.gp = 0;
+    G.gA = (nodes * 4 + 3) & ~int64_t(3);
+    G.total = G.gA + (d->n_particles <= 32 ? nodes * max_channels(d) * 20 : 0);
+    return G;
+}
+// The input gradient requested from the encoder adjoint; g_p4 == nullptr: none (the adjoint's launches are unchanged).
+struct InputGrad {
+    double* g_p4 = nullptr;      // (B,N,4) out, with respect to the caller's unscaled p4
+    double* scratch = nullptr;   // input_grad_scratch
+};
+
 // Scratch of the tiled training step (lgae_train_step_tiled_scratch_doubles):
 //   [gA | g_r | decoder rows, encoder rows | reduce scratch (psum) | dec_tail counter]
 // gA is sized for the larger model and used by the decoder adjoint, then by the encoder adjoint (same stream, in that order).
@@ -443,12 +473,21 @@ static int enc_forward_launch(const LgaeModelDesc* d, const double* theta, const
 // Launch sequence of the encoder adjoint; appends its blocks / segments to `plan` (no reduce).
 static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
                                double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, PartPlan& plan,
-                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr, TiledBufs tiled = {}) {
+                               cudaStream_t st, bool with_latent = true, AuxStream* aux = nullptr, TiledBufs tiled = {},
+                               InputGrad ig = {}) {
     if (batch > 0) {
         const Layout L = layout(d, batch);
         const int64_t rows = (int64_t)batch * d->n_particles;
         const int nl = d->n_levels;
         int cur = 0;
+        double* gp = nullptr;   // input gradient: dL/dp of the levels
+        double* ig_gA = nullptr;
+        if (ig.g_p4) {
+            const InputGradScratch G = input_grad_scratch(d, batch);
+            gp = ig.scratch + G.gp;
+            ig_gA = tiled.gA ? tiled.gA : ig.scratch + G.gA;
+            if (cudaMemsetAsync(gp, 0, (size_t)rows * 4 * sizeof(double), st) != cudaSuccess) return check_launch("memset gp");
+        }
         if (with_latent)   // otherwise the fused bridge adjoint already left dL/dS, dL/dV of the last level in gS[0], gV[0]
             LGAE_TRY(run_enc_latent_bwd(d, theta, batch, ws + L.S[nl], ws + L.V[nl], sel, g_lat00, g_lat11, ws + L.gS[cur], ws + L.gV[cur], &plan, st));
         // The scalar features of the last level only reach the latent scalars: without a gradient on those the
@@ -470,8 +509,11 @@ static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, cons
             } else {
                 if (L.rsave[l] < 0 || L.gr[l] < 0) return LGAE_E_UNSUPPORTED;
                 LGAE_TRY(run_level_bwd(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ws + L.sums[l], ws + L.rsave[l],
-                                       ws + L.gr[l], g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st));
+                                       ws + L.gr[l], g_spre, ws + L.gV[cur], ws + L.gS[cur ^ 1], ws + L.gV[cur ^ 1], nullptr, &plan, st,
+                                       ig_gA));
             }
+            if (gp)   // before the next level's adjoint overwrites gA
+                LGAE_TRY(run_pgrad_level(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], ig_gA, gp, st));
             if (aux && l == 0) {
                 // the input-map adjoint (small) runs next to the last radial adjoint; both only feed the final reduce
                 LGAE_CUDA_TRY(cudaEventRecord(aux->fork[1], st), "aux fork");
@@ -490,6 +532,9 @@ static int enc_backward_launch(const LgaeModelDesc* d, const double* theta, cons
             LGAE_CUDA_TRY(cudaStreamWaitEvent(st, aux->join[2], 0), "aux join wait");
         else
             LGAE_TRY(run_enc_input_bwd(d, p4, ws + L.mass, batch, ws + L.gS[cur], ws + L.gV[cur], &plan, st));
+        if (gp)
+            LGAE_TRY(run_pgrad_input(d, theta, p4, batch, ws + L.gS[cur], ws + L.gV[cur], gp, has_input_scale(d) ? d->input_scale : 1.0,
+                                     ig.g_p4, st));
     }
     return LGAE_OK;
 }
@@ -569,18 +614,58 @@ int lgae_encoder_forward(const LgaeModelDesc* d, const double* theta, const doub
     return enc_forward_launch(d, theta, x, node_mask, batch, ws, lat00, lat11, sel, true, (cudaStream_t)stream);
 }
 
+}  // extern "C"
+
+// lgae_encoder_backward(_p4) and lgae_encoder_backward_tiled(_p4); ig.g_p4 == nullptr: no input gradient.
+static int encoder_backward_impl(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
+                                 double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
+                                 double* partials_or_scratch, double l1_lambda, double* loss_accumulate, bool tiled, InputGrad ig,
+                                 void* stream) {
+    LGAE_TRY(check_desc(d));
+    if (d->is_decoder || !theta || !gtheta || !partials_or_scratch || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
+    if (ig.g_p4 && batch > 0 && !ig.scratch) return LGAE_E_BADARG;
+    // before anything is launched
+    if (tiled) LGAE_TRY(tiled_check(d));
+    else if (d->n_particles > 32) return LGAE_E_UNSUPPORTED;   // the per-lane adjoint holds one particle per lane
+    if (ig.g_p4) LGAE_TRY(pgrad_check(d));
+    PartPlan plan;
+    TiledBufs bufs;
+    if (tiled) {
+        const TiledScratch T = tiled_scratch(d, batch);
+        plan.base = partials_or_scratch + T.part;
+        bufs = TiledBufs{partials_or_scratch + T.gA, partials_or_scratch + T.gr};
+    } else {
+        plan.base = partials_or_scratch;
+    }
+    int rc = LGAE_OK;
+    p4 = scaled_input(d, p4, batch, ws, false, (cudaStream_t)stream, &rc);   // the forward left the scaled momenta in the workspace
+    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream, true, nullptr,
+                                 bufs, ig));
+    return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
+}
+
+extern "C" {
+
 int lgae_encoder_backward(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
                           double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
                           double* partials, double l1_lambda, double* loss_accumulate, void* stream) {
-    LGAE_TRY(check_desc(d));
-    if (d->is_decoder || !theta || !gtheta || !partials || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
-    if (d->n_particles > 32) return LGAE_E_UNSUPPORTED;   // before anything is launched: the adjoint holds one particle per lane
-    PartPlan plan;
-    plan.base = partials;
-    int rc = LGAE_OK;
-    p4 = scaled_input(d, p4, batch, ws, false, (cudaStream_t)stream, &rc);   // the forward left the scaled momenta in the workspace
-    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream));
-    return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
+    return encoder_backward_impl(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, gtheta, partials, l1_lambda, loss_accumulate,
+                                 false, InputGrad{}, stream);
+}
+
+int lgae_encoder_backward_p4(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
+                             double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
+                             double* partials, double l1_lambda, double* loss_accumulate, double* g_p4, double* gp_scratch, void* stream) {
+    return encoder_backward_impl(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, gtheta, partials, l1_lambda, loss_accumulate,
+                                 false, InputGrad{g_p4, gp_scratch}, stream);
+}
+
+int64_t lgae_encoder_input_grad_scratch_doubles(const LgaeModelDesc* d, int32_t batch) {
+    const int rc = check_desc(d);
+    if (rc == LGAE_E_BADARG || batch < 0 || d->is_decoder) return -1;
+    if (rc != LGAE_OK || pgrad_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    if (d->n_particles > 32 && tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;   // the tiled adjoint runs these jets
+    return input_grad_scratch(d, batch).total;
 }
 
 int lgae_decoder_forward(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws, double* recon,
@@ -610,17 +695,16 @@ int lgae_decoder_backward(const LgaeModelDesc* d, const double* theta, const dou
 int lgae_encoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
                                 double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
                                 double* scratch, double l1_lambda, double* loss_accumulate, void* stream) {
-    LGAE_TRY(check_desc(d));
-    if (d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
-    LGAE_TRY(tiled_check(d));
-    const TiledScratch T = tiled_scratch(d, batch);
-    PartPlan plan;
-    plan.base = scratch + T.part;
-    int rc = LGAE_OK;
-    p4 = scaled_input(d, p4, batch, ws, false, (cudaStream_t)stream, &rc);
-    LGAE_TRY(enc_backward_launch(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, plan, (cudaStream_t)stream, true, nullptr,
-                                 TiledBufs{scratch + T.gA, scratch + T.gr}));
-    return run_reduce_plan(&plan, d->n_params, gtheta, theta, l1_lambda, loss_accumulate, (cudaStream_t)stream);
+    return encoder_backward_impl(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, gtheta, scratch, l1_lambda, loss_accumulate,
+                                 true, InputGrad{}, stream);
+}
+
+int lgae_encoder_backward_tiled_p4(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
+                                   double* ws, const int32_t* sel, const double* g_lat00, const double* g_lat11, double* gtheta,
+                                   double* scratch, double l1_lambda, double* loss_accumulate, double* g_p4, double* gp_scratch,
+                                   void* stream) {
+    return encoder_backward_impl(d, theta, p4, node_mask, batch, ws, sel, g_lat00, g_lat11, gtheta, scratch, l1_lambda, loss_accumulate,
+                                 true, InputGrad{g_p4, gp_scratch}, stream);
 }
 
 int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws,
@@ -860,6 +944,21 @@ int lgae_normalize_p4(const double* p4, int32_t batch, int32_t n, double* out, d
     if (batch < 0 || n < 1 || (batch > 0 && (!p4 || !out))) return LGAE_E_BADARG;
     if (batch == 0) return LGAE_OK;
     return run_normalize(p4, batch, n, out, factor, (cudaStream_t)stream);
+}
+
+int lgae_normalize_p4_backward(const double* p4, int32_t batch, int32_t n, const double* g_out, const double* g_factor, double* g_p4,
+                               void* stream) {
+    if (batch < 0 || n < 1 || (batch > 0 && (!p4 || !g_p4))) return LGAE_E_BADARG;
+    if (batch == 0) return LGAE_OK;
+    return run_normalize_bwd(p4, batch, n, g_out, g_factor, g_p4, (cudaStream_t)stream);
+}
+
+int lgae_chamfer_target_grad(const double* recon, const double* target, int32_t batch, int32_t n, int32_t m, int32_t get_real,
+                             const double* g_loss, double* g_target, void* stream) {
+    if (batch < 0 || n < 1 || m < 1 || (batch > 0 && (!recon || !target || !g_target))) return LGAE_E_BADARG;
+    if (get_real < LGAE_GET_REAL_REAL || get_real > LGAE_GET_REAL_NORM) return LGAE_E_BADARG;
+    if (batch == 0) return LGAE_OK;
+    return run_chamfer_target_grad(recon, target, batch, n, m, get_real, g_loss, g_target, (cudaStream_t)stream);
 }
 
 int lgae_l1(const double* theta, int64_t n, double lambda, double* out_accumulate, double* gtheta_accumulate, void* stream) {

@@ -604,8 +604,10 @@ LGAE_DEV void mix_adjoint_block(int k, int Cout, int C5, int nm, int lane, const
 //      g_r for radial_bwd_kernel; role 2 (own = neighbour) accumulates dL/dS_lane, dL/dV_lane in registers; R_{lane,o} is
 //      streamed from r_save, prefetched.  Decoder: adjoint of the O(N) closed form (constant radial weights);
 //   3. when the CTA runs out of jets: one compact row of parameter-gradient partials (mix weights, decoder biases).
-template <bool ENC, int MAXT, int MINB>
-__global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a) {
+// GA (encoder): also write gA, the adjoints of the neighbour sums, to g_a (B,N,C,10) complex for the input-gradient kernels
+// (lgae_input_grad.cu).
+template <bool ENC, bool GA>
+LGAE_DEV void level_bwd_body(const LevelArgs& a, double* g_a) {
     extern __shared__ __align__(128) double smem[];
     const int N = a.N, C = a.C, Cout = a.Cout;
     const int tid = threadIdx.x, lane = tid & 31, c = tid >> 5;
@@ -748,6 +750,11 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
             }
         }
         __syncthreads();  // gA_s of every channel is complete (role 2 reads other lanes' entries)
+        if (GA && live) {
+            cplx* dst = reinterpret_cast<cplx*>(g_a) + ((int64_t)(b * N + i) * C + c) * 10;
+#pragma unroll
+            for (int e = 0; e < 10; ++e) dst[e] = gA_s[(c * 10 + e) * 32 + lane];
+        }
         // ---- 2. adjoint of the neighbour sums ----
         cplx gy[4] = {czero(), czero(), czero(), czero()};
         if (!ENC) {
@@ -950,6 +957,11 @@ __global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a
     }
 }
 
+template <bool ENC, int MAXT, int MINB>
+__global__ void __launch_bounds__(MAXT, MINB) level_bwd_kernel(const LevelArgs a) { level_bwd_body<ENC, false>(a, nullptr); }
+template <int MAXT, int MINB>
+__global__ void __launch_bounds__(MAXT, MINB) level_bwd_ga_kernel(const LevelArgs a, double* g_a) { level_bwd_body<true, true>(a, g_a); }
+
 // ------------------------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------------------------
@@ -969,7 +981,7 @@ static int launch_level_fwd(const LevelArgs& a, cudaStream_t st) {
 }
 
 template <bool ENC>
-static int launch_level_bwd(const LevelArgs& a, int grid, cudaStream_t st) {
+static int launch_level_bwd(const LevelArgs& a, int grid, cudaStream_t st, double* g_a) {
     if (a.N > 32) return LGAE_E_UNSUPPORTED;
     const LevelBwdSmem L = level_bwd_smem(ENC, a.N, a.C, a.Cout);
     const size_t bytes = (size_t)L.total * sizeof(double);
@@ -977,6 +989,14 @@ static int launch_level_bwd(const LevelArgs& a, int grid, cudaStream_t st) {
     LaunchScope ls_("level_bwd", st);
 #define LGAE_LAUNCH(MAXT, MINB)                                               \
     {                                                                         \
+        if constexpr (ENC) {                                                  \
+            if (g_a) {                                                        \
+                auto kern = level_bwd_ga_kernel<MAXT, (MINB)>;                \
+                if (int rc = ensure_smem((const void*)kern, bytes)) return rc; \
+                launch_k(kern, dim3(grid), dim3(32 * a.C), bytes, st, a, g_a); \
+                return check_launch("level_bwd");                             \
+            }                                                                 \
+        }                                                                     \
         auto kern = level_bwd_kernel<ENC, MAXT, (MINB)>;                      \
         if (int rc = ensure_smem((const void*)kern, bytes)) return rc;        \
         launch_k(kern, dim3(grid), dim3(32 * a.C), bytes, st, a);                               \
@@ -1038,10 +1058,11 @@ int run_level_fwd(const LgaeModelDesc* d, int level, const double* theta, const 
 }
 
 // Adjoint of one level (without the adjoint of the radial functions: the encoder streams dL/dR to g_r for
-// run_radial_bwd).  Reserves a block of `plan` for the per-CTA partial rows and declares its segments.
+// run_radial_bwd).  Reserves a block of `plan` for the per-CTA partial rows and declares its segments.  Encoder with g_a != NULL:
+// also writes the adjoints of the neighbour sums to g_a (B,N,C,10) complex, for the input gradient.
 int run_level_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
                   const double* s_in, const double* v_in, const double* sums, const double* r_save, double* g_r, const double* g_s_pre,
-                  const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st) {
+                  const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st, double* g_a) {
     if (!d || level < 0 || level >= d->n_levels || !plan) return LGAE_E_BADARG;
     if (batch <= 0) return LGAE_OK;
     LevelArgs a;
@@ -1068,7 +1089,7 @@ int run_level_bwd(const LgaeModelDesc* d, int level, const double* theta, const 
     seg(a.off_m00, a.po_m00, nm2); seg(a.off_m11, a.po_m11, nm2);
     if (rc != LGAE_OK) return rc;
     if (a.C < 1 || a.C > LGAE_MAX_CHANNELS || a.Cout < 1 || a.Cout > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
-    return enc ? launch_level_bwd<true>(a, grid, st) : launch_level_bwd<false>(a, grid, st);
+    return enc ? launch_level_bwd<true>(a, grid, st, g_a) : launch_level_bwd<false>(a, grid, st, nullptr);
 }
 
 // Width (doubles) of one row of partials of the level adjoint.

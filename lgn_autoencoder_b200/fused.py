@@ -199,6 +199,29 @@ def encoder_backward_tiled_raw(plan: FusedPlan, theta, p4, node_mask, ws, sel, g
     return gtheta
 
 
+def encoder_backward_p4_raw(plan: FusedPlan, theta, p4, node_mask, ws, sel, g00, g11, tiled: bool):
+    """The encoder adjoint with the gradient with respect to p4 (lgae_encoder_backward_p4 / _tiled_p4) -> (gtheta, g_p4)."""
+    lib = plan._lib
+    dev = p4.device
+    b = p4.shape[0]
+    gtheta = torch.empty(plan.n_params, dtype=torch.float64, device=dev)
+    g_p4 = torch.empty_like(p4)
+    n = lib.lgae_encoder_input_grad_scratch_doubles(C.byref(plan.desc), b)
+    if n < 0:
+        raise NotImplementedError("input gradient not supported by the fused B200 path for this configuration")
+    gp = torch.empty(max(int(n), 1), dtype=torch.float64, device=dev)
+    if tiled:
+        scratch = plan.tiled_scratch(b, dev)
+        check(lib.lgae_encoder_backward_tiled_p4(C.byref(plan.desc), ptr(theta), ptr(p4), ptr(node_mask), b, ptr(ws), ptr(sel), ptr(g00),
+                                                 ptr(g11), ptr(gtheta), ptr(scratch), 0.0, None, ptr(g_p4), ptr(gp), _stream()),
+              "encoder_backward_tiled_p4")
+    else:
+        part = plan.partials(b, dev)
+        check(lib.lgae_encoder_backward_p4(C.byref(plan.desc), ptr(theta), ptr(p4), ptr(node_mask), b, ptr(ws), ptr(sel), ptr(g00),
+                                           ptr(g11), ptr(gtheta), ptr(part), 0.0, None, ptr(g_p4), ptr(gp), _stream()), "encoder_backward_p4")
+    return gtheta, g_p4
+
+
 def decoder_forward_raw(plan: FusedPlan, theta, lat11, want_gen00: bool = False):
     lib = plan._lib
     b = lat11.shape[1]
@@ -276,6 +299,10 @@ class _EncoderFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g00, g11):
         plan = ctx.plan
+        if ctx.needs_input_grad[2]:
+            gtheta, g_p4 = encoder_backward_p4_raw(plan, ctx.theta, ctx.p4, ctx.node_mask, ctx.ws, ctx.sel, _contig(g00), _contig(g11),
+                                                   tiled=plan.n_particles > 32)
+            return None, gtheta, g_p4, None, None
         bwd = encoder_backward_raw if plan.n_particles <= 32 else encoder_backward_tiled_raw   # one particle per lane, or tiled
         gtheta = bwd(plan, ctx.theta, ctx.p4, ctx.node_mask, ctx.ws, ctx.sel, _contig(g00), _contig(g11))
         return None, gtheta, None, None, None
@@ -320,13 +347,20 @@ class _ChamferFn(torch.autograd.Function):
         jet = torch.empty(b, dtype=torch.float64, device=dev)
         g = torch.empty_like(recon)
         check(lib.lgae_chamfer(ptr(recon), ptr(target), b, n, m, mode, ptr(loss), ptr(jet), None, ptr(g), _stream()), "chamfer")
-        ctx.save_for_backward(g)
+        ctx.save_for_backward(g, recon, target)
+        ctx.mode = mode
         return loss
 
     @staticmethod
     def backward(ctx, g_loss):
-        (g,) = ctx.saved_tensors
-        return g * g_loss, None, None
+        g, recon, target = ctx.saved_tensors
+        g_target = None
+        if ctx.needs_input_grad[1]:
+            g_loss = g_loss.contiguous()
+            g_target = torch.empty_like(target)
+            check(_lib.load().lgae_chamfer_target_grad(ptr(recon), ptr(target), recon.shape[1], recon.shape[2], target.shape[1], ctx.mode,
+                                                       ptr(g_loss), ptr(g_target), _stream()), "chamfer_target_grad")
+        return g * g_loss, g_target, None
 
 
 def chamfer_loss(recon: torch.Tensor, target: torch.Tensor, get_real: str = "real") -> torch.Tensor:
@@ -364,11 +398,28 @@ def anomaly_scores(recon: torch.Tensor, target: torch.Tensor, get_real: str = "r
     return {name: out[:, i] for i, name in enumerate(SCORE_NAMES)}
 
 
+class _NormalizeFn(torch.autograd.Function):
+    """normalize_p4 'overall_max'; the adjoint routes the factor's gradient to the maxima as torch's amax does."""
+
+    @staticmethod
+    def forward(ctx, p4):
+        lib = _lib.load()
+        p4 = p4.contiguous()
+        out = torch.empty_like(p4)
+        f = torch.empty((p4.shape[0], 1, 1), dtype=torch.float64, device=p4.device)
+        check(lib.lgae_normalize_p4(ptr(p4), p4.shape[0], p4.shape[1], ptr(out), ptr(f), _stream()), "normalize_p4")
+        ctx.save_for_backward(p4)
+        return out, f
+
+    @staticmethod
+    def backward(ctx, g_out, g_f):
+        (p4,) = ctx.saved_tensors
+        g_p4 = torch.empty_like(p4)
+        check(_lib.load().lgae_normalize_p4_backward(ptr(p4), p4.shape[0], p4.shape[1], ptr(_contig(g_out)), ptr(_contig(g_f)), ptr(g_p4),
+                                                     _stream()), "normalize_p4_backward")
+        return g_p4
+
+
 def normalize_p4(p4: torch.Tensor):
-    """normalize_p4(p4, 'overall_max') (utils/normalize_p4.py:39-52) -> (normalised, factor (B,1,1))."""
-    lib = _lib.load()
-    p4 = p4.contiguous()
-    out = torch.empty_like(p4)
-    f = torch.empty(p4.shape[0], dtype=torch.float64, device=p4.device)
-    check(lib.lgae_normalize_p4(ptr(p4), p4.shape[0], p4.shape[1], ptr(out), ptr(f), _stream()), "normalize_p4")
-    return out, f.view(-1, 1, 1)
+    """normalize_p4(p4, 'overall_max') (utils/normalize_p4.py:39-52) -> (normalised, factor (B,1,1)), differentiable in p4."""
+    return _NormalizeFn.apply(p4)
