@@ -50,6 +50,17 @@ extern "C" {
 #define LGAE_LATENT_SUM 4
 #define LGAE_LATENT_MIX 5    /* nodes x channels mixed by the latent MixReps; no pooling                  */
 
+/* CGMLP activations (LgaeModelDesc::mlp_activation), the reference's get_activation_fn table.  Any other code is
+ * refused with LGAE_E_UNSUPPORTED when has_mlp is set. */
+#define LGAE_ACT_LEAKYRELU 0 /* LeakyReLU(0.01)                                                           */
+#define LGAE_ACT_RELU 1
+#define LGAE_ACT_ELU 2       /* alpha = 1                                                                  */
+#define LGAE_ACT_SIGMOID 3
+#define LGAE_ACT_LOGSIGMOID 4
+#define LGAE_ACT_TANH 5
+#define LGAE_ACT_ATAN 6
+#define LGAE_ACT_COUNT 7
+
 /* get_real modes (utils/utils.py:194-207): how the complex reconstruction becomes the real 4-momenta the loss sees.
  * The reference's default is 'real' (main.py:295-300); examples/main.sh and the benchmarked configuration use 'sum'. */
 #define LGAE_GET_REAL_REAL 0
@@ -72,7 +83,7 @@ typedef struct LgaeModelDesc {
     int32_t mlp_width[LGAE_MAX_LEVELS];     /* hidden width of level l = mlp_width_mul * 2 * C_{l+1}        */
     int32_t latent_mode;                    /* encoder: LGAE_LATENT_*                                       */
     int32_t tau_s, tau_v;                   /* encoder: latent MixReps outputs; decoder: latent inputs      */
-    int32_t reserved;
+    int32_t mlp_activation;                 /* CGMLP hidden-layer activation: LGAE_ACT_* (0: LeakyReLU(0.01))  */
     int64_t n_params;                       /* length of theta                                              */
     int64_t off_in00, off_in11;             /* input_func_node.weights.(0, 0) / (1, 1): (2, C_0, 1)         */
     int64_t off_rad_a[LGAE_MAX_LEVELS], off_rad_b[LGAE_MAX_LEVELS], off_rad_c[LGAE_MAX_LEVELS];

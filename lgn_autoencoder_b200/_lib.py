@@ -13,6 +13,8 @@ MAX_LINEAR = 12
 MAX_CHANNELS = 8
 
 LATENT_MODES = {"mean": 0, "average": 0, "min&max": 1, "min": 2, "max": 3, "sum": 4, "mix": 5}
+# CGMLP activations (LGAE_ACT_*): the names of the reference's get_activation_fn table
+ACTIVATIONS = {"leakyrelu": 0, "relu": 1, "elu": 2, "sigmoid": 3, "logsigmoid": 4, "tanh": 5, "atan": 6}
 
 
 class LgaeModelDesc(C.Structure):
@@ -28,7 +30,7 @@ class LgaeModelDesc(C.Structure):
         ("latent_mode", C.c_int32),
         ("tau_s", C.c_int32),
         ("tau_v", C.c_int32),
-        ("reserved", C.c_int32),
+        ("mlp_activation", C.c_int32),
         ("n_params", C.c_int64),
         ("off_in00", C.c_int64),
         ("off_in11", C.c_int64),

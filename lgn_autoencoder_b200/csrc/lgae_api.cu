@@ -243,6 +243,7 @@ static int check_desc(const LgaeModelDesc* d) {
     for (int l = 0; l <= d->n_levels; ++l)
         if (d->channels[l] < 1 || d->channels[l] > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
     if (d->has_mlp && (d->mlp_hidden < 1 || d->mlp_hidden + 1 > LGAE_MAX_LINEAR)) return LGAE_E_UNSUPPORTED;
+    if (d->has_mlp && (d->mlp_activation < 0 || d->mlp_activation >= LGAE_ACT_COUNT)) return LGAE_E_UNSUPPORTED;
     return LGAE_OK;
 }
 

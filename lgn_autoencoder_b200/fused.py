@@ -14,7 +14,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from ._lib import LATENT_MODES, LgaeModelDesc, check, ptr
+from ._lib import ACTIVATIONS, LATENT_MODES, LgaeModelDesc, check, ptr
 
 GET_REAL_MODES = {"real": 0, "imag": 1, "sum": 2, "mean": 3, "norm": 4}
 
@@ -38,7 +38,7 @@ class FusedPlan:
 
     def __init__(self, kind: str, shapes: "OrderedDict[str, Tuple[int, ...]]", *, n_particles: int, channels: Sequence[int],
                  num_basis_fn: int = 10, mlp: bool = True, mlp_depth: int = 6, mlp_width: int = 6, latent_mode: str = "mean",
-                 tau_s: int = 1, tau_v: int = 1, input_scale: float = 1.0):
+                 tau_s: int = 1, tau_v: int = 1, input_scale: float = 1.0, activation: str = "leakyrelu"):
         assert kind in ("encoder", "decoder")
         self.kind = kind
         self.names: List[str] = list(shapes)
@@ -67,6 +67,9 @@ class FusedPlan:
             d.channels[i] = c
         d.has_mlp = 1 if mlp else 0
         d.mlp_hidden = int(mlp_depth)
+        if activation.lower() not in ACTIVATIONS:
+            raise ValueError(f"Activation function {activation} not implemented!")
+        d.mlp_activation = ACTIVATIONS[activation.lower()]
         d.tau_s, d.tau_v = self.tau_s, self.tau_v
         d.n_params = self.n_params
         d.input_scale = float(input_scale)   # encoder: p4 * scale (lgn_encoder.py:371), applied inside the library

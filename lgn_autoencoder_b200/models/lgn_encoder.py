@@ -77,7 +77,8 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         if self._fused_reason is None:
             self._build_plan("encoder", n_particles=self.num_input_particles, channels=list(num_channels), num_basis_fn=num_basis_fn,
                              mlp=mlp, mlp_depth=mlp_depth if mlp else 0, mlp_width=mlp_width if mlp else 0,
-                             latent_mode=map_to_latent, tau_s=tau_latent_scalars, tau_v=tau_latent_vectors, input_scale=scale)
+                             latent_mode=map_to_latent, tau_s=tau_latent_scalars, tau_v=tau_latent_vectors, input_scale=scale,
+                             activation=activation)
             if self.num_input_particles > 32:
                 self._tiled_reason = self._plan.tiled_reason()
 
@@ -96,8 +97,8 @@ class LGNEncoder(FusedParamsMixin, CGModule):
             return f"map_to_latent {self.map_to_latent!r}"
         if max(self.num_channels) > 8:
             return "more than 8 channels"
-        if self.mlp and (self.activation.lower() != "leakyrelu" or not self.mlp_depth or self.mlp_depth < 1):
-            return "MLP activation other than leakyrelu / depth 0"
+        if self.mlp and (not self.mlp_depth or self.mlp_depth < 1):
+            return "MLP depth 0"
         if self.mlp and any(((self.mlp_width * 2 * c + 7) // 8) > 6 for c in self.num_channels[1:]):
             return "MLP hidden width above 48 (the fused MLP keeps all layers' weights in shared memory)"
         if 2 * self.num_basis_fn > 32:
