@@ -6,7 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SOURCES = ["lgae_api.cu", "lgae_glue.cu", "lgae_level.cu", "lgae_radial.cu", "lgae_mlp.cu", "lgae_cg.cu", "lgae_layers.cu", "lgae_optim.cu", "lgae_collective.cu",
-           "lgae_input_grad.cu", "lgae_mlp_act_relu.cu", "lgae_mlp_act_sigmoid.cu", "lgae_mlp_act_tanh.cu"]
+           "lgae_input_grad.cu", "lgae_mlp_act_relu.cu", "lgae_mlp_act_sigmoid.cu", "lgae_mlp_act_tanh.cu",
+           *[f"lgae_mlp_streamed_{a}.cu" for a in ("leakyrelu", "relu", "elu", "sigmoid", "logsigmoid", "tanh", "atan")]]
 LIB = os.path.join(HERE, "liblgae_b200.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 

@@ -55,6 +55,7 @@ int run_mlp_pack(const LgaeModelDesc* d, const double* theta, double* out, const
 int mlp_padded_width(const LgaeModelDesc* d, int level);
 int64_t mlp_part_width(const LgaeModelDesc* d, int level);
 int mlp_bwd_grid();
+bool mlp_tiling_supported(const LgaeModelDesc* d, int level);
 int run_enc_input(const LgaeModelDesc* d, const double* theta, const double* p4, int B, double* mass, double* S, double* V, cudaStream_t st);
 int run_enc_input_bwd(const LgaeModelDesc* d, const double* p4, const double* mass, int B, const double* gS, const double* gV, PartPlan* plan, cudaStream_t st);
 int run_enc_latent(const LgaeModelDesc* d, const double* theta, int B, const double* S, const double* V, double* lat00, double* lat11, int32_t* sel, cudaStream_t st, int parts = 3);
@@ -244,6 +245,8 @@ static int check_desc(const LgaeModelDesc* d) {
         if (d->channels[l] < 1 || d->channels[l] > LGAE_MAX_CHANNELS) return LGAE_E_UNSUPPORTED;
     if (d->has_mlp && (d->mlp_hidden < 1 || d->mlp_hidden + 1 > LGAE_MAX_LINEAR)) return LGAE_E_UNSUPPORTED;
     if (d->has_mlp && (d->mlp_activation < 0 || d->mlp_activation >= LGAE_ACT_COUNT)) return LGAE_E_UNSUPPORTED;
+    for (int l = 0; d->has_mlp && l < d->n_levels; ++l)
+        if (!mlp_tiling_supported(d, l)) return LGAE_E_UNSUPPORTED;   // hidden width above 96: no MLP kernel takes it
     return LGAE_OK;
 }
 

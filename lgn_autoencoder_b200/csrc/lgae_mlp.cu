@@ -1,8 +1,9 @@
-// CGMLP (lgn/models/lgn_levels.py:191-227): weight packing and the dispatch of the MLP kernels (lgae_mlp.cuh) by activation
-// and tiling; the LeakyReLU kernels are instantiated here.
+// CGMLP (lgn/models/lgn_levels.py:191-227): weight packing and the dispatch of the MLP kernels (lgae_mlp.cuh, and
+// lgae_mlp_streamed.cuh for the layers those cannot hold) by activation and tiling; the resident LeakyReLU kernels are
+// instantiated here.
 #include <cstring>
 
-#include "lgae_mlp.cuh"
+#include "lgae_mlp_streamed.cuh"
 
 namespace lgae {
 
@@ -102,10 +103,17 @@ LGAE_MLP_INSTANCES(extern, LGAE_ACT_SIGMOID)
 LGAE_MLP_INSTANCES(extern, LGAE_ACT_LOGSIGMOID)
 LGAE_MLP_INSTANCES(extern, LGAE_ACT_TANH)
 LGAE_MLP_INSTANCES(extern, LGAE_ACT_ATAN)
+// The streamed kernels come from lgae_mlp_streamed_*.cu, one unit per activation.
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_LEAKYRELU)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_RELU)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_ELU)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_SIGMOID)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_LOGSIGMOID)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_TANH)
+LGAE_MLP_STREAMED_INSTANCES(extern, LGAE_ACT_ATAN)
 
-// nti = ceil(2C'/8): 1 for C' <= 4 output channels, 2 for C' = 5..8.  The hidden width is mlp_width * 2C' >= nin, and the
-// modules admit widths up to 48 (ntw <= 6), so with nti = 2 every ntw from 2 to 6 is reachable.  (LGAE_MLP_INSTANCES in
-// lgae_mlp.cuh lists the same tilings.)
+// nti = ceil(2C'/8): 1 for C' <= 4 output channels, 2 for C' = 5..8.  The hidden width is mlp_width * 2C' >= nin, so with
+// nti = 2 every ntw from 2 to 6 is reachable.  (LGAE_MLP_INSTANCES in lgae_mlp.cuh lists the same tilings.)
 template <int ACT>
 static int launch_mlp_shape(MlpArgs& a, int ntw, int nti, bool bwd, cudaStream_t st) {
 #define LGAE_MLP_CASE(W, I) \
@@ -115,6 +123,34 @@ static int launch_mlp_shape(MlpArgs& a, int ntw, int nti, bool bwd, cudaStream_t
     LGAE_MLP_CASE(2, 2) LGAE_MLP_CASE(3, 2) LGAE_MLP_CASE(4, 2) LGAE_MLP_CASE(5, 2) LGAE_MLP_CASE(6, 2)
     LGAE_MLP_CASE(8, 2) LGAE_MLP_CASE(9, 2)
 #undef LGAE_MLP_CASE
+    return LGAE_E_UNSUPPORTED;
+}
+
+// The streamed kernels' range: hidden widths 49..96 (LGAE_MLP_STREAMED_INSTANCES lists the same tilings).
+static bool mlp_streamed_tiling(int ntw, int nti) { return ntw >= 7 && ntw <= 12 && nti >= 1 && nti <= 2; }
+
+// The tilings one of the two families takes: the resident instances cover nti <= ntw <= 6 and (8, 2), (9, 2), the streamed
+// kernels 7 <= ntw <= 12.  (Whether a resident instance's shared memory holds all layers at the model's depth is decided at
+// launch; the streamed kernels take the ones it does not in their range.)
+bool mlp_tiling_supported(const LgaeModelDesc* d, int level) {
+    const int ntw = (d->mlp_width[level] + 7) / 8, nti = (2 * d->channels[level + 1] + 7) / 8;
+    return nti >= 1 && nti <= 2 && ntw >= nti && ntw <= 12;
+}
+
+// Resident kernels wherever they have an instance whose shared memory holds all layers; the streamed kernels exactly where
+// they do not.  Both read the same packed weights and write the same activations and partial rows, so a level may run the
+// resident forward and the streamed adjoint.
+template <int ACT>
+static int launch_mlp_any(MlpArgs& a, int ntw, int nti, bool bwd, cudaStream_t st) {
+    const int rc = launch_mlp_shape<ACT>(a, ntw, nti, bwd, st);
+    if (rc != LGAE_E_UNSUPPORTED || !mlp_streamed_tiling(ntw, nti)) return rc;
+#define LGAE_MLP_STREAMED_CASE(W)                                      \
+    if (ntw == W)                                                      \
+        return nti == 1 ? launch_mlp_streamed<W, 1, ACT>(a, bwd, st) \
+                        : launch_mlp_streamed<W, 2, ACT>(a, bwd, st);
+    LGAE_MLP_STREAMED_CASE(7) LGAE_MLP_STREAMED_CASE(8) LGAE_MLP_STREAMED_CASE(9)
+    LGAE_MLP_STREAMED_CASE(10) LGAE_MLP_STREAMED_CASE(11) LGAE_MLP_STREAMED_CASE(12)
+#undef LGAE_MLP_STREAMED_CASE
     return LGAE_E_UNSUPPORTED;
 }
 
@@ -154,13 +190,13 @@ int run_mlp(const LgaeModelDesc* d, int level, const double* theta, const double
     }
     const int ntw = (a.width + 7) / 8, nti = (a.nin + 7) / 8;
     switch (d->mlp_activation) {
-        case LGAE_ACT_LEAKYRELU: return launch_mlp_shape<LGAE_ACT_LEAKYRELU>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_RELU: return launch_mlp_shape<LGAE_ACT_RELU>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_ELU: return launch_mlp_shape<LGAE_ACT_ELU>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_SIGMOID: return launch_mlp_shape<LGAE_ACT_SIGMOID>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_LOGSIGMOID: return launch_mlp_shape<LGAE_ACT_LOGSIGMOID>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_TANH: return launch_mlp_shape<LGAE_ACT_TANH>(a, ntw, nti, bwd, st);
-        case LGAE_ACT_ATAN: return launch_mlp_shape<LGAE_ACT_ATAN>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_LEAKYRELU: return launch_mlp_any<LGAE_ACT_LEAKYRELU>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_RELU: return launch_mlp_any<LGAE_ACT_RELU>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_ELU: return launch_mlp_any<LGAE_ACT_ELU>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_SIGMOID: return launch_mlp_any<LGAE_ACT_SIGMOID>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_LOGSIGMOID: return launch_mlp_any<LGAE_ACT_LOGSIGMOID>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_TANH: return launch_mlp_any<LGAE_ACT_TANH>(a, ntw, nti, bwd, st);
+        case LGAE_ACT_ATAN: return launch_mlp_any<LGAE_ACT_ATAN>(a, ntw, nti, bwd, st);
         default: return LGAE_E_UNSUPPORTED;
     }
 }

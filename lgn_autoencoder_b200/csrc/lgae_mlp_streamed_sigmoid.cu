@@ -1,0 +1,8 @@
+// Streamed-weight CGMLP kernels (lgae_mlp_streamed.cuh) with the sigmoid activation.
+#include "lgae_mlp_streamed.cuh"
+
+namespace lgae {
+
+LGAE_MLP_STREAMED_INSTANCES(, LGAE_ACT_SIGMOID)
+
+}  // namespace lgae

@@ -99,8 +99,8 @@ class LGNEncoder(FusedParamsMixin, CGModule):
             return "more than 8 channels"
         if self.mlp and (not self.mlp_depth or self.mlp_depth < 1):
             return "MLP depth 0"
-        if self.mlp and any(((self.mlp_width * 2 * c + 7) // 8) > 6 for c in self.num_channels[1:]):
-            return "MLP hidden width above 48 (the fused MLP keeps all layers' weights in shared memory)"
+        if self.mlp and any(((self.mlp_width * 2 * c + 7) // 8) > 12 for c in self.num_channels[1:]):
+            return "MLP hidden width above 96"
         if 2 * self.num_basis_fn > 32:
             return "more than 16 radial basis functions"
         return None
