@@ -96,6 +96,10 @@ typedef struct LgaeModelDesc {
     int64_t off_graph00, off_graph11;       /* decoder latent_to_graph: (2, N, tau_s) / (2, N, tau_v)        */
     int64_t off_out00, off_out11;           /* decoder mix_to_output: (2, 1, C_L)                            */
     double input_scale;                     /* encoder: p4 is multiplied by this first (lgn_encoder.py:371); 0 means 1 */
+    /* Maximal irrep dimension of every level: 0 or 2 = maxdim 2 (nodes (0,0), (1,1)); 3 = maxdim 3 (nodes (0,0), (1,1), (2,0),
+     * (0,2), (2,2)), which the forward entry points run and everything else refuses with LGAE_E_UNSUPPORTED.  Others: refused. */
+    int32_t maxdim;
+    int64_t off_mix20[LGAE_MAX_LEVELS], off_mix02[LGAE_MAX_LEVELS], off_mix22[LGAE_MAX_LEVELS];   /* maxdim 3: cat_mix weights */
 } LgaeModelDesc;
 
 /* ---- library / device ---------------------------------------------------------------------------- */
@@ -121,6 +125,9 @@ int64_t lgae_workspace_doubles(const LgaeModelDesc* d, int32_t batch);
  * 6 = MLP activations of level (hidden, B*N, padded width), 7 = radial weights of level (B,N,C,32,4) (encoder, N <= 32),
  * 8 = dL/dR of level (B,N,C,32,4) (encoder, N <= 32; one buffer per level). */
 int64_t lgae_workspace_offset(const LgaeModelDesc* d, int32_t batch, int32_t kind, int32_t level);
+/* maxdim 3 (forward only): the workspace holds kinds 0, 1 (S, V: the (0,0) and (1,1) parts), 2 (pre-MLP scalars), 3 (y,
+ * decoder), 5 (masses), 6 (MLP activations) as above and kind 9 = H_in[level] (B,N,C,15,2), the (2,0) | (0,2) | (2,2) parts
+ * (level >= 1), plus the neighbour sums of the level being evaluated; no saved state for an adjoint (kinds 4, 7, 8 return -1). */
 /* Doubles of scratch for the per-CTA rows of parameter-gradient partials the backward entry points write (every
  * backward kernel owns a block of compact rows; one reduce launch sums them into gtheta, in a fixed order). */
 int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch);

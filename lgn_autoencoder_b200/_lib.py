@@ -52,6 +52,10 @@ class LgaeModelDesc(C.Structure):
         ("off_out00", C.c_int64),
         ("off_out11", C.c_int64),
         ("input_scale", C.c_double),
+        ("maxdim", C.c_int32),   # 0 / 2: maxdim 2; 3: maxdim 3 (forward entry points only)
+        ("off_mix20", C.c_int64 * MAX_LEVELS),
+        ("off_mix02", C.c_int64 * MAX_LEVELS),
+        ("off_mix22", C.c_int64 * MAX_LEVELS),
     ]
 
 

@@ -16,6 +16,11 @@ namespace lgae {
 // ---- implemented in the other translation units -------------------------------------------------------------
 int run_level_fwd(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
                   const double* s_in, const double* v_in, double* sums, double* r_save, double* s_pre, double* v_out, cudaStream_t st);
+int run_md3_level_fwd(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
+                      const double* s_in, const double* v_in, const double* h_in, double* nbr, double* s_pre, double* v_out, double* h_out,
+                      cudaStream_t st);
+int md3_level_check(const LgaeModelDesc* d);
+int64_t md3_nbr_doubles(const LgaeModelDesc* d, int level, int64_t batch);
 int run_level_bwd(const LgaeModelDesc* d, int level, const double* theta, const double* p_or_y, const uint8_t* node_mask, int batch,
                   const double* s_in, const double* v_in, const double* sums, const double* r_save, double* g_r, const double* g_s_pre,
                   const double* g_v_out, double* g_s_in, double* g_v_in, double* g_y, PartPlan* plan, cudaStream_t st,
@@ -197,6 +202,7 @@ struct Layout {
     int64_t S[LGAE_MAX_LEVELS + 1], V[LGAE_MAX_LEVELS + 1];
     int64_t sums[LGAE_MAX_LEVELS], spre[LGAE_MAX_LEVELS], acts[LGAE_MAX_LEVELS], rsave[LGAE_MAX_LEVELS], wpack[LGAE_MAX_LEVELS];
     int64_t y, mass, gS[2], gV[2], gSpre, gy, gr[LGAE_MAX_LEVELS], nrm, pscaled, total;
+    int64_t H[LGAE_MAX_LEVELS + 1], nbr;   // maxdim 3 only: (2,0) | (0,2) | (2,2) parts of the nodes, neighbour sums of one level
 };
 static bool has_input_scale(const LgaeModelDesc* d) { return !d->is_decoder && d->input_scale != 0.0 && d->input_scale != 1.0; }
 static int max_channels(const LgaeModelDesc* d) {
@@ -204,7 +210,36 @@ static int max_channels(const LgaeModelDesc* d) {
     for (int l = 0; l <= d->n_levels; ++l) m = d->channels[l] > m ? d->channels[l] : m;
     return m;
 }
+static bool is_md3(const LgaeModelDesc* d) { return d->maxdim == 3; }
+// maxdim 3 (forward only): [y | mass | S, V, H per level | spre, acts, wpack per level | nbr | pscaled]; -1 for what it lacks
+static Layout layout_md3(const LgaeModelDesc* d, int64_t B) {
+    Layout L;
+    memset(&L, 0xff, sizeof(L));
+    const int64_t nodes = B * d->n_particles;
+    int64_t o = 0;
+    auto take = [&](int64_t n) { const int64_t r = o; o += (n + 3) & ~int64_t(3); return r; };   // 32-byte granules
+    L.y = take(nodes * 8);
+    L.mass = take(nodes);
+    for (int l = 0; l <= d->n_levels; ++l) {
+        L.S[l] = take(nodes * d->channels[l] * 2);
+        L.V[l] = take(nodes * d->channels[l] * 8);
+        L.H[l] = l > 0 ? take(nodes * d->channels[l] * 30) : -1;   // level 0 holds (0,0) and (1,1) only
+    }
+    int64_t nbr = 0;
+    for (int l = 0; l < d->n_levels; ++l) {
+        L.spre[l] = d->has_mlp ? take(nodes * d->channels[l + 1] * 2) : L.S[l + 1];
+        L.acts[l] = d->has_mlp ? take((int64_t)d->mlp_hidden * nodes * mlp_padded_width(d, l)) : 0;
+        L.wpack[l] = take(mlp_pack_doubles(d, l));
+        const int64_t n = md3_nbr_doubles(d, l, B);
+        nbr = n > nbr ? n : nbr;
+    }
+    L.nbr = take(nbr);
+    L.pscaled = has_input_scale(d) ? take(nodes * 4) : -1;
+    L.total = o;
+    return L;
+}
 static Layout layout(const LgaeModelDesc* d, int64_t B) {
+    if (is_md3(d)) return layout_md3(d, B);
     Layout L;
     const int64_t nodes = B * d->n_particles;
     int64_t o = 0;
@@ -235,6 +270,8 @@ static Layout layout(const LgaeModelDesc* d, int64_t B) {
     // encoder with an input scale: the scaled momenta every kernel of the model reads
     L.pscaled = has_input_scale(d) ? take(nodes * 4) : -1;
     L.total = o;
+    for (int l = 0; l <= LGAE_MAX_LEVELS; ++l) L.H[l] = -1;
+    L.nbr = -1;
     return L;
 }
 
@@ -247,6 +284,8 @@ static int check_desc(const LgaeModelDesc* d) {
     if (d->has_mlp && (d->mlp_activation < 0 || d->mlp_activation >= LGAE_ACT_COUNT)) return LGAE_E_UNSUPPORTED;
     for (int l = 0; d->has_mlp && l < d->n_levels; ++l)
         if (!mlp_tiling_supported(d, l)) return LGAE_E_UNSUPPORTED;   // hidden width above 96: no MLP kernel takes it
+    if (d->maxdim != 0 && d->maxdim != 2 && d->maxdim != 3) return LGAE_E_UNSUPPORTED;
+    if (d->maxdim == 3 && md3_level_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
     return LGAE_OK;
 }
 
@@ -414,11 +453,13 @@ int64_t lgae_workspace_offset(const LgaeModelDesc* d, int32_t batch, int32_t kin
         case 6: return level < d->n_levels ? L.acts[level] : -1;
         case 7: return level < d->n_levels ? L.rsave[level] : -1;
         case 8: return level < d->n_levels ? L.gr[level] : -1;
+        case 9: return L.H[level];
         default: return -1;
     }
 }
 int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch) {
     if (check_desc(d) != LGAE_OK || batch < 0) return -1;
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // maxdim 3: forward only
     int64_t n = glue_part_doubles(d, batch) + reduce_scratch_doubles();
     for (int l = 0; l < d->n_levels; ++l) {
         n += (int64_t)level_bwd_grid(batch) * level_part_width(d, l);
@@ -430,13 +471,14 @@ int64_t lgae_partials_doubles(const LgaeModelDesc* d, int32_t batch) {
 int64_t lgae_backward_tiled_scratch_doubles(const LgaeModelDesc* d, int32_t batch) {
     const int rc = check_desc(d);
     if (rc == LGAE_E_BADARG || batch < 0) return -1;
-    if (rc != LGAE_OK || tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    if (rc != LGAE_OK || is_md3(d) || tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
     return tiled_scratch(d, batch).total;
 }
 int64_t lgae_train_step_tiled_scratch_doubles(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int32_t batch) {
     const int re = check_desc(enc), rd = check_desc(dec);
     if (re == LGAE_E_BADARG || rd == LGAE_E_BADARG || batch < 0 || enc->is_decoder || !dec->is_decoder) return -1;
-    if (re != LGAE_OK || rd != LGAE_OK || tiled_check(enc) != LGAE_OK || tiled_check(dec) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    if (re != LGAE_OK || rd != LGAE_OK || is_md3(enc) || is_md3(dec) || tiled_check(enc) != LGAE_OK || tiled_check(dec) != LGAE_OK)
+        return LGAE_E_UNSUPPORTED;
     if (const int rc = train_step_glue_check(enc, dec)) return rc == LGAE_E_BADARG ? -1 : LGAE_E_UNSUPPORTED;
     return step_scratch(enc, dec, batch).total;
 }
@@ -604,6 +646,39 @@ static int dec_backward_launch(const LgaeModelDesc* d, const double* theta, cons
     return LGAE_OK;
 }
 
+// LGNEncoder.forward at maxdim 3: the same input map, scalar MLPs and latent glue as at maxdim 2 around the maxdim-3 level
+// kernels (lgae_md3.cu); nothing is kept for an adjoint.
+static int enc_forward_md3(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
+                           double* ws, double* lat00, double* lat11, int32_t* sel, cudaStream_t st) {
+    const Layout L = layout(d, batch);
+    const int64_t rows = (int64_t)batch * d->n_particles;
+    LGAE_TRY(run_mlp_pack(d, theta, ws, L.wpack, st));
+    LGAE_TRY(run_enc_input(d, theta, p4, batch, ws + L.mass, ws + L.S[0], ws + L.V[0], st));
+    for (int l = 0; l < d->n_levels; ++l) {
+        LGAE_TRY(run_md3_level_fwd(d, l, theta, p4, node_mask, batch, ws + L.S[l], ws + L.V[l], l > 0 ? ws + L.H[l] : nullptr, ws + L.nbr,
+                                   ws + L.spre[l], ws + L.V[l + 1], ws + L.H[l + 1], st));
+        if (d->has_mlp)
+            LGAE_TRY(run_mlp(d, l, theta, ws + L.wpack[l], ws + L.spre[l], rows, ws + L.acts[l], ws + L.S[l + 1], nullptr, nullptr, nullptr, false, st));
+    }
+    return run_enc_latent(d, theta, batch, ws + L.S[d->n_levels], ws + L.V[d->n_levels], lat00, lat11, sel, st);
+}
+
+// LGNDecoder.forward at maxdim 3; scalars_unused: the last level's scalar MLP feeds only gen00 and is skipped, as at maxdim 2.
+static int dec_forward_md3(const LgaeModelDesc* d, const double* theta, const double* lat11, int32_t batch, double* ws, double* recon,
+                           double* gen00, cudaStream_t st, bool scalars_unused) {
+    const Layout L = layout(d, batch);
+    const int64_t rows = (int64_t)batch * d->n_particles;
+    LGAE_TRY(run_mlp_pack(d, theta, ws, L.wpack, st));
+    LGAE_TRY(run_dec_input(d, theta, batch, lat11, ws + L.y, ws + L.S[0], ws + L.V[0], st));
+    for (int l = 0; l < d->n_levels; ++l) {
+        LGAE_TRY(run_md3_level_fwd(d, l, theta, ws + L.y, nullptr, batch, ws + L.S[l], ws + L.V[l], l > 0 ? ws + L.H[l] : nullptr, ws + L.nbr,
+                                   ws + L.spre[l], ws + L.V[l + 1], ws + L.H[l + 1], st));
+        if (d->has_mlp && !(scalars_unused && l == d->n_levels - 1))
+            LGAE_TRY(run_mlp(d, l, theta, ws + L.wpack[l], ws + L.spre[l], rows, ws + L.acts[l], ws + L.S[l + 1], nullptr, nullptr, nullptr, false, st));
+    }
+    return run_dec_output(d, theta, batch, ws + L.S[d->n_levels], ws + L.V[d->n_levels], recon, gen00, st);
+}
+
 extern "C" {
 
 int lgae_encoder_forward(const LgaeModelDesc* d, const double* theta, const double* p4, const uint8_t* node_mask, int32_t batch,
@@ -615,6 +690,7 @@ int lgae_encoder_forward(const LgaeModelDesc* d, const double* theta, const doub
     int rc = LGAE_OK;
     const double* x = scaled_input(d, p4, batch, ws, true, (cudaStream_t)stream, &rc);
     if (rc) return rc;
+    if (is_md3(d)) return enc_forward_md3(d, theta, x, node_mask, batch, ws, lat00, lat11, sel, (cudaStream_t)stream);
     return enc_forward_launch(d, theta, x, node_mask, batch, ws, lat00, lat11, sel, true, (cudaStream_t)stream);
 }
 
@@ -626,6 +702,7 @@ static int encoder_backward_impl(const LgaeModelDesc* d, const double* theta, co
                                  double* partials_or_scratch, double l1_lambda, double* loss_accumulate, bool tiled, InputGrad ig,
                                  void* stream) {
     LGAE_TRY(check_desc(d));
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // maxdim 3: forward only
     if (d->is_decoder || !theta || !gtheta || !partials_or_scratch || batch < 0 || (batch > 0 && (!p4 || !ws))) return LGAE_E_BADARG;
     if (ig.g_p4 && batch > 0 && !ig.scratch) return LGAE_E_BADARG;
     // before anything is launched
@@ -667,7 +744,7 @@ int lgae_encoder_backward_p4(const LgaeModelDesc* d, const double* theta, const 
 int64_t lgae_encoder_input_grad_scratch_doubles(const LgaeModelDesc* d, int32_t batch) {
     const int rc = check_desc(d);
     if (rc == LGAE_E_BADARG || batch < 0 || d->is_decoder) return -1;
-    if (rc != LGAE_OK || pgrad_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
+    if (rc != LGAE_OK || is_md3(d) || pgrad_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;
     if (d->n_particles > 32 && tiled_check(d) != LGAE_OK) return LGAE_E_UNSUPPORTED;   // the tiled adjoint runs these jets
     return input_grad_scratch(d, batch).total;
 }
@@ -680,6 +757,7 @@ int lgae_decoder_forward(const LgaeModelDesc* d, const double* theta, const doub
     if (!theta || !lat11 || !ws || !recon) return LGAE_E_BADARG;
     // gen00 == NULL: the caller does not want the output scalars, and the adjoint never reads the last level's saved
     // activations when there is no gradient on them, so the last level's scalar MLP is not evaluated
+    if (is_md3(d)) return dec_forward_md3(d, theta, lat11, batch, ws, recon, gen00, (cudaStream_t)stream, !gen00 && !keep_dead_mlp());
     return dec_forward_launch(d, theta, lat11, batch, ws, recon, gen00, true, (cudaStream_t)stream, true, true, !gen00 && !keep_dead_mlp());
 }
 
@@ -687,6 +765,7 @@ int lgae_decoder_backward(const LgaeModelDesc* d, const double* theta, const dou
                           const double* g_recon, const double* g_gen00, double* g_lat11, double* gtheta, double* partials,
                           double l1_lambda, double* loss_accumulate, void* stream) {
     LGAE_TRY(check_desc(d));
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // maxdim 3: forward only
     if (!d->is_decoder || !theta || !gtheta || !partials || batch < 0 || (batch > 0 && (!lat11 || !ws || !g_recon || !g_lat11)))
         return LGAE_E_BADARG;
     if (d->n_particles > 32) return LGAE_E_UNSUPPORTED;   // before anything is launched: the adjoint holds one particle per lane
@@ -715,6 +794,7 @@ int lgae_decoder_backward_tiled(const LgaeModelDesc* d, const double* theta, con
                                 const double* g_recon, const double* g_gen00, double* g_lat11, double* gtheta, double* scratch,
                                 double l1_lambda, double* loss_accumulate, void* stream) {
     LGAE_TRY(check_desc(d));
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // maxdim 3: forward only
     if (!d->is_decoder || !theta || !gtheta || !scratch || batch < 0 || (batch > 0 && (!lat11 || !ws || !g_recon || !g_lat11)))
         return LGAE_E_BADARG;
     LGAE_TRY(tiled_check(d));
@@ -731,6 +811,7 @@ void* lgae_aux_stream(void) {
 }
 
 int64_t lgae_train_step_partials_doubles(const LgaeModelDesc* enc, const LgaeModelDesc* dec, int32_t batch) {
+    if (check_desc(enc) == LGAE_OK && check_desc(dec) == LGAE_OK && batch >= 0 && (is_md3(enc) || is_md3(dec))) return LGAE_E_UNSUPPORTED;
     const int64_t a = lgae_partials_doubles(enc, batch), b = lgae_partials_doubles(dec, batch);
     if (a < 0 || b < 0) return -1;
     // + the fused decoder tail's rows (one per jet) and one trailing double whose first 4 bytes are its completion counter
@@ -759,6 +840,7 @@ static int train_step_impl(const LgaeModelDesc* enc, const LgaeModelDesc* dec, c
                            bool tiled, void* stream) {
     LGAE_TRY(check_desc(enc));
     LGAE_TRY(check_desc(dec));
+    if (is_md3(enc) || is_md3(dec)) return LGAE_E_UNSUPPORTED;   // maxdim 3: forward only
     if (enc->is_decoder || !dec->is_decoder || batch < 1 || gtheta_dec_offset < enc->n_params) return LGAE_E_BADARG;
     if (get_real < LGAE_GET_REAL_REAL || get_real > LGAE_GET_REAL_NORM || phase < 0 || phase > 2) return LGAE_E_BADARG;
     if (!theta_enc || !theta_dec || !p4_in || !p4 || !ws_enc || !ws_dec || !lat00 || !lat11 || !sel || !recon || !g_recon || !g_lat11 ||
@@ -975,6 +1057,7 @@ int lgae_level_forward(const LgaeModelDesc* d, int32_t level, const double* thet
                        int32_t batch, const double* s_in, const double* v_in, double* sums, double* r_save, double* s_pre, double* v_out,
                        void* stream) {
     LGAE_TRY(check_desc(d));
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // the stage-level entry points are the maxdim-2 level
     if (!theta || !p_or_y || !s_in || !v_in || !sums || !s_pre || !v_out || batch < 0 || level < 0 || level >= d->n_levels) return LGAE_E_BADARG;
     if (!d->is_decoder && r_save && d->n_particles > 32) return LGAE_E_UNSUPPORTED;   // the saved radial weights are a 32-particle layout
     if (!d->is_decoder && d->n_particles <= 32 && r_save)
@@ -986,6 +1069,7 @@ int lgae_level_backward(const LgaeModelDesc* d, int32_t level, const double* the
                         double* g_r_scratch, const double* g_s_pre, const double* g_v_out, double* g_s_in, double* g_v_in,
                         double* g_y_accumulate, double* gtheta, double* partials, void* stream) {
     LGAE_TRY(check_desc(d));
+    if (is_md3(d)) return LGAE_E_UNSUPPORTED;   // the stage-level entry points are the maxdim-2 level
     if (!theta || !p_or_y || !s_in || !v_in || !sums || !g_v_out || !g_s_in || !g_v_in || !gtheta || !partials || batch < 0 || level < 0 ||
         level >= d->n_levels)
         return LGAE_E_BADARG;

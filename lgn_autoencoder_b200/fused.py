@@ -38,7 +38,7 @@ class FusedPlan:
 
     def __init__(self, kind: str, shapes: "OrderedDict[str, Tuple[int, ...]]", *, n_particles: int, channels: Sequence[int],
                  num_basis_fn: int = 10, mlp: bool = True, mlp_depth: int = 6, mlp_width: int = 6, latent_mode: str = "mean",
-                 tau_s: int = 1, tau_v: int = 1, input_scale: float = 1.0, activation: str = "leakyrelu"):
+                 tau_s: int = 1, tau_v: int = 1, input_scale: float = 1.0, activation: str = "leakyrelu", maxdim: int = 2):
         assert kind in ("encoder", "decoder")
         self.kind = kind
         self.names: List[str] = list(shapes)
@@ -58,7 +58,11 @@ class FusedPlan:
         self.n_levels = len(self.channels) - 1
         self.latent_mode = latent_mode
         self.tau_s, self.tau_v = int(tau_s), int(tau_v)
+        if int(maxdim) not in (2, 3):
+            raise NotImplementedError(f"maxdim {maxdim} is not implemented by the fused B200 path (2, or 3 forward only)")
+        self.maxdim = int(maxdim)
         d = LgaeModelDesc()
+        d.maxdim = self.maxdim
         d.is_decoder = 1 if kind == "decoder" else 0
         d.n_levels = self.n_levels
         d.n_particles = self.n_particles
@@ -92,6 +96,8 @@ class FusedPlan:
             d.off_rad_w1[l], d.off_rad_b1[l] = o(pre + ".linear.1.weight"), o(pre + ".linear.1.bias")
             mixp = f"lgn_cg.node_levels.{l}.cat_mix.mix_reps.weights."
             d.off_mix00[l], d.off_mix11[l] = o(mixp + "(0, 0)"), o(mixp + "(1, 1)")
+            if self.maxdim == 3:
+                d.off_mix20[l], d.off_mix02[l], d.off_mix22[l] = o(mixp + "(2, 0)"), o(mixp + "(0, 2)"), o(mixp + "(2, 2)")
             if mlp:
                 d.mlp_width[l] = int(mlp_width) * 2 * self.channels[l + 1]
                 for i in range(int(mlp_depth) + 1):
@@ -126,6 +132,10 @@ class FusedPlan:
             raise NotImplementedError("configuration not supported by the fused B200 path")
         return torch.empty(max(int(n), 1), dtype=torch.float64, device=device)
 
+    def forward_supported(self) -> bool:
+        """True if the library's forward entry points take this descriptor (no GPU needed)."""
+        return self._lib.lgae_workspace_doubles(C.byref(self.desc), 1) >= 0
+
     def partials(self, batch: int, device) -> torch.Tensor:
         n = self._lib.lgae_partials_doubles(C.byref(self.desc), batch)
         return torch.empty(max(int(n), 1), dtype=torch.float64, device=device)
@@ -154,13 +164,21 @@ class FusedPlan:
             n *= s
         return ws[off:off + n].view(shape)
 
-    def node_features(self, ws: torch.Tensor, batch: int, level: int) -> Dict[Tuple[int, int], torch.Tensor]:
+    def node_features(self, ws: torch.Tensor, batch: int, level: int, mlp: bool = True) -> Dict[Tuple[int, int], torch.Tensor]:
         """Planar (2,B,N,C,d) copies of the node features entering level ``level`` (level == n_levels: the
-        output of the last level), in the reference's GVec part order [(1,1), (0,0)]."""
+        output of the last level), in the reference's GVec part order: [(1,1), (0,0)] at maxdim 2; at maxdim 3 the order
+        of md3_layout.node_order (the MixReps set order, with (0,0) last after a scalar MLP, ``mlp``)."""
         n, c = self.n_particles, self.channels[level]
         s = self.ws_tensor(ws, batch, 0, level, (batch, n, c, 2))
         v = self.ws_tensor(ws, batch, 1, level, (batch, n, c, 4, 2))
-        return OrderedDict([((1, 1), v.permute(4, 0, 1, 2, 3).contiguous()), ((0, 0), s.permute(3, 0, 1, 2).unsqueeze(-1).contiguous())])
+        parts = {(1, 1): v.permute(4, 0, 1, 2, 3).contiguous(), (0, 0): s.permute(3, 0, 1, 2).unsqueeze(-1).contiguous()}
+        if self.maxdim == 2 or level == 0:
+            return OrderedDict([((1, 1), parts[(1, 1)]), ((0, 0), parts[(0, 0)])])
+        from . import md3_layout
+        h = self.ws_tensor(ws, batch, 9, level, (batch, n, c, 15, 2)).permute(4, 0, 1, 2, 3)
+        for key, lo, hi in (((2, 0), 0, 3), ((0, 2), 3, 6), ((2, 2), 6, 15)):
+            parts[key] = h[..., lo:hi].contiguous()
+        return OrderedDict((k, parts[k]) for k in md3_layout.node_order("mlp" if mlp else "nomlp"))
 
 
 # -----------------------------------------------------------------------------------------------------------

@@ -112,13 +112,13 @@ class FusedParamsMixin:
 
     def l1_norm(self):
         """sum |p| over all parameters (lgn_encoder.py:249-250), evaluated on the flat buffer in one reduction."""
-        if self._plan is None:
+        if self._plan is None or not self.fused:   # models that train on the composite (maxdim 3) sum per tensor
             return sum(p.abs().sum() for p in self.parameters())
         return _FlatNormFn.apply(self._theta_node(), 1)
 
     def l2_norm(self):
         """sum p^2 over all parameters (lgn_encoder.py:252-253)."""
-        if self._plan is None:
+        if self._plan is None or not self.fused:
             return sum(torch.pow(p, 2).sum() for p in self.parameters())
         return _FlatNormFn.apply(self._theta_node(), 2)
 

@@ -60,17 +60,22 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         self.num_learnable_parameters = sum(p.nelement() for p in self.parameters() if p.requires_grad)
 
         self._fused_reason = self._why_not_fused()
+        self._forward_reason = self._why_not_fused(maxdims=(2, 3))   # forward-only calls: maxdim 3 too
         self._tiled_reason = None   # why autograd calls with N > 32 train through the composite (None: the tiled fused adjoint)
-        if self._fused_reason is None:
+        if self._forward_reason is None:
             self._build_plan("decoder", n_particles=num_output_particles, channels=list(num_channels), num_basis_fn=num_basis_fn, mlp=mlp,
                              mlp_depth=mlp_depth if mlp else 0, mlp_width=mlp_width if mlp else 0, tau_s=tau_latent_scalars,
-                             tau_v=tau_latent_vectors, activation=activation)
-            if num_output_particles > 32:
+                             tau_v=tau_latent_vectors, activation=activation, maxdim=maxdim[0])
+            if not self.fused and not self._plan.forward_supported():
+                self._forward_reason = "maxdim-3 level kernels: shared memory does not fit this configuration"
+            if self.fused and num_output_particles > 32:
                 self._tiled_reason = self._plan.tiled_reason()
 
-    def _why_not_fused(self):
-        if any(m != 2 for m in self.level_maxdim):
-            return f"maxdim {self.level_maxdim} (fused path: 2)"
+    def _why_not_fused(self, maxdims=(2,)):
+        """None if the sm_100a fused path implements this configuration, else the reason.  ``maxdims``: the maxdim every level
+        may have (2: training and forward; 3: the forward only, csrc/lgae_md3.cu)."""
+        if not any(all(m == md for m in self.level_maxdim) for md in maxdims):
+            return f"maxdim {self.level_maxdim} (fused path: {' or '.join(map(str, maxdims))})"
         if any(z != 1 for z in self.max_zf):
             return f"max_zf {self.max_zf} (fused path: 1)"
         if self.tau_output_scalars != 1 or self.tau_output_vectors != 1:
@@ -85,7 +90,13 @@ class LGNDecoder(FusedParamsMixin, CGModule):
 
     @property
     def fused(self) -> bool:
+        """Trains (and runs) on the fused path."""
         return self._fused_reason is None
+
+    @property
+    def fused_forward(self) -> bool:
+        """Calls that need no gradient run on the fused path (maxdim 2, and maxdim 3 forward-only)."""
+        return self._forward_reason is None
 
     def forward(self, latent_features, covariance_test=False, nodes_all=None):
         """latent GVec {(0,0): (2,B,1,T_s,1), (1,1): (2,B,1,T_v,4)} -> (2,B,N,4) complex Cartesian momenta.  With
@@ -99,6 +110,9 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         needs_grad = torch.is_grad_enabled() and (lat11.requires_grad or any(p.requires_grad for p in self.parameters()))
         if self.fused and not (needs_grad and self.num_output_particles > 32 and self._tiled_reason is not None):
             return self._forward_fused(lat11, covariance_test, nodes_all)
+        # maxdim 3: the fused forward for calls that need no gradient (the adjoint is the composite's autograd)
+        if self.fused_forward and not self.fused and not needs_grad:
+            return self._forward_fused(lat11, covariance_test, nodes_all)
         return self._forward_generic(latent_features, covariance_test, nodes_all)
 
     def _forward_fused(self, lat11, covariance_test, nodes_all):
@@ -111,7 +125,7 @@ class LGNDecoder(FusedParamsMixin, CGModule):
         recon, gen00 = out
         gen = GVec({(0, 0): gen00, (1, 1): p_cplx_to_rep(recon)[(1, 1)].unsqueeze(-2)}, ignore_check=True)
         for l in range(self.num_cg_levels + 1):
-            nodes_all.append(GVec(self._plan.node_features(holder["ws"], b, l), ignore_check=True))
+            nodes_all.append(GVec(self._plan.node_features(holder["ws"], b, l, mlp=self.mlp), ignore_check=True))
         nodes_all.append(gen)
         return gen, nodes_all
 

@@ -73,20 +73,24 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         self.num_learnable_parameters = sum(p.nelement() for p in self.parameters() if p.requires_grad)
 
         self._fused_reason = self._why_not_fused()
+        self._forward_reason = self._why_not_fused(maxdims=(2, 3))   # forward-only calls: maxdim 3 too
         self._tiled_reason = None   # why autograd calls with N > 32 train through the composite (None: the tiled fused adjoint)
-        if self._fused_reason is None:
+        if self._forward_reason is None:
             self._build_plan("encoder", n_particles=self.num_input_particles, channels=list(num_channels), num_basis_fn=num_basis_fn,
                              mlp=mlp, mlp_depth=mlp_depth if mlp else 0, mlp_width=mlp_width if mlp else 0,
                              latent_mode=map_to_latent, tau_s=tau_latent_scalars, tau_v=tau_latent_vectors, input_scale=scale,
-                             activation=activation)
-            if self.num_input_particles > 32:
+                             activation=activation, maxdim=maxdim[0])
+            if not self.fused and not self._plan.forward_supported():
+                self._forward_reason = "maxdim-3 level kernels: shared memory does not fit this configuration"
+            if self.fused and self.num_input_particles > 32:
                 self._tiled_reason = self._plan.tiled_reason()
 
     # ---------------------------------------------------------------------------------------------------------
-    def _why_not_fused(self):
-        """None if the sm_100a fused path implements this configuration, else the reason."""
-        if any(m != 2 for m in self.level_maxdim):
-            return f"maxdim {self.level_maxdim} (fused path: 2)"
+    def _why_not_fused(self, maxdims=(2,)):
+        """None if the sm_100a fused path implements this configuration, else the reason.  ``maxdims``: the maxdim every level
+        may have (2: training and forward; 3: the forward only, csrc/lgae_md3.cu)."""
+        if not any(all(m == md for m in self.level_maxdim) for md in maxdims):
+            return f"maxdim {self.level_maxdim} (fused path: {' or '.join(map(str, maxdims))})"
         if any(z != 1 for z in self.max_zf):
             return f"max_zf {self.max_zf} (fused path: 1)"
         if self.jet_features:
@@ -107,7 +111,13 @@ class LGNEncoder(FusedParamsMixin, CGModule):
 
     @property
     def fused(self) -> bool:
+        """Trains (and runs) on the fused path."""
         return self._fused_reason is None
+
+    @property
+    def fused_forward(self) -> bool:
+        """Calls that need no gradient run on the fused path (maxdim 2, and maxdim 3 forward-only)."""
+        return self._forward_reason is None
 
     # ---------------------------------------------------------------------------------------------------------
     def forward(self, data: Union[Dict[str, torch.Tensor], torch.Tensor, np.ndarray], covariance_test: bool = False
@@ -124,6 +134,9 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         # layer-level composite, whose autograd covers any N; forward-only calls keep the fused kernels
         needs_grad = torch.is_grad_enabled() and (p4.requires_grad or any(p.requires_grad for p in self.parameters()))
         if self.fused and "scalars" not in data and not (needs_grad and p4.shape[1] > 32 and self._tiled_reason is not None):
+            return self._forward_fused(data, p4, covariance_test)
+        # maxdim 3: the fused forward for calls that need no gradient (the adjoint is the composite's autograd)
+        if self.fused_forward and not self.fused and "scalars" not in data and not needs_grad:
             return self._forward_fused(data, p4, covariance_test)
         return self._forward_generic(data, p4, covariance_test)
 
@@ -149,7 +162,7 @@ class LGNEncoder(FusedParamsMixin, CGModule):
         if not covariance_test:
             return latent
         b = p4.shape[0]
-        nodes_all = [GVec(self._plan.node_features(holder["ws"], b, l), ignore_check=True) for l in range(self.num_cg_levels + 1)]
+        nodes_all = [GVec(self._plan.node_features(holder["ws"], b, l, mlp=self.mlp), ignore_check=True) for l in range(self.num_cg_levels + 1)]
         return latent, nodes_all
 
     # generic layer-level composite (any maxdim / pooling); follows the call sequence of lgn_encoder.py:255-412

@@ -439,8 +439,8 @@ class FusedInference:
 
     def __init__(self, encoder, decoder, batch: int, normalize: bool = True, use_labels: bool = False, use_graph: bool = True,
                  get_real: str = "real"):
-        if not (getattr(encoder, "fused", False) and getattr(decoder, "fused", False)):
-            raise NotImplementedError("FusedInference needs the fused (maxdim 2) encoder and decoder")
+        if not (getattr(encoder, "fused_forward", False) and getattr(decoder, "fused_forward", False)):
+            raise NotImplementedError("FusedInference needs the fused (maxdim 2 or 3) encoder and decoder")
         self.get_real = fused.get_real_mode(get_real)
         self.enc, self.dec, self.B = encoder, decoder, int(batch)
         self.pe, self.pd = encoder._plan, decoder._plan
