@@ -32,6 +32,7 @@ struct CgArgs {
 
 constexpr int CG_THREADS = 256;
 constexpr int CG_ITEMS = 4;   // work items per thread held in registers
+constexpr size_t CG_SMEM_MAX = 227 * 1024;   // dynamic shared memory one sm_100 CTA may opt in to
 
 // Term list of one ordering (0: by output component, 1: by a, 2: by d) -> shared memory.
 struct TermsSm {
@@ -1044,7 +1045,9 @@ int lgae_cg_product_forward(const LgaeCgPairDesc* d, const int32_t* tab, const d
         launch_k(cg_agg_fwd_kron_kernel<D>, grid, dim3(CG_THREADS), bytes + kb, st, p);               \
         return check_launch("cg_aggregate_fwd");                                                      \
     }
-            LGAE_KRON(1) LGAE_KRON(3) LGAE_KRON(4) LGAE_KRON(9)
+            if (bytes + kb <= CG_SMEM_MAX) {   // the Kronecker form also holds IB * C * d1 * d2 of K
+                LGAE_KRON(1) LGAE_KRON(3) LGAE_KRON(4) LGAE_KRON(9)
+            }
 #undef LGAE_KRON
             if (int rc = ensure_smem((const void*)cg_agg_fwd_block_kernel, bytes)) return rc;
             launch_k(cg_agg_fwd_block_kernel, grid, dim3(CG_THREADS), bytes, st, p);
@@ -1101,9 +1104,11 @@ int lgae_cg_product_backward(const LgaeCgPairDesc* d, const int32_t* tab, const 
                 const dim3 grid(q.B, (q.N + ib - 1) / ib);
                 const size_t kbytes = terms_doubles(p.n_terms, p.d1 + 1) * sizeof(double) +
                                       ((size_t)p.NJ * p.C * p.d1 + (size_t)ib * p.C * p.n_comp + (size_t)ib * p.C * p.d1 * p.d2) * sizeof(cplx);
+                // the Kronecker form also holds IB * C * d1 * d2 of gK: the generic kernel where that does not fit
+                const bool kron_fits = kbytes <= CG_SMEM_MAX;
                 bool done = false;
 #define LGAE_KRON(D)                                                                                          \
-    if (!done && p.d2 == D) {                                                                                 \
+    if (!done && kron_fits && p.d2 == D) {                                                                    \
         if (int rc = ensure_smem((const void*)cg_agg_bwd_edge_kron_kernel<D>, kbytes)) return rc;             \
         launch_k(cg_agg_bwd_edge_kron_kernel<D>, grid, dim3(CG_THREADS), kbytes, st, q);                      \
         done = true;                                                                                          \
